@@ -2,6 +2,7 @@
 """bench.py — chain-iterations/s of the openMCMC hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c2|c1|c3|c4a|c4b|c5|c5full]
+                    [--dump-outputs DIR]
 
 A "step" is one sweep (every sampler once) over all chains of the workload; `value` = chain-iterations/s with the
 inputs resident in HBM; `e2e` = the same metric through the public API (`MCMC(...).run_mcmc()`) with HOST inputs, the
@@ -86,7 +87,14 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the comparison legs (sweep forms, fitted values, ESS "
                                                              "run, c3 sub-record, strong scaling)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's stored iteration of every array in "
+                         "MCMC.store (rank 0's chains) as DIR/<name>.npy, float64, at most 64 MB in all (a fixed "
+                         "seeded sample of the elements of an array too large for that)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 implementation; --impl reference has none to dump")
+    return args
 
 
 def config_of(args, wl):
@@ -652,6 +660,30 @@ def e2e_leg(ctx, wl, key, C, n, p, steps, thin, upload_blocks):
     return out
 
 
+DUMP_BYTES = 60 * 10 ** 6      # under 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, store):
+    """What a caller of the timed run receives for its last step -- the last stored iteration of every array of
+    `MCMC.store` -- as out_dir/<name>.npy in float64, so that two builds can be compared output for output.  Small
+    arrays are written whole; an array larger than its share of DUMP_BYTES is cut to a sample of its flat elements
+    drawn with a fixed seed (sorted indices), the same for the same shapes."""
+    import numpy as np
+
+    last = {}
+    for name, arr in store.items():
+        a = np.asarray(arr, dtype=np.float64)
+        last[name] = a[-1] if name == "log_post" else a[..., -1]    # log_post is [n_iter, C]; the rest end in n_iter
+    os.makedirs(out_dir, exist_ok=True)
+    budget, left = DUMP_BYTES, len(last)
+    for name, a in sorted(last.items(), key=lambda kv: kv[1].nbytes):
+        share = budget // left
+        if a.nbytes > share:
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, share // 8, replace=False))]
+        budget, left = budget - a.nbytes, left - 1
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 def fp64_dgemm_peak(ctx):
     torch = ctx.torch
     a = torch.randn(6144, 6144, dtype=torch.float64, device=ctx.dev)
@@ -757,6 +789,8 @@ def run_b200(args, wl, key):
     clk = clocks.stop()
     ess = ess_record(ctx, M, wl, n, ms_max)
     M.collect()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, M.store)
     status_bad = int(((M.status & 3) != 0).sum())
     accept = {s.param: s.accept_rate.get_acceptance_rate() for s in samplers if hasattr(s, "accept_rate")}
     value = C * world * args.steps / (ms_max * 1e-3)

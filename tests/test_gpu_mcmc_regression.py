@@ -49,8 +49,9 @@ def build(g, n_chains=1, response=True):
 @pytest.mark.parametrize("name", NAMES)
 def test_mcmc_replays_reference_chain(name):
     from openmcmc_b200.mcmc import MCMC
+    from test_oracle_vs_golden import _load
 
-    g = dict(np.load(os.path.join(GOLD, name + ".npz")))
+    g = _load(name)
     mdl, samplers, state = build(g)
     n_iter = g["store_beta"].shape[1]
     dd = {"beta": {"z": g["z"]}, "tau": {"g": g["g_tau"]}, "lambda": {"g": g["g_lambda"]}}
