@@ -16,6 +16,9 @@ namespace {
 
 constexpr int DD_THREADS = 256;
 constexpr int PMAX = 512;
+// above this p the left-looking warp kernel (14 chains per SM) runs instead of the register one (8): measured faster at
+// p = 48, 56, 63 and 64 with 4096 chains (profiles/r03_draw_only.txt)
+constexpr int LEFT_MIN_P = 40;
 
 __device__ __forceinline__ double vec_at(const omc_vec_t& v, int chain, int i, double dflt) {
   return v.ptr ? v.ptr[(long long)chain * v.chain_stride + i] : dflt;
@@ -364,13 +367,17 @@ extern "C" int omc_nn_dense_draw(const omc_nn_dense_t* args, void* stream) {
     OMC_LAUNCH_CHECK();
     return 0;
   }
-  // p <= 64 without probes: one warp per chain, Q in registers (dense_warp.cu).  Probes (Q, b, L, mu of the parity
-  // tests) go through the kernels that keep the factor addressable: one thread per column (p <= 32) or the blocked
-  // Cholesky (dense_blocked.cu), which also serves 64 < p <= 512.  OMC_DENSE_DRAW_IMPL = warp | columns | blocked
-  // forces one of them where it applies (A/B timing, tools/perf_dense_draw.py).
+  // p <= 64 without probes: one warp per chain (dense_warp.cu), the left-looking kernel with the factor in shared
+  // memory above LEFT_MIN_P, Q in registers below.  Probes (Q, b, L, mu of the parity tests) go through the kernels
+  // that keep the factor addressable: one thread per column (p <= 32) or the blocked Cholesky (dense_blocked.cu), which
+  // also serves 64 < p <= 512.  OMC_DENSE_DRAW_IMPL = left | warp | columns | blocked forces one of them where it
+  // applies (A/B timing, tools/perf_dense_draw.py).
   static const char impl = [] { const char* e = getenv("OMC_DENSE_DRAW_IMPL"); return e ? e[0] : '\0'; }();
   const bool probes = args->probe_Q || args->probe_b || args->probe_L || args->probe_mu;
-  if (p <= 64 && !probes && (impl == '\0' || impl == 'w')) return omc_launch_warp_draw(*args, (cudaStream_t)stream);
+  if (p <= 64 && !probes) {
+    if ((impl == '\0' && p > LEFT_MIN_P) || (impl == 'l' && p > 32)) return omc_launch_left_draw(*args, (cudaStream_t)stream);
+    if (impl == '\0' || impl == 'w') return omc_launch_warp_draw(*args, (cudaStream_t)stream);
+  }
   if (impl != 'b' || p <= 0) {
     if (p <= 8) return launch_dense_draw<8>(*args, (cudaStream_t)stream);
     if (p <= 16) return launch_dense_draw<16>(*args, (cudaStream_t)stream);

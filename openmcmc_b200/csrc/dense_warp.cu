@@ -1,45 +1,45 @@
-// omc_nn_dense_draw for p <= 64 without probes: ONE WARP per chain, the whole posterior precision in REGISTERS.
+// omc_nn_dense_draw for p <= 64 without probes: ONE WARP per chain.
 //
 //   Q = lambda*P0 + tau*G, L = chol(Q), x = L^-T (L^-1 b + z)          ref: sampler.py:154-207, gmrf.py:167-198, 29-61
 //   (= mu + L^-T z with mu = L^-T L^-1 b, the reference's two solves folded into one backward substitution)
 //
-// The lower triangle of Q lives in the warp as 8 x 8 tiles in the accumulator layout of mma.sync.m8n8k4.f64: lane
-// (g = lane / 4, kq = lane % 4) holds elements [g][2kq], [g][2kq+1] of every tile -- 36 tiles = 72 doubles per lane at
-// p = 64.  No shared memory, no CTA barrier: the CTA-wide kernels of the first round spent 40-55 % of a chain's life
-// at barriers around their serial sections (profiles/r02_ncu_blocked64.txt) with 4-5 chains resident per SM;
-// here 8 chains are resident per SM and every one of them always has work to issue.
+// Q is handled as 8 x 8 tiles in the accumulator layout of mma.sync.m8n8k4.f64: lane (g = lane / 4, kq = lane % 4)
+// holds elements [g][2kq], [g][2kq+1] of a tile.  No CTA barrier: the CTA-wide kernels of the first round spent 40-55 %
+// of a chain's life at barriers around their serial sections (profiles/r02_ncu_blocked64.txt).  Two forms:
 //
-// Right-looking by block columns k (tools/gen/warp_chol_model.py is the lane-level numpy model of this file):
-//   * the 8 pivots of block column k: pivot from the diagonal tile by shuffle, 1/sqrt by MUFU.RSQ64H + two Newton
-//     steps, scale column, rank-1 update of the remaining columns of EVERY tile of the block column (independent work
-//     across the tiles hides the pivot chain); the right-hand side b (row layout, element 8i + g) rides along, so
-//     w = L^-1 b is there when the factorisation ends; 1/L_cc replaces L_cc on the diagonal;
-//   * trailing update on the FP64 tensor pipe: T(i, j) -= L(i, k) L(j, k)' as two DMMA.8x8x4 per tile, the operand
-//     fragments being the panel tiles re-laid out inside their quads (4 shuffles per tile, once per block column).
+// * Register kernel (nn_warp_draw_kernel, small p): the whole lower block triangle in registers (36 tiles = 72 doubles
+//   per lane at p = 64), right-looking by block columns k (tools/gen/warp_chol_model.py is its lane-level numpy model):
+//   the pivot stages of block column k (below), then the trailing update T(i, j) -= L(i, k) L(j, k)' as two
+//   DMMA.8x8x4 per tile, the operand fragments being the panel tiles re-laid out inside their quads (4 shuffles per
+//   tile).  At p = 64 it needs 254 registers per thread: 8 chains per SM.
+// * Left-looking kernel (nn_left_draw_kernel, larger p; dense_draw.cu selects): only block column k in registers
+//   (<= 16 doubles per lane, read from the record at the top of step k), the finished factor in the warp's slice of
+//   shared memory.  Step k: C(i, k) = Q(i, k) - sum_{j<k} L(i, j) L(k, j)', i >= k, on the tensor pipe with both operand
+//   fragments (element [g][4s + kq] of a tile) read straight from shared memory; the pivot stages of column k; L(:, k)
+//   back to shared memory.  Every tile sees the same DMMAs with the same operands in the same order as in the
+//   right-looking form.  At p = 64: 128 registers and 16,352 bytes of shared memory per warp, 14 chains per SM,
+//   persistent warps, the next chain's record prefetched into L2 while the current one runs.  (A register copy of
+//   block column k + 1 loaded one step ahead does not fit in the 128 registers: 4 of the 14 warps share one quarter
+//   of the register file.)
+//
+// Pivot stages of block column k (both forms): pivot from the diagonal tile by shuffle, 1/sqrt by MUFU.RSQ64H + two
+// Newton steps, scale column, rank-1 update of the remaining columns of EVERY tile of the block column (independent work
+// across the tiles hides the pivot chain); the right-hand side b (row layout, element 8i + g) rides along, so
+// w = L^-1 b is there when the factorisation ends; 1/L_cc replaces L_cc on the diagonal.
 // Backward solve L' x = w + z block by block from the bottom: partial sums of the off-diagonal products stay private
 // per lane and are reduced over g (3 xor-shuffles) once per block; the 8 x 8 diagonal solves are quad-local.
 // Epilogue: rss(beta) = rss0 - 2 d'c0 + d'G d from the centre record (omc.h), G read a second time (L2).
-// Warps are persistent (chain = warp id, + number of warps, ...).  With packed even-p records (STAGE) the record of a
-// warp's NEXT chain is on its way into that warp's shared-memory slab (1-D bulk copies through the TMA engine, one per
-// row of the lower block triangle, completion on a per-warp mbarrier) while the current chain is factorised out of
-// registers: a third of a chain's life was the HBM latency of its 36 tile loads with nothing to overlap it
-// (profiles/r02_ncu_warp64_v1.txt, r02_ncu_warp64_lines.txt for the shipped kernel).
 #include "../../include/omc.h"
 #include "omc_common.cuh"
 #include "omc_internal.h"
 
+#include <utility>
+
 namespace {
 
 constexpr unsigned FULL = 0xffffffffu;
-constexpr int WARPS_PER_CTA = 4;
-// -DDW_DMMA_PANEL=1: panel tiles by the tensor pipe (L(i,k) = T(i,k) L_kk^-T, the inverse transpose built by running the
-// pivot stages on an identity tile) instead of inside the pivot stages.  Correct (the parity tests pass with it) and 870
-// instructions per chain fewer, but MEASURED slower at p = 64: 0.121 against 0.114 ms -- the rank-1 updates of the panel
-// tiles are the independent work that hides the pivot chain (profiles/r02_ncu_warp64_lines.txt).
-#ifndef DW_DMMA_PANEL
-#define DW_DMMA_PANEL 0
-#endif
-constexpr bool DMMA_PANEL = DW_DMMA_PANEL != 0;
+constexpr int WARPS_PER_CTA = 4;   // register kernel
+constexpr int LL_WARPS = 14;       // left-looking kernel: one CTA of 14 warps per SM (448 threads x 128 registers)
 
 __device__ __forceinline__ double wvec_at(const omc_vec_t& v, int chain, int i, double dflt) {
   return v.ptr ? v.ptr[(long long)chain * v.chain_stride + i] : dflt;
@@ -63,167 +63,95 @@ __device__ __forceinline__ double shx(double v, int m) { return __shfl_xor_sync(
 
 #define TI(i, j) ((i) * ((i) + 1) / 2 + (j))
 
-__device__ __forceinline__ unsigned smem_addr(const void* q) { return (unsigned)__cvta_generic_to_shared(q); }
-__device__ __forceinline__ void wbar_init(unsigned long long* bar) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;\n" ::"r"(smem_addr(bar)));
-  asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-}
-__device__ __forceinline__ void wbar_expect(unsigned long long* bar, unsigned bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(smem_addr(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void wbar_wait(unsigned long long* bar, unsigned parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred P1;\n"
-      "DW_WAIT_LOOP:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n"
-      "@P1 bra DW_WAIT_DONE;\n"
-      "bra DW_WAIT_LOOP;\n"
-      "DW_WAIT_DONE:\n"
-      "}\n" ::"r"(smem_addr(bar)),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void wbulk(void* dst, const void* src, unsigned bytes, unsigned long long* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n" ::"r"(
-                   smem_addr(dst)),
-               "l"(src), "r"(bytes), "r"(smem_addr(bar))
-               : "memory");
+template <int... K, class F>
+__device__ __forceinline__ void static_for(std::integer_sequence<int, K...>, F f) {
+  (f(std::integral_constant<int, K>{}), ...);
 }
 
-// Shared-memory slab of one warp (STAGE): the rows of block row i hold columns 0 .. 8(i+1)-1 at a stride that is
-// 8 (mod 16) doubles, so the 16-byte tile reads of a quarter-warp (rows g, g+1) fall into disjoint bank groups.
-template <int PB>
-struct Slab {
-  __host__ __device__ static constexpr int stride(int i) { return 8 * (i + 1) + ((i & 1) ? 8 : 0); }
-  __host__ __device__ static constexpr int row_off(int i) {           // first double of block row i
-    // sum_{q<i} 8 * (8 (q+1) + 8 (q odd)) = 32 i (i+1) + 64 floor(i/2)
-    return 32 * i * (i + 1) + 64 * (i / 2);
-  }
-  static constexpr int G_OFF = row_off(PB);                           // g = X'Wy (8 PB doubles)
-  static constexpr int CEN_OFF = G_OFF + 8 * PB;                       // 2 x centre record beta_hat | c0 | rss0 | cnt (16 PB + 2 each):
-  static constexpr int CEN_LEN = 16 * PB + 2;                          //   the epilogue reads it after the NEXT chain's copies started
-  static constexpr int BAR_OFF = CEN_OFF + 2 * CEN_LEN;                // the mbarrier
-  static constexpr int DOUBLES = BAR_OFF + 2;
+// Per-chain inputs of the draw
+struct ChainIn {
+  const double* rec;   // sufficient-statistics record: G (p x p) | g (p) | ...
+  const double* P0;    // this chain's prior precision (null: identity)
+  double tau, lam, diag_scale;
+  bool dense;
 };
+__device__ __forceinline__ ChainIn chain_in(const omc_nn_dense_t& a, int chain) {
+  ChainIn c;
+  c.rec = a.stats.ptr + (long long)chain * a.stats.chain_stride;
+  c.P0 = a.prior_P.ptr ? a.prior_P.ptr + (long long)chain * a.prior_P.chain_stride : nullptr;
+  c.tau = wvec_at(a.tau, chain, 0, 1.0);
+  c.lam = wvec_at(a.lambda, chain, 0, 1.0);
+  c.diag_scale = a.mode == 1 ? 1.0 + a.ridge_rel : 1.0;
+  c.dense = a.prior_kind == OMC_MAT_DENSE;
+  return c;
+}
 
-// Sends the record of chain c on its way into the warp's slab: every lane issues the bulk copies of two rows of the
-// lower block triangle, lane 0 those of g and of the centre record and the expected byte count (the phase cannot
-// complete before lane 0 has arrived, whatever the order in which the copies land).  Whole warp calls this.
-template <int PB>
-__device__ __forceinline__ void slab_issue(const omc_nn_dense_t& a, int c, double* slab, unsigned long long* bar, int lane,
-                                           int slot) {
-  const double* rec = a.stats.ptr + (long long)c * a.stats.chain_stride;
-  constexpr int P = 8 * PB;
-#pragma unroll
-  for (int q = 0; q < (P + 31) / 32; ++q) {
-    const int r = lane + 32 * q;
-    if (r < P) {
-      const int i = r >> 3, gr = r & 7;
-      wbulk(slab + Slab<PB>::row_off(i) + gr * Slab<PB>::stride(i), rec + (long long)r * P, 64u * (unsigned)(i + 1), bar);
+// Elements [g][2kq], [g][2kq+1] of tile (i, j) of Q (sampler.py:180-186); rows / columns >= p are padded with the
+// identity.  VEC: p even and a 16-byte aligned record, so col + 1 < p whenever col < p.
+template <bool VEC>
+__device__ __forceinline__ void q_pair(const omc_nn_dense_t& a, const ChainIn& ci, int p, int i, int j, int g, int kq,
+                                       double& q0, double& q1) {
+  const int row = 8 * i + g, col = 8 * j + 2 * kq;
+  q0 = 0.0;
+  q1 = 0.0;
+  if (row < p) {
+    if (VEC) {
+      if (col < p) {
+        const double2 v = *reinterpret_cast<const double2*>(ci.rec + (long long)row * p + col);
+        q0 = ci.tau * v.x;
+        q1 = ci.tau * v.y;
+      }
+    } else {
+      if (col < p) q0 = ci.tau * ci.rec[(long long)row * p + col];
+      if (col + 1 < p) q1 = ci.tau * ci.rec[(long long)row * p + col + 1];
     }
-  }
-  if (lane == 0) {
-    unsigned total = 0;
-#pragma unroll
-    for (int i = 0; i < PB; ++i) total += 8u * 64u * (unsigned)(i + 1);
-    wbulk(slab + Slab<PB>::G_OFF, rec + (long long)P * P, 8u * P, bar);
-    total += 8u * P;
-    if (a.center.ptr) {
-      wbulk(slab + Slab<PB>::CEN_OFF + slot * Slab<PB>::CEN_LEN, a.center.ptr + (long long)c * a.center.chain_stride,
-            8u * (2 * P + 2), bar);
-      total += 8u * (2 * P + 2);
+    if (ci.dense) {
+      if (col < p) q0 = fma(ci.lam, ci.P0[(long long)row * p + col], q0);
+      if (col + 1 < p) q1 = fma(ci.lam, ci.P0[(long long)row * p + col + 1], q1);
+      if (i == j) {
+        if (row == col) q0 *= ci.diag_scale;
+        if (row == col + 1) q1 *= ci.diag_scale;
+      }
+    } else if (i == j) {
+      const double pr = a.prior_kind == OMC_MAT_DIAG ? ci.P0[row] : (ci.P0 ? ci.P0[0] : 1.0);
+      if (row == col) q0 = fma(ci.lam, pr, q0) * ci.diag_scale;
+      if (row == col + 1) q1 = fma(ci.lam, pr, q1) * ci.diag_scale;
     }
-    wbar_expect(bar, total);
+  } else if (i == j) {
+    if (row == col) q0 = 1.0;
+    if (row == col + 1) q1 = 1.0;
   }
 }
 
-// One chain, one warp.  STAGE: the tiles come from the warp's slab (already landed); as soon as they are in registers
-// lane 0 sends the record of `next_chain` (< 0: none) on its way.
-template <int PB, bool VEC, bool STAGE>
-__device__ __forceinline__ void warp_chain(const omc_nn_dense_t& a, int chain, double* slab, unsigned long long* bar,
-                                           int next_chain, int slot) {
-  const int lane = threadIdx.x & 31;
-  const int g = lane >> 2, kq = lane & 3, p = a.p;
-  const double* __restrict__ rec = a.stats.ptr + (long long)chain * a.stats.chain_stride;
-  const double tau = wvec_at(a.tau, chain, 0, 1.0);
-  const double lam = wvec_at(a.lambda, chain, 0, 1.0);
-  const bool solve_only = a.mode == 1;
-  const bool dense = a.prior_kind == OMC_MAT_DENSE;
-  const double* P0 = a.prior_P.ptr ? a.prior_P.ptr + (long long)chain * a.prior_P.chain_stride : nullptr;
-  const double diag_scale = solve_only ? 1.0 + a.ridge_rel : 1.0;
-
-  // ---- Q tiles (sampler.py:180-186); rows / columns >= p are padded with the identity
-  double T[PB * (PB + 1) / 2][2];
-#pragma unroll
-  for (int i = 0; i < PB; ++i)
-#pragma unroll
-    for (int j = 0; j <= i; ++j) {
-      const int row = 8 * i + g, col = 8 * j + 2 * kq;
-      double q0 = 0.0, q1 = 0.0;
-      if (row < p) {
-        if (STAGE) {                                     // p == 8 PB: every row / column is live
-          const double2 v = *reinterpret_cast<const double2*>(slab + Slab<PB>::row_off(i) + g * Slab<PB>::stride(i) + col);
-          q0 = tau * v.x;
-          q1 = tau * v.y;
-        } else if (VEC) {                                // p even, 16-byte aligned record: col + 1 < p whenever col < p
-          if (col < p) {
-            const double2 v = *reinterpret_cast<const double2*>(rec + (long long)row * p + col);
-            q0 = tau * v.x;
-            q1 = tau * v.y;
-          }
-        } else {
-          if (col < p) q0 = tau * rec[(long long)row * p + col];
-          if (col + 1 < p) q1 = tau * rec[(long long)row * p + col + 1];
-        }
-        if (dense) {
-          if (col < p) q0 = fma(lam, P0[(long long)row * p + col], q0);
-          if (col + 1 < p) q1 = fma(lam, P0[(long long)row * p + col + 1], q1);
-        } else if (i == j) {
-          const double pr = a.prior_kind == OMC_MAT_DIAG ? P0[row] : (P0 ? P0[0] : 1.0);
-          if (row == col) q0 = fma(lam, pr, q0) * diag_scale;
-          if (row == col + 1) q1 = fma(lam, pr, q1) * diag_scale;
-        }
-        if (dense && i == j) {
-          if (row == col) q0 *= diag_scale;
-          if (row == col + 1) q1 *= diag_scale;
-        }
-      } else if (i == j) {
-        if (row == col) q0 = 1.0;
-        if (row == col + 1) q1 = 1.0;
-      }
-      T[TI(i, j)][0] = q0;
-      T[TI(i, j)][1] = q1;
-    }
-  // ---- b = (lam*P0) mu0 + tau*g in row layout: w[i] = element 8i + g (replicated over kq)
-  double w[PB];
+// b = (lam*P0) mu0 + tau*g in row layout: w[i] = element 8i + g (replicated over kq)
+template <int PB>
+__device__ __forceinline__ void rhs_rows(const omc_nn_dense_t& a, const ChainIn& ci, int p, int chain, int g,
+                                         double (&w)[PB]) {
 #pragma unroll
   for (int i = 0; i < PB; ++i) {
     const int row = 8 * i + g;
     double bc = 0.0;
     if (row < p) {
       double sacc;
-      if (dense) {
+      if (ci.dense) {
         sacc = 0.0;
-        for (int j = 0; j < p; ++j) sacc += lam * P0[(long long)row * p + j] * wvec_at(a.mu0, chain, j, 0.0);
+        for (int j = 0; j < p; ++j) sacc += ci.lam * ci.P0[(long long)row * p + j] * wvec_at(a.mu0, chain, j, 0.0);
       } else {
-        const double pr = a.prior_kind == OMC_MAT_DIAG ? P0[row] : (P0 ? P0[0] : 1.0);
-        sacc = lam * pr * wvec_at(a.mu0, chain, row, 0.0);
+        const double pr = a.prior_kind == OMC_MAT_DIAG ? ci.P0[row] : (ci.P0 ? ci.P0[0] : 1.0);
+        sacc = ci.lam * pr * wvec_at(a.mu0, chain, row, 0.0);
       }
-      bc = sacc + tau * (STAGE ? slab[Slab<PB>::G_OFF + row] : rec[(long long)p * p + row]);
+      bc = sacc + ci.tau * ci.rec[(long long)p * p + row];
     }
     w[i] = bc;
   }
-  if (STAGE) {
-    __syncwarp();                                        // every lane has its tiles and g: the slab is free again
-    if (next_chain >= 0) {
-      asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");   // generic reads before async-proxy writes
-      slab_issue<PB>(a, next_chain, slab, bar, lane, slot ^ 1);
-    }
-  }
-  // ---- z: lane (g, kq) owns the pair of elements 8g + 2kq, +1 (Philox block = pair index, as in the other kernels)
-  double z0 = 0.0, z1 = 0.0;
-  if (!solve_only && g < PB) {
+}
+
+// z: lane (g, kq) owns the pair of elements 8g + 2kq, +1 (Philox block = pair index, as in the other kernels)
+template <int PB>
+__device__ __forceinline__ void draw_z(const omc_nn_dense_t& a, int p, int chain, int g, int kq, double& z0, double& z1) {
+  z0 = 0.0;
+  z1 = 0.0;
+  if (a.mode != 1 && g < PB) {
     const int e0 = 8 * g + 2 * kq;
     if (a.debug_z) {
       const double* dz = a.debug_z + (a.rng.sweep ? (long long)(*a.rng.sweep) : 0ll) * a.debug_sweep_stride + (long long)chain * p;
@@ -236,112 +164,53 @@ __device__ __forceinline__ void warp_chain(const omc_nn_dense_t& a, int chain, d
       if (e0 + 1 >= p) z1 = 0.0;
     }
   }
+}
 
-  // ---- factorisation by block columns
-  bool bad = false;
-#pragma unroll
-  for (int k = 0; k < PB; ++k) {
-    // DMMA_PANEL: the column operations of the 8 pivot stages run on the diagonal tile and on an identity tile E only
-    // (E becomes L_kk^-T); the tiles below follow as L(i,k) = T(i,k) E on the tensor pipe and the right-hand side as
-    // w_i -= L(i,k) w_k, instead of 8 serial rank-1 steps on every tile of the block column
-    constexpr int PANEL_END_OFF = DMMA_PANEL ? 1 : PB;
-    double E[2] = {(g == 2 * kq) ? 1.0 : 0.0, (g == 2 * kq + 1) ? 1.0 : 0.0};
+// The 8 pivot stages of block column k on the panel tiles tile(i), i = k .. PB-1 (tile(i) -> double[2] in accumulator
+// layout, tile(k) the diagonal one), with w riding along.  bad: a pivot was not positive (warp-uniform).
+template <int PB, class Tile>
+__device__ __forceinline__ void factor_panel(Tile tile, double (&w)[PB], int k, int g, int kq, bool& bad) {
 #pragma unroll 1
-    for (int jq = 0; jq < 4; ++jq) {
-      const bool own = kq == jq;
+  for (int jq = 0; jq < 4; ++jq) {
+    const bool own = kq == jq;
 #pragma unroll
-      for (int reg = 0; reg < 2; ++reg) {
-        const int jj = 2 * jq + reg;
-        const double piv = shf(T[TI(k, k)][reg], 4 * jj + jq);
-        if (!(piv > 0.0)) bad = true;
-        const double rd = wrsqrt(piv);
+    for (int reg = 0; reg < 2; ++reg) {
+      const int jj = 2 * jq + reg;
+      double* D = tile(k);
+      const double piv = shf(D[reg], 4 * jj + jq);
+      if (!(piv > 0.0)) bad = true;
+      const double rd = wrsqrt(piv);
 #pragma unroll
-        for (int i = k; i < (DMMA_PANEL ? k + PANEL_END_OFF : PB); ++i) T[TI(i, k)][reg] = own ? T[TI(i, k)][reg] * rd : T[TI(i, k)][reg];
-        if (DMMA_PANEL) E[reg] = own ? E[reg] * rd : E[reg];
-        const double wc = shf(w[k], 4 * jj) * rd;
-        if (g == jj) w[k] = wc;
-        double lc0 = shf(T[TI(k, k)][reg], 8 * kq + jq);        // L[2kq][jj]
-        double lc1 = shf(T[TI(k, k)][reg], 8 * kq + 4 + jq);    // L[2kq+1][jj]
-        if (!(2 * kq > jj)) lc0 = 0.0;
-        if (!(2 * kq + 1 > jj)) lc1 = 0.0;
-        if (DMMA_PANEL) {
-          const double le = shf(E[reg], 4 * g + jq);
-          E[0] = fma(-le, lc0, E[0]);
-          E[1] = fma(-le, lc1, E[1]);
-        }
+      for (int i = k; i < PB; ++i) tile(i)[reg] = own ? tile(i)[reg] * rd : tile(i)[reg];
+      const double wc = shf(w[k], 4 * jj) * rd;
+      if (g == jj) w[k] = wc;
+      double lc0 = shf(D[reg], 8 * kq + jq);        // L[2kq][jj]
+      double lc1 = shf(D[reg], 8 * kq + 4 + jq);    // L[2kq+1][jj]
+      if (!(2 * kq > jj)) lc0 = 0.0;
+      if (!(2 * kq + 1 > jj)) lc1 = 0.0;
 #pragma unroll
-        for (int i = k; i < (DMMA_PANEL ? k + PANEL_END_OFF : PB); ++i) {
-          const double lg = shf(T[TI(i, k)][reg], 4 * g + jq);  // L[8i + g][8k + jj]
-          T[TI(i, k)][0] = fma(-lg, lc0, T[TI(i, k)][0]);
-          T[TI(i, k)][1] = fma(-lg, lc1, T[TI(i, k)][1]);
-          if (i == k) {
-            if (g > jj) w[k] = fma(-lg, wc, w[k]);
-          } else {
-            w[i] = fma(-lg, wc, w[i]);
-          }
-        }
-        if (own && g == jj) T[TI(k, k)][reg] = rd;              // 1 / L_cc on the diagonal from here on
-      }
-    }
-    if (k + 1 < PB) {
-      if (DMMA_PANEL) {
-        // B fragments of E: lane (g, kq), step s needs E[4s + kq][g], held by lane (4s + kq, g >> 1), register g & 1
-        double Bf[2];
-#pragma unroll
-        for (int s = 0; s < 2; ++s) {
-          const int src = 4 * (4 * s + kq) + (g >> 1);
-          const double e0 = shf(E[0], src), e1 = shf(E[1], src);
-          Bf[s] = (g & 1) ? e1 : e0;
-        }
-        const double wk0 = shf(w[k], 4 * (2 * kq)), wk1 = shf(w[k], 4 * (2 * kq + 1));
-#pragma unroll
-        for (int i = k + 1; i < PB; ++i) {
-          double c0 = 0.0, c1 = 0.0;
-#pragma unroll
-          for (int s = 0; s < 2; ++s) {
-            const int src = 4 * g + 2 * s + (kq >> 1);
-            const double v0 = shf(T[TI(i, k)][0], src), v1 = shf(T[TI(i, k)][1], src);
-            wdmma(c0, c1, (kq & 1) ? v1 : v0, Bf[s]);
-          }
-          T[TI(i, k)][0] = c0;
-          T[TI(i, k)][1] = c1;
-          double t = fma(c0, wk0, c1 * wk1);
-          t += shx(t, 1);
-          t += shx(t, 2);
-          w[i] -= t;
+      for (int i = k; i < PB; ++i) {
+        double* T = tile(i);
+        const double lg = shf(T[reg], 4 * g + jq);  // L[8i + g][8k + jj]
+        T[0] = fma(-lg, lc0, T[0]);
+        T[1] = fma(-lg, lc1, T[1]);
+        if (i == k) {
+          if (g > jj) w[k] = fma(-lg, wc, w[k]);
+        } else {
+          w[i] = fma(-lg, wc, w[i]);
         }
       }
-      // panel tiles as operand fragments: f_s = element [g][4s + kq] (quad-local re-layout)
-      double R[PB][2];
-#pragma unroll
-      for (int i = k + 1; i < PB; ++i)
-#pragma unroll
-        for (int s = 0; s < 2; ++s) {
-          const int src = 4 * g + 2 * s + (kq >> 1);
-          const double v0 = shf(T[TI(i, k)][0], src), v1 = shf(T[TI(i, k)][1], src);
-          R[i][s] = (kq & 1) ? v1 : v0;
-        }
-#pragma unroll
-      for (int j = k + 1; j < PB; ++j)
-#pragma unroll
-        for (int i = j; i < PB; ++i) {
-          wdmma(T[TI(i, j)][0], T[TI(i, j)][1], -R[i][0], R[j][0]);
-          wdmma(T[TI(i, j)][0], T[TI(i, j)][1], -R[i][1], R[j][1]);
-        }
+      if (own && g == jj) D[reg] = rd;              // 1 / L_cc on the diagonal from here on
     }
   }
-  double* beta = a.beta + (long long)chain * p;
-  if (bad) {
-    if (solve_only) {                 // the centre may be any point: fall back to the origin
-      for (int c = lane; c < p; c += 32) beta[c] = 0.0;
-      return;
-    }
-    if (lane == 0 && a.status) atomicOr(&a.status[chain], OMC_STATUS_NOT_PD);
-    for (int c = lane; c < p; c += 32) beta[c] = nan("");
-    return;
-  }
+}
 
-  // ---- r = w + z in column layout; racc = per-lane partial sums (the g == 0 lanes start from r)
+// Backward solve L' x = w + z, x -> beta.  ldiag(j, c, l0, l1): L_jj[c][2kq], L_jj[c][2kq+1] (1 / L_cc on the
+// diagonal; only the lower triangle is used); loff(j, tc, r): L(j, tc)[g][2kq + r], tc < j.
+template <int PB, class Diag, class Off>
+__device__ __forceinline__ void back_solve(double* beta, int p, const double (&w)[PB], double z0, double z1, int g, int kq,
+                                           Diag ldiag, Off loff) {
+  // r = w + z in column layout; racc = per-lane partial sums (the g == 0 lanes start from r)
   double racc[PB][2];
 #pragma unroll
   for (int tc = 0; tc < PB; ++tc)
@@ -362,8 +231,8 @@ __device__ __forceinline__ void warp_chain(const omc_nn_dense_t& a, int chain, d
 #pragma unroll
       for (int reg = 1; reg >= 0; --reg) {
         const int c = 2 * cq + reg;
-        const double l0 = shf(T[TI(j, j)][0], 4 * c + kq);      // L_jj[c][2kq]   (1 / L_cc on the diagonal)
-        const double l1 = shf(T[TI(j, j)][1], 4 * c + kq);      // L_jj[c][2kq+1]
+        double l0, l1;
+        ldiag(j, c, l0, l1);
         const double mine = reg ? v1 * l1 : v0 * l0;
         const double xc = shf(mine, 4 * g + cq);
         if (kq == cq) { if (reg) v1 = xc; else v0 = xc; }
@@ -381,17 +250,32 @@ __device__ __forceinline__ void warp_chain(const omc_nn_dense_t& a, int chain, d
       const double xg = (g & 1) ? a1 : a0;                      // x[8j + g]
 #pragma unroll
       for (int tc = 0; tc < j; ++tc) {
-        racc[tc][0] = fma(-T[TI(j, tc)][0], xg, racc[tc][0]);
-        racc[tc][1] = fma(-T[TI(j, tc)][1], xg, racc[tc][1]);
+        racc[tc][0] = fma(-loff(j, tc, 0), xg, racc[tc][0]);
+        racc[tc][1] = fma(-loff(j, tc, 1), xg, racc[tc][1]);
       }
     }
   }
-  if (!a.center.ptr || !a.rss_out) return;
+}
 
-  // ---- rss(beta) = rss0 - 2 d'c0 + d'G d  (omc.h), d = beta - beta_hat; beta is read back through L2
+// Not positive definite: beta = 0 in solve-only mode (the centre may be any point: fall back to the origin), else NaN
+// and the status flag
+__device__ __forceinline__ void not_pd(const omc_nn_dense_t& a, int chain, double* beta, int lane) {
+  if (a.mode == 1) {
+    for (int c = lane; c < a.p; c += 32) beta[c] = 0.0;
+    return;
+  }
+  if (lane == 0 && a.status) atomicOr(&a.status[chain], OMC_STATUS_NOT_PD);
+  for (int c = lane; c < a.p; c += 32) beta[c] = nan("");
+}
+
+// rss(beta) = rss0 - 2 d'c0 + d'G d  (omc.h), d = beta - beta_hat; beta is read back through L2, G from the record
+// again (not as |L'd|^2 - lam d'P0 d, which would carry the factorisation's backward error, ~cond(Q))
+template <int PB, bool VEC>
+__device__ __forceinline__ void rss_epilogue(const omc_nn_dense_t& a, int p, int chain, const double* __restrict__ rec,
+                                             const double* beta, int lane) {
+  const int g = lane >> 2, kq = lane & 3;
   __syncwarp();
-  const double* cen = STAGE ? slab + Slab<PB>::CEN_OFF + slot * Slab<PB>::CEN_LEN
-                            : a.center.ptr + (long long)chain * a.center.chain_stride;
+  const double* cen = a.center.ptr + (long long)chain * a.center.chain_stride;
   double acc = 0.0;
   double dcol[PB][2], drow[PB];
 #pragma unroll
@@ -430,69 +314,235 @@ __device__ __forceinline__ void warp_chain(const omc_nn_dense_t& a, int chain, d
   if (lane == 0) a.rss_out[(long long)chain * a.stats.chain_stride] = cen[2 * p] + acc;
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Register kernel: one chain, one warp, the lower block triangle of Q in registers.
+template <int PB, bool VEC>
+__device__ __forceinline__ void warp_chain(const omc_nn_dense_t& a, int chain) {
+  const int lane = threadIdx.x & 31;
+  const int g = lane >> 2, kq = lane & 3, p = a.p;
+  const ChainIn ci = chain_in(a, chain);
+
+  double T[PB * (PB + 1) / 2][2];
+#pragma unroll
+  for (int i = 0; i < PB; ++i)
+#pragma unroll
+    for (int j = 0; j <= i; ++j) q_pair<VEC>(a, ci, p, i, j, g, kq, T[TI(i, j)][0], T[TI(i, j)][1]);
+  double w[PB];
+  rhs_rows<PB>(a, ci, p, chain, g, w);
+  double z0, z1;
+  draw_z<PB>(a, p, chain, g, kq, z0, z1);
+
+  // ---- factorisation by block columns, right-looking
+  bool bad = false;
+#pragma unroll
+  for (int k = 0; k < PB; ++k) {
+    factor_panel<PB>([&](int i) -> double* { return T[TI(i, k)]; }, w, k, g, kq, bad);
+    if (k + 1 < PB) {
+      // panel tiles as operand fragments: f_s = element [g][4s + kq] (quad-local re-layout)
+      double R[PB][2];
+#pragma unroll
+      for (int i = k + 1; i < PB; ++i)
+#pragma unroll
+        for (int s = 0; s < 2; ++s) {
+          const int src = 4 * g + 2 * s + (kq >> 1);
+          const double v0 = shf(T[TI(i, k)][0], src), v1 = shf(T[TI(i, k)][1], src);
+          R[i][s] = (kq & 1) ? v1 : v0;
+        }
+#pragma unroll
+      for (int j = k + 1; j < PB; ++j)
+#pragma unroll
+        for (int i = j; i < PB; ++i) {
+          wdmma(T[TI(i, j)][0], T[TI(i, j)][1], -R[i][0], R[j][0]);
+          wdmma(T[TI(i, j)][0], T[TI(i, j)][1], -R[i][1], R[j][1]);
+        }
+    }
+  }
+  double* beta = a.beta + (long long)chain * p;
+  if (bad) return not_pd(a, chain, beta, lane);
+  back_solve<PB>(
+      beta, p, w, z0, z1, g, kq,
+      [&](int j, int c, double& l0, double& l1) {
+        l0 = shf(T[TI(j, j)][0], 4 * c + kq);
+        l1 = shf(T[TI(j, j)][1], 4 * c + kq);
+      },
+      [&](int j, int tc, int r) { return T[TI(j, tc)][r]; });
+  if (a.center.ptr && a.rss_out) rss_epilogue<PB, VEC>(a, p, chain, ci.rec, beta, lane);
+}
+
 // resident CTAs (of 4 warps) per SM the register allocation aims at: 72 doubles of tiles per lane at PB = 8
 template <int PB>
 constexpr int ctas_per_sm() { return PB <= 2 ? 5 : (PB <= 4 ? 3 : 2); }
 
-template <int PB, bool VEC, bool STAGE>
+template <int PB, bool VEC>
 __global__ void __launch_bounds__(32 * WARPS_PER_CTA, ctas_per_sm<PB>()) nn_warp_draw_kernel(omc_nn_dense_t a) {
-  extern __shared__ __align__(16) double dsm[];
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const int n_warps = gridDim.x * WARPS_PER_CTA;
-  int chain = blockIdx.x * WARPS_PER_CTA + wid;
-  if (chain >= a.n_chains) return;                       // warp-uniform
-  if (!STAGE) {
-    for (; chain < a.n_chains; chain += n_warps) warp_chain<PB, VEC, false>(a, chain, nullptr, nullptr, -1, 0);
-    return;
+  const int chain = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5);
+  if (chain < a.n_chains) warp_chain<PB, VEC>(a, chain);   // warp-uniform
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Left-looking kernel.  Shared-memory slice of one warp: the PB(PB-1)/2 off-diagonal tiles of L full, then the PB-1
+// first diagonal tiles as packed lower triangles (36 doubles, element [r][c] at r(r+1)/2 + c, 1 / L_cc on the
+// diagonal); the last diagonal tile stays in registers.
+template <int PB>
+struct LeftSmem {
+  static constexpr int DIAG_OFF = 64 * (PB * (PB - 1) / 2);
+  static constexpr int DOUBLES = DIAG_OFF + 36 * (PB - 1);                // 2044 at PB = 8
+  __host__ __device__ static constexpr int off(int i, int j) { return 64 * (i * (i - 1) / 2 + j); }   // tile (i, j), i > j
+};
+// Position of element [r][c] inside an off-diagonal tile: pair 2f + s of fragment lane f = 4r + (c & 3), s = c >> 2,
+// so that a lane reads both of its operand fragments ([g][kq], [g][4 + kq]) as one 16-byte load.  XOR 2 on rows
+// r & 2: the 8-byte stores of one accumulator register by a half-warp (rows 4h .. 4h+3) then hit 16 distinct banks.
+__device__ __forceinline__ int lpos(int r, int c) { return (8 * r + 2 * (c & 3) + (c >> 2)) ^ (r & 2); }
+
+// FULL: p = 8 PB and a 16-byte aligned record (16-byte loads, every bound known at compile time); else any p of the
+// block count, element by element
+template <int PB, bool FULL>
+__device__ __forceinline__ void left_chain(const omc_nn_dense_t& a, int chain, int next_chain, double* sm) {
+  using S = LeftSmem<PB>;
+  constexpr bool VEC = FULL;
+  const int lane = threadIdx.x & 31;
+  const int g = lane >> 2, kq = lane & 3, p = FULL ? 8 * PB : a.p;
+  const ChainIn ci = chain_in(a, chain);
+
+  // the next chain's record (and centre record) on its way into L2 while this one runs; every byte of both is read
+  if (VEC && next_chain >= 0) {
+    const char* nrec = reinterpret_cast<const char*>(a.stats.ptr + (long long)next_chain * a.stats.chain_stride);
+    const unsigned bytes = 8u * (unsigned)(p * p + p);                   // p (p + 1) is even: a multiple of 16
+    const unsigned chunk = ((bytes + 32u * 16u - 1u) / (32u * 16u)) * 16u;
+    const unsigned o = chunk * (unsigned)lane;
+    if (o < bytes) {
+      const unsigned n = bytes - o < chunk ? bytes - o : chunk;
+      asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;\n" ::"l"(nrec + o), "r"(n) : "memory");
+    }
+    const double* ncen = a.center.ptr + (long long)next_chain * a.center.chain_stride;
+    if (lane == 0 && a.center.ptr && a.rss_out && (((unsigned long long)ncen) & 15ull) == 0)
+      asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;\n" ::"l"(ncen),
+                   "r"(16u * (unsigned)(p + 1))
+                   : "memory");
   }
-  double* slab = dsm + wid * Slab<PB>::DOUBLES;
-  unsigned long long* bar = reinterpret_cast<unsigned long long*>(slab + Slab<PB>::BAR_OFF);
-  if (lane == 0) wbar_init(bar);
-  __syncwarp();
-  slab_issue<PB>(a, chain, slab, bar, lane, 0);
-  unsigned parity = 0;
-  for (; chain < a.n_chains; chain += n_warps) {
-    wbar_wait(bar, parity);
-    parity ^= 1u;
+
+  double C[PB][2];   // block column k: C[i] = tile (i, k), i >= k
+  double w[PB];
+  rhs_rows<PB>(a, ci, p, chain, g, w);
+  __syncwarp();      // the previous chain's reads of the slice are done
+
+  bool bad = false;
+  // the steps are unrolled by hand: every register array must be indexed by constants
+  static_for(std::make_integer_sequence<int, PB>{}, [&](auto kc) {
+    constexpr int k = decltype(kc)::value;
+    // block column k from the record (in L2 by now): its latency overlaps the fragment reads and DMMAs below
+#pragma unroll
+    for (int i = k; i < PB; ++i) q_pair<VEC>(a, ci, p, i, k, g, kq, C[i][0], C[i][1]);
+    // C(i, k) -= L(i, j) L(k, j)', j < k: A = element [g][4s + kq] of L(i, j), B the same element of L(k, j)
+#pragma unroll
+    for (int j = 0; j < k; ++j) {
+      const int fr = (2 * lane) ^ (g & 2);
+      const double2 bk = *reinterpret_cast<const double2*>(sm + S::off(k, j) + fr);
+      wdmma(C[k][0], C[k][1], -bk.x, bk.x);
+      wdmma(C[k][0], C[k][1], -bk.y, bk.y);
+#pragma unroll
+      for (int i = k + 1; i < PB; ++i) {
+        const double2 ai = *reinterpret_cast<const double2*>(sm + S::off(i, j) + fr);
+        wdmma(C[i][0], C[i][1], -ai.x, bk.x);
+        wdmma(C[i][0], C[i][1], -ai.y, bk.y);
+      }
+    }
+    factor_panel<PB>([&](int i) -> double* { return C[i]; }, w, k, g, kq, bad);
+    if (k + 1 < PB) {
+#pragma unroll
+      for (int i = k + 1; i < PB; ++i) {
+        sm[S::off(i, k) + lpos(g, 2 * kq)] = C[i][0];
+        sm[S::off(i, k) + lpos(g, 2 * kq + 1)] = C[i][1];
+      }
+      double* dt = sm + S::DIAG_OFF + 36 * k + g * (g + 1) / 2;
+      if (2 * kq <= g) dt[2 * kq] = C[k][0];
+      if (2 * kq + 1 <= g) dt[2 * kq + 1] = C[k][1];
+      __syncwarp();
+    }
+  });
+  double* beta = a.beta + (long long)chain * p;
+  if (bad) return not_pd(a, chain, beta, lane);
+  double z0, z1;
+  draw_z<PB>(a, p, chain, g, kq, z0, z1);
+  back_solve<PB>(
+      beta, p, w, z0, z1, g, kq,
+      [&](int j, int c, double& l0, double& l1) {
+        if (j == PB - 1) {
+          l0 = shf(C[PB - 1][0], 4 * c + kq);
+          l1 = shf(C[PB - 1][1], 4 * c + kq);
+        } else {                                      // above the diagonal (unused): another element of the tile
+          const double* dt = sm + S::DIAG_OFF + 36 * j + c * (c + 1) / 2 + 2 * kq;
+          l0 = dt[0];
+          l1 = dt[1];
+        }
+      },
+      [&](int j, int tc, int r) { return sm[S::off(j, tc) + lpos(g, 2 * kq + r)]; });
+  if (a.center.ptr && a.rss_out) rss_epilogue<PB, VEC>(a, p, chain, ci.rec, beta, lane);
+}
+
+template <int PB, bool FULL>
+__global__ void __launch_bounds__(32 * LL_WARPS, 1) nn_left_draw_kernel(omc_nn_dense_t a) {
+  extern __shared__ __align__(16) double dsm[];
+  const int wid = threadIdx.x >> 5;
+  const int n_warps = gridDim.x * LL_WARPS;
+  double* sm = dsm + wid * LeftSmem<PB>::DOUBLES;
+  for (int chain = blockIdx.x * LL_WARPS + wid; chain < a.n_chains; chain += n_warps) {   // warp-uniform
     const int nxt = chain + n_warps;
-    warp_chain<PB, VEC, true>(a, chain, slab, bar, nxt < a.n_chains ? nxt : -1, (int)(parity ^ 1u));
+    left_chain<PB, FULL>(a, chain, nxt < a.n_chains ? nxt : -1, sm);
   }
 }
 
+bool vec_ok(const omc_nn_dense_t& a) {
+  return (a.p & 1) == 0 && (((unsigned long long)a.stats.ptr) & 15ull) == 0 && (a.stats.chain_stride & 1) == 0;
+}
+
 template <int PB>
-int launch_pb(const omc_nn_dense_t& a, cudaStream_t st) {
-  const bool vec = (a.p & 1) == 0 && (((unsigned long long)a.stats.ptr) & 15ull) == 0 && (a.stats.chain_stride & 1) == 0;
-  const bool cen_ok = !a.center.ptr || ((((unsigned long long)a.center.ptr) & 15ull) == 0 && (a.center.chain_stride & 1) == 0 &&
-                                         a.center.chain_stride >= 2 * a.p + 2);
-  const bool stage = vec && cen_ok && a.p == 8 * PB && PB >= 7;       // packed rows; below ~56 columns the direct loads measured faster
-  // persistent warps: as many CTAs of 4 warps as are resident at once (two per SM at PB = 8: 254 registers per thread)
-  const int ctas_needed = (a.n_chains + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
-  const int ctas_max = ctas_per_sm<PB>() * omc_sm_count();
-  const unsigned grid = (unsigned)((ctas_needed < ctas_max || !stage) ? ctas_needed : ctas_max);   // persistent only when staged
-  if (stage) {
-    const int smem = WARPS_PER_CTA * Slab<PB>::DOUBLES * (int)sizeof(double);
-    OMC_CHECK_CUDA(cudaFuncSetAttribute(nn_warp_draw_kernel<PB, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    nn_warp_draw_kernel<PB, true, true><<<grid, 32 * WARPS_PER_CTA, smem, st>>>(a);
-  } else if (vec) {
-    nn_warp_draw_kernel<PB, true, false><<<grid, 32 * WARPS_PER_CTA, 0, st>>>(a);
-  } else {
-    nn_warp_draw_kernel<PB, false, false><<<grid, 32 * WARPS_PER_CTA, 0, st>>>(a);
-  }
+int launch_warp_pb(const omc_nn_dense_t& a, cudaStream_t st) {
+  const unsigned grid = (unsigned)((a.n_chains + WARPS_PER_CTA - 1) / WARPS_PER_CTA);
+  if (vec_ok(a)) nn_warp_draw_kernel<PB, true><<<grid, 32 * WARPS_PER_CTA, 0, st>>>(a);
+  else nn_warp_draw_kernel<PB, false><<<grid, 32 * WARPS_PER_CTA, 0, st>>>(a);
   OMC_LAUNCH_CHECK();
   return 0;
+}
+
+template <int PB, bool FULL>
+int launch_left(const omc_nn_dense_t& a, unsigned grid, cudaStream_t st) {
+  const int smem = LL_WARPS * LeftSmem<PB>::DOUBLES * (int)sizeof(double);
+  OMC_CHECK_CUDA(cudaFuncSetAttribute(nn_left_draw_kernel<PB, FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  nn_left_draw_kernel<PB, FULL><<<grid, 32 * LL_WARPS, smem, st>>>(a);
+  OMC_LAUNCH_CHECK();
+  return 0;
+}
+
+template <int PB>
+int launch_left_pb(const omc_nn_dense_t& a, cudaStream_t st) {
+  // persistent warps: one CTA of 14 warps per SM
+  const int ctas_needed = (a.n_chains + LL_WARPS - 1) / LL_WARPS;
+  const int sms = omc_sm_count();
+  const unsigned grid = (unsigned)(ctas_needed < sms ? ctas_needed : sms);
+  return vec_ok(a) && a.p == 8 * PB ? launch_left<PB, true>(a, grid, st) : launch_left<PB, false>(a, grid, st);
 }
 
 }  // namespace
 
 int omc_launch_warp_draw(const omc_nn_dense_t& a, cudaStream_t st) {
   switch ((a.p + 7) / 8) {
-    case 1: return launch_pb<1>(a, st);
-    case 2: return launch_pb<2>(a, st);
-    case 3: return launch_pb<3>(a, st);
-    case 4: return launch_pb<4>(a, st);
-    case 5: return launch_pb<5>(a, st);
-    case 6: return launch_pb<6>(a, st);
-    case 7: return launch_pb<7>(a, st);
-    default: return launch_pb<8>(a, st);
+    case 1: return launch_warp_pb<1>(a, st);
+    case 2: return launch_warp_pb<2>(a, st);
+    case 3: return launch_warp_pb<3>(a, st);
+    case 4: return launch_warp_pb<4>(a, st);
+    case 5: return launch_warp_pb<5>(a, st);
+    case 6: return launch_warp_pb<6>(a, st);
+    case 7: return launch_warp_pb<7>(a, st);
+    default: return launch_warp_pb<8>(a, st);
+  }
+}
+
+int omc_launch_left_draw(const omc_nn_dense_t& a, cudaStream_t st) {
+  switch ((a.p + 7) / 8) {
+    case 5: return launch_left_pb<5>(a, st);
+    case 6: return launch_left_pb<6>(a, st);
+    case 7: return launch_left_pb<7>(a, st);
+    default: return launch_left_pb<8>(a, st);
   }
 }

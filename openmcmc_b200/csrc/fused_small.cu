@@ -89,8 +89,10 @@ __device__ __forceinline__ void op_quadform(const omc_quadform_t& a, int c, int 
   }
 }
 
+// 7 CTAs per SM (<= 72 registers): the 1024 CTAs of 4096 chains at 32 lanes per chain run in one wave on 148 SMs
+// (6 at the 80 registers the compiler picks unbounded: 1.15 waves)
 template <int LPC>
-__global__ void __launch_bounds__(FS_THREADS) fused_small_kernel(const __grid_constant__ omc_fused_small_t a) {
+__global__ void __launch_bounds__(FS_THREADS, 7) fused_small_kernel(const __grid_constant__ omc_fused_small_t a) {
   const long long gtid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long nthreads = (long long)gridDim.x * blockDim.x;
   const long long chain_ll = gtid / LPC;

@@ -13,5 +13,7 @@ enum OmcMatKind { OMC_MAT_EYE = 0, OMC_MAT_DIAG = 1, OMC_MAT_DENSE = 2 };
 #include <cuda_runtime.h>
 int omc_launch_blocked_draw(const omc_nn_dense_t& a, cudaStream_t st);
 long long omc_blocked_workspace_doubles(int p);
-// dense_warp.cu: one warp per chain, Q in registers (p <= 64, no probes)
+// dense_warp.cu: one warp per chain (p <= 64, no probes); Q in registers, or left-looking with L in shared memory
+// (32 < p <= 64)
 int omc_launch_warp_draw(const omc_nn_dense_t& a, cudaStream_t st);
+int omc_launch_left_draw(const omc_nn_dense_t& a, cudaStream_t st);

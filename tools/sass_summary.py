@@ -4,7 +4,8 @@
     python tools/sass_summary.py > profiles/r02_sass_summary.txt
 
 Counts the mnemonics that prove which hardware paths the kernels use: DMMA (FP64 tensor pipe; tcgen05 has no f64 kind),
-UBLKCP (1-D bulk copies through the TMA engine), SYNCS (mbarrier), LDGSTS, MUFU.RSQ64H, MEMBAR, and the absence of
+UBLKCP (1-D bulk copies through the TMA engine), SYNCS (mbarrier), LDGSTS, MUFU.RSQ64H, MEMBAR, local-memory traffic
+(LDL / STL: spills), and the absence of
 UTMALDG / UTCxMMA / LDTM (no 2-D tensor maps, no tcgen05: the tiles are 1-D and the arithmetic is fp64).
 """
 import collections
@@ -17,7 +18,7 @@ import tempfile
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "openmcmc_b200", "libomc.so")
 KEYS = ["DMMA", "DFMA", "DMUL", "DADD", "MUFU.RSQ64H", "MUFU.RCP64H", "UBLKCP", "SYNCS", "LDGSTS", "MEMBAR", "SHFL", "BAR.SYNC",
-        "ATOM", "RED", "LDS", "STS", "LDG", "STG", "UTMALDG", "UTCHMMA", "UTCQMMA", "LDTM", "HMMA", "IMMA"]
+        "ATOM", "RED", "LDS", "STS", "LDG", "STG", "LDL", "STL", "UTMALDG", "UTCHMMA", "UTCQMMA", "LDTM", "HMMA", "IMMA"]
 
 
 def main():
@@ -53,7 +54,7 @@ def main():
             short = re.sub(r"\(anonymous namespace\)::", "", short)
             short = re.sub(r"\(.*", "", short)[-90:]
             print(f"   {c['_n']:6d}  {short:90s} " + " ".join(f"{k}={c[k]}" for k in KEYS if c[k] and k in
-                                                                  ("DMMA", "UBLKCP", "SYNCS", "LDGSTS", "MUFU.RSQ64H", "MEMBAR", "BAR.SYNC")))
+                                                                  ("DMMA", "UBLKCP", "SYNCS", "LDGSTS", "MUFU.RSQ64H", "MEMBAR", "BAR.SYNC", "LDL", "STL")))
 
 
 if __name__ == "__main__":
