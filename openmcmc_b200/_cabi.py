@@ -359,7 +359,7 @@ EXTRA_STRUCTS["omc_rj_mmala_t"] = RJMmala
 
 
 def lib_path() -> str:
-    """In-tree libomc.so; OMC_LIB overrides it (tools/tune_reg_pass.sh and tools/ab_dense_draw.sh time builds with it)."""
+    """In-tree libomc.so; OMC_LIB overrides it (tools/ab_dense_draw.sh times builds with it)."""
     return os.environ.get("OMC_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), _LIB_NAME)
 
 

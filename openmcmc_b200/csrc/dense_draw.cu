@@ -10,7 +10,6 @@
 #include "omc_common.cuh"
 #include "omc_internal.h"
 #include "omc_special.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -123,7 +122,7 @@ __global__ void __launch_bounds__(DD_THREADS) nn_truncated_scan_kernel(omc_nn_de
 // The previous CTA-wide kernel (256 threads, matrix in shared memory, 3 barriers per column) took 0.66 ms for the
 // 4096 chains of C2, a fifth of the sweep once the pass over X became a pure stream.
 template <int PR>
-__global__ void __launch_bounds__((PR < 32 ? 32 : PR), (PR == 64 ? 5 : (PR == 32 ? 10 : 16))) nn_dense_draw_kernel(omc_nn_dense_t a) {
+__global__ void __launch_bounds__((PR < 32 ? 32 : PR), (PR == 32 ? 10 : 16)) nn_dense_draw_kernel(omc_nn_dense_t a) {
   constexpr int NT = PR < 32 ? 32 : PR;
   constexpr int LD = PR + 2;                 // column stride (doubles): 16-byte aligned columns
   extern __shared__ __align__(16) double sm[];
@@ -370,20 +369,15 @@ extern "C" int omc_nn_dense_draw(const omc_nn_dense_t* args, void* stream) {
   // p <= 64 without probes: one warp per chain (dense_warp.cu), the left-looking kernel with the factor in shared
   // memory above LEFT_MIN_P, Q in registers below.  Probes (Q, b, L, mu of the parity tests) go through the kernels
   // that keep the factor addressable: one thread per column (p <= 32) or the blocked Cholesky (dense_blocked.cu), which
-  // also serves 64 < p <= 512.  OMC_DENSE_DRAW_IMPL = left | warp | columns | blocked forces one of them where it
-  // applies (A/B timing, tools/perf_dense_draw.py).
-  static const char impl = [] { const char* e = getenv("OMC_DENSE_DRAW_IMPL"); return e ? e[0] : '\0'; }();
+  // also serves 64 < p <= 512.
   const bool probes = args->probe_Q || args->probe_b || args->probe_L || args->probe_mu;
   if (p <= 64 && !probes) {
-    if ((impl == '\0' && p > LEFT_MIN_P) || (impl == 'l' && p > 32)) return omc_launch_left_draw(*args, (cudaStream_t)stream);
-    if (impl == '\0' || impl == 'w') return omc_launch_warp_draw(*args, (cudaStream_t)stream);
+    if (p > LEFT_MIN_P) return omc_launch_left_draw(*args, (cudaStream_t)stream);
+    return omc_launch_warp_draw(*args, (cudaStream_t)stream);
   }
-  if (impl != 'b' || p <= 0) {
-    if (p <= 8) return launch_dense_draw<8>(*args, (cudaStream_t)stream);
-    if (p <= 16) return launch_dense_draw<16>(*args, (cudaStream_t)stream);
-    if (p <= 32) return launch_dense_draw<32>(*args, (cudaStream_t)stream);
-    if (impl == 'c' && p <= 64) return launch_dense_draw<64>(*args, (cudaStream_t)stream);
-  }
+  if (p <= 8) return launch_dense_draw<8>(*args, (cudaStream_t)stream);
+  if (p <= 16) return launch_dense_draw<16>(*args, (cudaStream_t)stream);
+  if (p <= 32) return launch_dense_draw<32>(*args, (cudaStream_t)stream);
   return omc_launch_blocked_draw(*args, (cudaStream_t)stream);
 }
 

@@ -538,9 +538,8 @@ int omc_launch_warp_draw(const omc_nn_dense_t& a, cudaStream_t st) {
   }
 }
 
-int omc_launch_left_draw(const omc_nn_dense_t& a, cudaStream_t st) {
+int omc_launch_left_draw(const omc_nn_dense_t& a, cudaStream_t st) {   // 40 < p <= 64 (dense_draw.cu: LEFT_MIN_P)
   switch ((a.p + 7) / 8) {
-    case 5: return launch_left_pb<5>(a, st);
     case 6: return launch_left_pb<6>(a, st);
     case 7: return launch_left_pb<7>(a, st);
     default: return launch_left_pb<8>(a, st);

@@ -981,9 +981,6 @@ int omc_mmala(const omc_mmala_t* a, void* stream) {
                               t.kind == OMC_TERM_UNIFORM_RESPONSE ||
                               (t.kind == OMC_TERM_NORMAL_RESPONSE && t.mat_kind != OMC_MAT_DENSE));
   }
-#ifdef OMC_MMALA_NO_DIAG
-  separable = false;
-#endif
   if (n <= 32 && separable) {   // diagonal Hessian: one element per lane, no matrix
     const size_t smem_d = (size_t)MD_WARPS * 2 * n * sizeof(double);
     mmala_diag_kernel<<<(a->model.n_chains + MD_WARPS - 1) / MD_WARPS, MD_WARPS * 32, smem_d, (cudaStream_t)stream>>>(*a);

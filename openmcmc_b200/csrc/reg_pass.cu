@@ -26,24 +26,10 @@
 
 namespace {
 
-// tuning knobs (overridable with -D for tools/tune_reg_pass.sh; defaults = measured best, see profiles/)
-#ifndef OMC_RP_KC
-#define OMC_RP_KC 64
-#endif
-#ifndef OMC_RP_NSTAGE
-#define OMC_RP_NSTAGE 3
-#endif
-#ifndef OMC_RP_TG
-#define OMC_RP_TG 1        // tile groups for PB >= 5 (1: every warp owns all tiles, 254 regs; 2: 18 tiles per warp)
-#endif
-#ifndef OMC_RP_MINBLOCKS
-#define OMC_RP_MINBLOCKS ((OMC_RP_TG == 1) ? 2 : 3)
-#endif
-#ifndef OMC_RP_USE_BULK
-#define OMC_RP_USE_BULK 1  // stage rows with cp.async.bulk (TMA engine) when shape/alignment allow
-#endif
-constexpr int KC = OMC_RP_KC;          // rows per pipeline stage
-constexpr int NSTAGE = OMC_RP_NSTAGE;  // pipeline stages
+// measured best (profiles/r01_reg_pass_loader_variants.txt)
+constexpr int KC = 64;             // rows per pipeline stage
+constexpr int NSTAGE = 3;          // pipeline stages
+constexpr int MINBLOCKS_WIDE = 2;  // CTAs per SM for the SYRK at PB >= 5 (every warp owns all tiles: 254 registers)
 constexpr int NWARP = 4;
 constexpr int NTHREADS = NWARP * 32;
 
@@ -110,14 +96,11 @@ struct Cfg {
   static constexpr int LD = 8 * PB + 4;  // padded row stride (doubles): (2g + 8k) mod 32 banks are distinct per phase
   static constexpr int STAGE_DOUBLES = KC * LD + 2 * KC;  // X tile | y | w
   static constexpr int NT = PB * (PB + 1) / 2;             // lower-triangle 8x8 tiles
-  static constexpr int TG = (PB >= 5) ? OMC_RP_TG : 1;     // tile groups (warps sharing the same rows)
   // chunked layout of the bulk path: a stage = 4 contiguous chunks of RC rows (one bulk copy each, rows packed at
   // stride 8*PB), chunk q shifted by 4 doubles so that the 4 k-lanes (one row from each chunk) hit distinct banks
   static constexpr int RC = KC / 4;
   static constexpr int CH = RC * 8 * PB + 4;
-  static constexpr int RG = NWARP / TG;                    // row groups
-  static constexpr int NTG = (NT + TG - 1) / TG;           // tiles per group
-  static constexpr int RED_DOUBLES = NWARP * (NTG * 64 + 8 * PB + 2);
+  static constexpr int RED_DOUBLES = NWARP * (NT * 64 + 8 * PB + 2);
   static constexpr int SMEM_DOUBLES = (NSTAGE * STAGE_DOUBLES > RED_DOUBLES) ? NSTAGE * STAGE_DOUBLES : RED_DOUBLES;
   static constexpr int BYTES = SMEM_DOUBLES * 8 + 64;  // + mbarriers
 };
@@ -127,7 +110,7 @@ struct Cfg {
 template <int PB, bool WEIGHTED, bool SYRK = true>
 struct Worker {
   using C = Cfg<PB>;
-  double acc[C::NTG][2];
+  double acc[C::NT][2];
   double gacc[PB];
   double bfrag[PB];
   double rss, cnt;
@@ -138,7 +121,7 @@ struct Worker {
     g = lane >> 2;
     kq = lane & 3;
 #pragma unroll
-    for (int t = 0; t < C::NTG; ++t) acc[t][0] = acc[t][1] = 0.0;
+    for (int t = 0; t < C::NT; ++t) acc[t][0] = acc[t][1] = 0.0;
 #pragma unroll
     for (int jb = 0; jb < PB; ++jb) {
       gacc[jb] = 0.0;
@@ -149,16 +132,14 @@ struct Worker {
     cnt = 0.0;
   }
 
-  // one stage = KC rows; row group `rg` takes k-steps (4 rows each) rg, rg+RG, ...; tile group G its share of tiles
-  template <int G, bool CHUNKED>
-  __device__ __forceinline__ void stage(const double* Xs, int rg) {
+  // one stage = KC rows; warp w takes k-steps (4 rows each) w, w+NWARP, ...
+  template <bool CHUNKED>
+  __device__ __forceinline__ void stage(const double* Xs, int w) {
     constexpr int LD = C::LD;
-    constexpr bool DO_G = SYRK && (G == 0);
-    constexpr bool DO_RSS = !SYRK || (G == C::TG - 1);
     const double* ys = Xs + KC * LD;
     const double* ws = ys + KC;
 #pragma unroll 2
-    for (int ks = rg; ks < KC / 4; ks += (SYRK ? C::RG : NWARP)) {
+    for (int ks = w; ks < KC / 4; ks += NWARP) {
       // padded layout: row 4ks+kq at stride LD ; chunked layout: row ks of chunk kq
       const int r = CHUNKED ? kq * C::RC + ks : 4 * ks + kq;
       const double* xr = CHUNKED ? Xs + kq * C::CH + ks * (8 * PB) + g : Xs + r * LD + g;
@@ -175,21 +156,21 @@ struct Worker {
 #pragma unroll
         for (int jb = 0; jb < PB; ++jb) bf[jb] = af[jb];
       }
-      // SYRK tiles of this group (lower triangle of the 8x8-block grid, row-major enumeration)
+      // SYRK tiles (lower triangle of the 8x8-block grid, row-major enumeration)
       if (SYRK) {
 #pragma unroll
         for (int i = 0; i < PB; ++i)
 #pragma unroll
           for (int j = 0; j <= i; ++j) {
             const int t = i * (i + 1) / 2 + j;
-            if (t / C::NTG == G) dmma884(acc[t - G * C::NTG][0], acc[t - G * C::NTG][1], af[i], bf[j]);
+            // t < NT always holds; without the test the compiler lays out the PB = 1 kernels differently from the
+            // measured build (profiles/r01_reg_pass_loader_variants.txt)
+            if (t < C::NT) dmma884(acc[t][0], acc[t][1], af[i], bf[j]);
           }
-      }
-      if (DO_G) {  // X' W y
 #pragma unroll
-        for (int jb = 0; jb < PB; ++jb) gacc[jb] = fma(bf[jb], yv, gacc[jb]);
+        for (int jb = 0; jb < PB; ++jb) gacc[jb] = fma(bf[jb], yv, gacc[jb]);   // X' W y
       }
-      if (DO_RSS) {  // residual of the 4 rows of this k-step
+      {  // residual of the 4 rows of this k-step
         double dot = 0.0, dot1 = 0.0;   // two chains of fused multiply-adds (the residual-only pass has no DMMA to hide them)
 #pragma unroll
         for (int jb = 0; jb < PB; jb += 2) {
@@ -213,14 +194,13 @@ struct Worker {
 //               queue behind LDGSTS; the < KC-row tail is staged synchronously.
 // BULK = false: generic cp.async (LDGSTS) path with zero-fill into the padded layout, any p / alignment.
 template <int PB, bool WEIGHTED, bool BULK, bool SYRK>
-__global__ void __launch_bounds__(NTHREADS, (PB > 4 && SYRK) ? OMC_RP_MINBLOCKS : 4) reg_pass_kernel(RegPassArgs a) {
+__global__ void __launch_bounds__(NTHREADS, (PB > 4 && SYRK) ? MINBLOCKS_WIDE : 4) reg_pass_kernel(RegPassArgs a) {
   using C = Cfg<PB>;
   constexpr int LD = C::LD;
   extern __shared__ __align__(16) double smem[];
 
   const int chain = blockIdx.y, split = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int tg = warp % C::TG, rg = warp / C::TG;
   const int p = a.p, n = a.n;
   const int row0 = split * a.rows_per_split;
   const int row1 = min(n, row0 + a.rows_per_split);
@@ -322,9 +302,7 @@ __global__ void __launch_bounds__(NTHREADS, (PB > 4 && SYRK) ? OMC_RP_MINBLOCKS 
       issue_stage(st + NSTAGE - 1);
     }
     const double* Xs = smem + (st % NSTAGE) * C::STAGE_DOUBLES;
-    if (!SYRK) wk.template stage<0, BULK>(Xs, warp);   // residual-only: every warp is a row group of its own
-    else if (C::TG == 1 || tg == 0) wk.template stage<0, BULK>(Xs, rg);
-    else wk.template stage<C::TG - 1, BULK>(Xs, rg);
+    wk.template stage<BULK>(Xs, warp);
   }
   if (!BULK) cp_async_wait<0>();
   __syncthreads();
@@ -342,9 +320,7 @@ __global__ void __launch_bounds__(NTHREADS, (PB > 4 && SYRK) ? OMC_RP_MINBLOCKS 
       if (WEIGHTED) ys[KC + r] = (r < valid) ? wc[r_base + r] : 0.0;
     }
     __syncthreads();
-    if (!SYRK) wk.template stage<0, true>(Xs, warp);
-    else if (C::TG == 1 || tg == 0) wk.template stage<0, true>(Xs, rg);
-    else wk.template stage<C::TG - 1, true>(Xs, rg);
+    wk.template stage<true>(Xs, warp);
     __syncthreads();
   }
   if (!SYRK) {
@@ -371,12 +347,12 @@ __global__ void __launch_bounds__(NTHREADS, (PB > 4 && SYRK) ? OMC_RP_MINBLOCKS 
     return;
   }
 
-  // ---- combine the row groups through shared memory (per warp: tiles | g | rss, cnt)
-  constexpr int WREC = C::NTG * 64 + 8 * PB + 2;
+  // ---- combine the warps through shared memory (per warp: tiles | g | rss, cnt)
+  constexpr int WREC = C::NT * 64 + 8 * PB + 2;
   double* red = smem + warp * WREC;
   const int g = lane >> 2, kq = lane & 3;
 #pragma unroll
-  for (int t = 0; t < C::NTG; ++t) {
+  for (int t = 0; t < C::NT; ++t) {
     red[t * 64 + 2 * lane] = wk.acc[t][0];
     red[t * 64 + 2 * lane + 1] = wk.acc[t][1];
   }
@@ -385,7 +361,7 @@ __global__ void __launch_bounds__(NTHREADS, (PB > 4 && SYRK) ? OMC_RP_MINBLOCKS 
     double v = wk.gacc[jb];
     v += omc_shfl_xor(v, 1);
     v += omc_shfl_xor(v, 2);
-    if (kq == 0) red[C::NTG * 64 + 8 * jb + g] = v;
+    if (kq == 0) red[C::NT * 64 + 8 * jb + g] = v;
   }
   {
     // lanes sharing kq hold identical copies of each row's residual -> keep the g == 0 lanes only
@@ -393,27 +369,24 @@ __global__ void __launch_bounds__(NTHREADS, (PB > 4 && SYRK) ? OMC_RP_MINBLOCKS 
     r = omc_warp_sum(r);
     c = omc_warp_sum(c);
     if (lane == 0) {
-      red[C::NTG * 64 + 8 * PB] = r;
-      red[C::NTG * 64 + 8 * PB + 1] = c;
+      red[C::NT * 64 + 8 * PB] = r;
+      red[C::NT * 64 + 8 * PB + 1] = c;
     }
   }
   __syncthreads();
 
-  if (rg == 0) {  // one writer warp per tile group
+  if (warp == 0) {  // one writer warp sums the four warps
     const int rec = p * p + p + 2;
     double* o = a.out + ((long long)chain * a.n_split + split) * rec;
-    const double* base = smem + tg * WREC;  // warp index of (tg, rg) is rg*TG + tg
 #pragma unroll
     for (int i = 0; i < PB; ++i)
 #pragma unroll
       for (int j = 0; j <= i; ++j) {
         const int t = i * (i + 1) / 2 + j;
-        if (t / C::NTG != tg) continue;
-        const int tl = t - tg * C::NTG;
 #pragma unroll
         for (int e = 0; e < 2; ++e) {
           double v = 0.0;
-          for (int q = 0; q < C::RG; ++q) v += base[q * C::TG * WREC + tl * 64 + 2 * lane + e];
+          for (int q = 0; q < NWARP; ++q) v += smem[q * WREC + t * 64 + 2 * lane + e];
           const int rr = 8 * i + g, cc = 8 * j + 2 * kq + e;
           if (rr < p && cc < p) {
             o[rr * p + cc] = v;
@@ -421,18 +394,16 @@ __global__ void __launch_bounds__(NTHREADS, (PB > 4 && SYRK) ? OMC_RP_MINBLOCKS 
           }
         }
       }
-    if (tg == 0) {
-      for (int c = lane; c < 8 * PB; c += 32) {
-        double v = 0.0;
-        for (int q = 0; q < C::RG; ++q) v += base[q * C::TG * WREC + C::NTG * 64 + c];
-        if (c < p) o[p * p + c] = v;
-      }
+    for (int c = lane; c < 8 * PB; c += 32) {
+      double v = 0.0;
+      for (int q = 0; q < NWARP; ++q) v += smem[q * WREC + C::NT * 64 + c];
+      if (c < p) o[p * p + c] = v;
     }
-    if (tg == C::TG - 1 && lane == 0) {
+    if (lane == 0) {
       double r = 0.0, c = 0.0;
-      for (int q = 0; q < C::RG; ++q) {
-        r += base[q * C::TG * WREC + C::NTG * 64 + 8 * PB];
-        c += base[q * C::TG * WREC + C::NTG * 64 + 8 * PB + 1];
+      for (int q = 0; q < NWARP; ++q) {
+        r += smem[q * WREC + C::NT * 64 + 8 * PB];
+        c += smem[q * WREC + C::NT * 64 + 8 * PB + 1];
       }
       o[p * p + p] = r;
       o[p * p + p + 1] = WEIGHTED ? c : (double)nrows;
@@ -467,7 +438,7 @@ template <int PB, bool SYRK>
 int launch_pb(const RegPassArgs& a, bool weighted, cudaStream_t st) {
   // bulk (TMA-engine) copies need fully packed rows (p == 8*PB) and 16-byte aligned chunk starts for X, y and w
   auto al16 = [](const void* q) { return (((unsigned long long)q) & 15ull) == 0; };
-  const bool bulk = OMC_RP_USE_BULK && (a.p == 8 * PB) && al16(a.X) && (a.strideX % 2 == 0) && al16(a.y) &&
+  const bool bulk = (a.p == 8 * PB) && al16(a.X) && (a.strideX % 2 == 0) && al16(a.y) &&
                     (a.strideY % 2 == 0) && (!weighted || (al16(a.w) && (a.strideW % 2 == 0)));
   if (weighted) return bulk ? launch_one<PB, true, true, SYRK>(a, st) : launch_one<PB, true, false, SYRK>(a, st);
   return bulk ? launch_one<PB, false, true, SYRK>(a, st) : launch_one<PB, false, false, SYRK>(a, st);

@@ -36,73 +36,20 @@
 #include "omc_common.cuh"
 #include "omc_internal.h"
 #include "omc_logtab.cuh"
-#include "omc_zigtab.cuh"
-
-#ifdef TG_EXP_TRACE
-// tuning aid (tools/tune_tridiag.sh): per-CTA phase timestamps of the solve kernel, read back with omc_debug_trace_read
-__device__ unsigned long long g_trace[32768 * 16];
-#define TG_TRACE(slot)                                                                      \
-  do {                                                                                      \
-    if (threadIdx.x == 0 && blockIdx.x < 32768) {                                           \
-      unsigned long long t_;                                                                \
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_));                                \
-      g_trace[blockIdx.x * 16 + (slot)] = t_;                                                \
-    }                                                                                       \
-  } while (0)
-#else
-#define TG_TRACE(slot)
-#endif
 
 namespace {
 
-#ifndef TG_K_DEF
-#define TG_K_DEF 18
-#endif
-constexpr int TG_K = TG_K_DEF;             // consecutive elements per thread (K/2 odd: 16-byte LDS stay conflict-free)
-#ifndef TG_NT_DEF
-#define TG_NT_DEF 128
-#endif
-constexpr int TG_NT = TG_NT_DEF;           // threads per CTA
+constexpr int TG_K = 18;                   // consecutive elements per thread (K/2 odd: 16-byte LDS stay conflict-free)
+constexpr int TG_NT = 128;                 // threads per CTA, in all three kernels
 constexpr int TG_NW = TG_NT / 32;
 constexpr int TG_TILE = TG_K * TG_NT;      // 2304 elements = 18432 bytes per staged array
 constexpr int TG_PAIRS = TG_K / 2;
-#ifndef TG_SNT_DEF
-#define TG_SNT_DEF 128
-#endif
-constexpr int TG_SNT = TG_SNT_DEF;         // threads per CTA of the SOLVE kernel: a solve tile is a 1/TG_SUB slice of an
-constexpr int TG_SNW = TG_SNT / 32;        // aggregate tile (the backward look-back runs at this granularity; with 32
-constexpr int TG_SUB = TG_NT / TG_SNT;     // threads a solve CTA is one warp and has no CTA barrier to wait at)
-constexpr int TG_STILE = TG_K * TG_SNT;
-static_assert(TG_NT % TG_SNT == 0 && TG_SNT % 32 == 0, "solve tile must divide the aggregate tile");
 constexpr unsigned FULL = 0xffffffffu;
-#ifndef TG_AGG_G
-#define TG_AGG_G 2                        // chains per CTA of the aggregate kernel (the shared P tile is staged once)
-#endif
-#ifndef TG_RNG_GROUP
-#define TG_RNG_GROUP 3                    // Philox blocks advanced in lock-step per thread
-#endif
-#ifndef TG_AGG_NORM_A
-#define TG_AGG_NORM_A 4                   // thread aggregate: power-of-two renormalisation after element pairs A and B (and at the
-#define TG_AGG_NORM_B 4                   // end); entries grow like u^k, so one mid-way stop keeps |d| up to 1e30 in range
-#endif
-#ifndef TG_AGG_NORM_SCAN
-#define TG_AGG_NORM_SCAN 0                // normalised inputs grow by < 2^63 over the five levels of the warp scan
-#endif
-#ifndef TG_PREFETCH_AHEAD
-#define TG_PREFETCH_AHEAD 0               // work items ahead whose y tile a CTA pulls into L2 (0 = off)
-#endif
-#ifndef TG_LB_WIN
-#define TG_LB_WIN 4                       // successors polled in the first look-back round
-#endif
-#ifndef TG_ZIGGURAT
-#define TG_BOX_MULLER 1                   // normals of the solve kernel: Box-Muller pairs (default) or the ziggurat below
-#ifndef TG_NORMALS_F64
-#define TG_NORMALS_F32 1                  // ... with the fp32-assisted generator (-DTG_NORMALS_F64: all-fp64 Box-Muller)
-#endif
-#endif
-#ifndef TG_SOLVE_MINB
-#define TG_SOLVE_MINB (512 / TG_SNT_DEF)   // resident solve CTAs per SM the register allocation aims at (lean variant)
-#endif
+constexpr int TG_AGG_G = 2;                // chains per CTA of the aggregate kernel (the shared P tile is staged once)
+constexpr int TG_AGG_NORM = 4;             // thread aggregate: power-of-two renormalisation after element pair 4 (and at the
+                                           // end); entries grow like u^k, so one mid-way stop keeps |d| up to 1e30 in range
+constexpr int TG_LB_WIN = 4;               // successors polled in the first look-back round
+constexpr int TG_SOLVE_MINB = 4;           // resident solve CTAs per SM the register allocation aims at (lean variant)
 
 // Look-back record of one tile.  Every payload travels in ONE 16-byte word together with its flag (16-byte accesses
 // are single transactions), so neither the writer nor the readers need a fence:
@@ -118,7 +65,7 @@ struct __align__(64) RecB {
 struct Workspace {
   unsigned long long epoch;   // advanced by the tile-scan kernel of every draw
   unsigned int pad[14];
-  // followed by: RecB[n_stiles][n_chains], per-tile partial sums double[n_stiles][n_chains][4],
+  // followed by: RecB[n_tiles][n_chains], per-tile partial sums double[n_tiles][n_chains][4],
   //              tile totals double[n_tiles][n_chains][8], tile inputs double2[n_tiles][n_chains],
   //              thread prefixes double[n_chains][n_tiles][7][TG_NT]
 };
@@ -127,19 +74,16 @@ __host__ __device__ inline long long align_up(long long x, long long a) { return
 
 struct Layout {
   long long off_recb, off_flags_end, off_parts, off_tt, off_sin, off_ex, total;
-  long long n_tiles;    // aggregate tiles (TG_TILE elements): tile totals / inputs / thread prefixes
-  long long n_stiles;   // solve tiles (TG_STILE elements): look-back records, partial sums
+  long long n_tiles;    // tiles of TG_TILE elements per chain
 };
 __host__ __device__ inline Layout make_layout(int n_chains, long long n) {
   Layout L;
   L.n_tiles = (n + TG_TILE - 1) / TG_TILE;
-  L.n_stiles = (n + TG_STILE - 1) / TG_STILE;
   const long long tc = L.n_tiles * n_chains;
-  const long long tcs = L.n_stiles * n_chains;
   L.off_recb = align_up(sizeof(Workspace), 128);
-  L.off_flags_end = L.off_recb + tcs * (long long)sizeof(RecB);
+  L.off_flags_end = L.off_recb + tc * (long long)sizeof(RecB);
   L.off_parts = align_up(L.off_flags_end, 128);
-  L.off_tt = align_up(L.off_parts + tcs * 32, 128);
+  L.off_tt = align_up(L.off_parts + tc * 32, 128);
   L.off_sin = L.off_tt + tc * 64;
   L.off_ex = align_up(L.off_sin + tc * 16, 128);
   L.total = L.off_ex + tc * 7 * TG_NT * 8;
@@ -173,15 +117,10 @@ __device__ __forceinline__ TM tm_mul(const TM& x, const TM& y) {  // x after y
 }
 // scale by a power of two so that the projective block (a b c d) has magnitude ~1 (exact; entries grow like u^k)
 __device__ __forceinline__ void tm_normalize(TM& t) {
-#ifdef TG_NORM_FMAX
-  const double mx = fmax(fmax(fabs(t.a), fabs(t.b)), fmax(fabs(t.c), fabs(t.d)));
-  int ex = ((__double2hiint(mx) >> 20) & 0x7ff) - 1023;
-#else
   // the high words of |a| .. |d| order like the magnitudes: the largest exponent comes out of three integer max
   const int hmx = max(max(__double2hiint(t.a) & 0x7fffffff, __double2hiint(t.b) & 0x7fffffff),
                       max(__double2hiint(t.c) & 0x7fffffff, __double2hiint(t.d) & 0x7fffffff));
   int ex = (hmx >> 20) - 1023;
-#endif
   ex = max(-1000, min(1000, ex));
   const double s = __hiloint2double((1023 - ex) << 20, 0);
   t.a *= s; t.b *= s; t.c *= s; t.d *= s; t.e *= s; t.f *= s; t.g *= s;
@@ -221,17 +160,9 @@ __device__ __forceinline__ double ld_nc_now(const double* p) {
 __device__ __forceinline__ double fast_rsqrt(double u) {
   double y;
   asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(u));
-#ifdef TG_RSQRT_NEWTON2
-  const double hu = 0.5 * u;
-  double e = fma(-hu, y * y, 0.5);
-  y = fma(y, e, y);
-  e = fma(-hu, y * y, 0.5);
-  y = fma(y, e, y);
-#else
   // one third-order step: with eps = 1 - u y^2 (|eps| ~ 2^-22), u^-1/2 = y (1 + eps/2 + 3 eps^2/8) + O(eps^3)
   const double eps = fma(-u, y * y, 1.0);
   y = fma(y, eps * fma(0.375, eps, 0.5), y);
-#endif
   return y;
 }
 
@@ -268,9 +199,6 @@ __device__ __forceinline__ void bulk_s2g(void* gdst, const void* smem_src, unsig
                : "memory");
   asm volatile("cp.async.bulk.commit_group;\n" ::: "memory");
 }
-__device__ __forceinline__ void bulk_prefetch_l2(const void* gsrc, unsigned bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;\n" ::"l"(gsrc), "r"(bytes) : "memory");
-}
 __device__ __forceinline__ void bulk_store_wait() { asm volatile("cp.async.bulk.wait_group.read 0;\n" ::: "memory"); }
 __device__ __forceinline__ bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
@@ -286,10 +214,9 @@ struct Stage {
 // Stage CNT arrays for the tile starting at element i_t.  Full interior tiles with 16-byte aligned sources go through
 // cp.async.bulk (issued here, completion on `bar`); everything else (last tile, odd alignments, absent arrays) through
 // plain loads.  Returns whether the bulk path was taken; stage_wait() makes the data visible to every thread.
-template <int CNT, int TILE = TG_TILE>
+template <int CNT>
 __device__ __forceinline__ bool stage_issue(const Stage (&st)[CNT], long long i_t, long long n, unsigned long long* bar,
-                                            int tid, int n_threads = TG_NT) {
-  constexpr int TG_TILE = TILE;   // (shadows the aggregate tile size inside this function)
+                                            int tid, int n_threads) {
   bool bulk = (i_t + TG_TILE < n);
 #pragma unroll
   for (int q = 0; q < CNT; ++q)
@@ -322,33 +249,24 @@ __device__ __forceinline__ void stage_wait(bool bulk, unsigned long long* bar) {
 }
 
 // ---------------------------------------------------------------------------------------------- normals
-// Two standard normals for elements (2*pair, 2*pair+1) of a chain from one Philox4x32-10 block; block index = element
-// pair index (position based, so the draw does not depend on tiling or sharding); pairs beyond 2^20 spill into the
-// second counter word.  Box-Muller in fp64 with purpose-built pieces (tools/rng_model.py is the numpy model):
-//   -ln U   : U = m 2^-(j+1) straight from the bits: j = leading zeros of word y (geometric), m in [1,2) from 52 further
-//             bits (no int->fp conversion); ln m = lc[i] + ln1p(m rc[i] - 1) with a 128-entry table on the top 7
-//             mantissa bits and a degree-7 series (|m rc - 1| <= 2^-8); absolute error 2e-15.  When y has 12 or more
-//             leading zeros (probability 2^-12) the bits below bit 20 are no longer free: the caller redoes the pair
-//             with normal_pair_slow (64-bit leading-zero count, mantissa = the bits right after the leading one).
-//   radius  : sqrt(2E) = 2E * rsqrt(2E)
-//   angle   : uniform in the first octant from 52 bits (Taylor sin / cos to 1 ulp on [0, pi/4]), three more bits swap
-//             sin <-> cos and pick the two signs
+// Counter of Philox block `block` of a chain: position based (the draw does not depend on tiling or sharding); blocks
+// beyond 2^20 spill into the second counter word.
+__device__ __forceinline__ uint4 normal_counter(unsigned long long sw, unsigned int gchain, unsigned int site,
+                                                unsigned long long block) {
+  return make_uint4((unsigned int)sw, (unsigned int)(sw >> 32) ^ (unsigned int)(block >> 20) * 0x9E3779B9u, gchain,
+                    (site << 20) | (unsigned int)(block & 0xFFFFFu));
+}
 __device__ __forceinline__ uint4 normal_block(unsigned long long sw, uint2 key, unsigned int gchain, unsigned int site,
-                                              unsigned long long pair) {
-  const uint4 ctr = make_uint4((unsigned int)sw, (unsigned int)(sw >> 32) ^ (unsigned int)(pair >> 20) * 0x9E3779B9u,
-                               gchain, (site << 20) | (unsigned int)(pair & 0xFFFFFu));
-  return philox4x32_10(ctr, key);
+                                              unsigned long long block) {
+  return philox4x32_10(normal_counter(sw, gchain, site, block), key);
 }
 // Philox4x32-10 on G counter blocks in lock-step: G independent multiply chains in flight per thread (one block at a
 // time leaves the thread waiting on every dependent IMAD.WIDE -> LOP3 pair).  Same values as philox4x32_10.
 template <int G>
 __device__ __forceinline__ void philox_group(uint4 (&ctr)[G], uint2 key) {
   const unsigned int M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
-#ifndef TG_PHILOX_R
-#define TG_PHILOX_R 10                    // (experiment knob; anything but 10 leaves the Philox4x32-10 stream)
-#endif
 #pragma unroll
-  for (int r = 0; r < TG_PHILOX_R; ++r) {
+  for (int r = 0; r < 10; ++r) {
 #pragma unroll
     for (int i = 0; i < G; ++i) {
       const unsigned int hi0 = __umulhi(M0, ctr[i].x), lo0 = M0 * ctr[i].x;
@@ -359,16 +277,16 @@ __device__ __forceinline__ void philox_group(uint4 (&ctr)[G], uint2 key) {
     key.y += W1;
   }
 }
-__device__ __forceinline__ uint4 normal_counter(unsigned long long sw, unsigned int gchain, unsigned int site,
-                                                unsigned long long pair) {
-  return make_uint4((unsigned int)sw, (unsigned int)(sw >> 32) ^ (unsigned int)(pair >> 20) * 0x9E3779B9u, gchain,
-                    (site << 20) | (unsigned int)(pair & 0xFFFFFu));
-}
-template <bool SMEM_TAB = false>
-__device__ __forceinline__ void normal_from(double jp1, double mm, int idx, uint4 b, double& z0, double& z1,
-                                            const double2* stab = nullptr) {
+// Two normals by Box-Muller in fp64 with purpose-built pieces (tools/rng_model.py is the numpy model), from
+// U = mm 2^-jp1 (mm in [1, 2), idx = its top 7 mantissa bits) and the angle bits in b.w, b.z:
+//   -ln U   : ln m = lc[i] + ln1p(m rc[i] - 1) with a 128-entry table on the top 7 mantissa bits and a degree-7 series
+//             (|m rc - 1| <= 2^-8); absolute error 2e-15
+//   radius  : sqrt(2E) = 2E * rsqrt(2E)
+//   angle   : uniform in the first octant from 52 bits (Taylor sin / cos to 1 ulp on [0, pi/4]), three more bits swap
+//             sin <-> cos and pick the two signs
+__device__ __forceinline__ void normal_from(double jp1, double mm, int idx, uint4 b, double& z0, double& z1) {
   // ---- radius
-  const double2 tab = SMEM_TAB ? stab[idx] : __ldg(reinterpret_cast<const double2*>(omc_logtab) + idx);
+  const double2 tab = __ldg(reinterpret_cast<const double2*>(omc_logtab) + idx);
   const double rr = fma(mm, tab.x, -1.0);
   double p = fma(rr, 1.0 / 7.0, -1.0 / 6.0);
   p = fma(p, rr, 1.0 / 5.0);
@@ -406,39 +324,24 @@ __device__ __forceinline__ void normal_from(double jp1, double mm, int idx, uint
   z0 = __hiloint2double(__double2hiint(a0) ^ (int)((b.w << 10) & 0x80000000u), __double2loint(a0));
   z1 = __hiloint2double(__double2hiint(a1) ^ (int)((b.w << 9) & 0x80000000u), __double2loint(a1));
 }
-// fast path; returns false when the pair has to be redone by normal_pair_slow
-template <bool SMEM_TAB = false>
-__device__ __forceinline__ bool normal_pair_fast(uint4 b, double& z0, double& z1, const double2* stab = nullptr) {
-  const int j = __clz((int)b.y);
-  const double mm = __hiloint2double((int)((b.y & 0x000FFFFFu) | 0x3FF00000u), (int)b.x);
-  normal_from<SMEM_TAB>((double)(j + 1), mm, (int)((b.y >> 13) & 127u), b, z0, z1, stab);
-  return b.y >= (1u << 20);
-}
-__device__ __noinline__ double2 normal_pair_slow(unsigned long long sw, uint2 key, unsigned int gchain, unsigned int site,
-                                                 unsigned long long pair) {
-  const uint4 b = normal_block(sw, key, gchain, site, pair);
-  const unsigned long long r = ((unsigned long long)b.y << 32) | b.x;
-  const int j = __clzll((long long)r);
-  const unsigned long long sh = (j >= 63) ? 0ull : (r << (j + 1));
-  const unsigned long long mb = sh >> 12;
-  const double mm = __longlong_as_double((long long)(0x3FF0000000000000ull | mb));
-  double2 z;
-  normal_from((double)(j + 1), mm, (int)(mb >> 45), b, z.x, z.y);
-  return z;
-}
 
 // ---------------------------------------------------------------------------------------------- fp32-assisted normals
-// Default generator (TG_NORMALS_F32; 0.607 -> 0.522 ms per C3 draw against the all-fp64 pair generator above,
-// profiles/r02_tridiag_variants.txt): FOUR normals per Philox4x32-10 block, Box-Muller with the transcendental parts on the special-
-// function unit in fp32 (lg2 / sqrt / sin / cos.approx, absolute error ~2^-21 each), the product r * (cos, sin) formed
-// in fp64 from the exactly converted factors.  The distribution differs from N(0,1) by ~1e-7 in Kolmogorov distance
-// (what curand_normal gives), invisible to any run shorter than ~1e13 draws per element, in exchange for ~45 of the
-// 68 instructions per element the fp64 generator above costs.  Stream layout: the thread's TG_K consecutive elements
-// (a "group") take blocks group * TG_F32_BLOCKS + k; words (x, y) of a block make elements 4k, 4k+1 of the group and
+// Generator of the solve kernel: FOUR normals per Philox4x32-10 block, Box-Muller with the transcendental parts on the
+// special-function unit in fp32 (lg2 / sqrt / sin / cos.approx, absolute error ~2^-21 each), the product r * (cos, sin)
+// formed in fp64 from the exactly converted factors.  The distribution differs from N(0,1) by ~1e-7 in Kolmogorov
+// distance (what curand_normal gives), invisible to any run shorter than ~1e13 draws per element, in exchange for ~45
+// of the 68 instructions per element of all-fp64 pairs.  Both generators it was measured against were removed:
+// all-fp64 Box-Muller pairs (normal_from for every pair) took 0.607 ms per C3 draw against 0.522 ms
+// (profiles/r02_tridiag_variants.txt); a Marsaglia-Tsang ziggurat had already lost to those pairs, 0.69 ms (256
+// layers) and 0.76 ms (1024 layers) against 0.605 ms at 64 x 1e6 -- the FP64-pipe share of the kernel fell from 46 % to
+// 23 %, but its random 16-byte table gathers doubled the long-scoreboard stalls and the instruction count did not fall
+// (profiles/r02_tridiag_ziggurat_variants.txt).  Stream layout: the thread's TG_K consecutive elements (a
+// "group") take blocks group * TG_F32_BLOCKS + k; words (x, y) of a block make elements 4k, 4k+1 of the group and
 // (z, w) elements 4k+2, 4k+3 -- a fixed function of the element index, independent of tiling and sharding.
 // A pair whose radius word is below 2^12 (probability 2^-20) is redone in fp64 with 32 more bits below it, so the
 // tail of the radius is exact beyond 6 sigma as well.
 constexpr int TG_F32_BLOCKS = (TG_PAIRS + 1) / 2;
+constexpr int TG_F32_GROUP = 3;            // Philox blocks advanced in lock-step per thread
 __device__ __forceinline__ bool normal_pair_f32(unsigned int w1, unsigned int w2, double& z0, double& z1) {
   const unsigned int fb = __float_as_uint(__uint2float_rz(w1));                       // top 24 bits of w1, exactly
   const float mant = __uint_as_float((fb & 0x007FFFFFu) | 0x3F800000u);               // [1, 2)
@@ -468,56 +371,6 @@ __device__ __noinline__ double2 normal_pair_f32_slow(unsigned long long sw, uint
   double2 z;
   normal_from((double)(j + 1), mm, (int)(mb >> 45), make_uint4(0u, 0u, half ? b2.w : b2.y, w2), z.x, z.y);
   return z;
-}
-
-// ---------------------------------------------------------------------------------------------- ziggurat normals
-// Alternative generator of the solve kernel (-DTG_ZIGGURAT; the Box-Muller pair above is the default because it
-// MEASURED faster, profiles/r02_tridiag_ziggurat_variants.txt: 0.605 ms per draw against 0.69 ms (256 layers, serial
-// slow path) and 0.76 ms (1024 layers, warp-cooperative slow path) at 64 x 1e6 -- the FP64-pipe share of the solve
-// kernel falls from 46 % to 23 %, but the random 16-byte table gathers double its long-scoreboard stalls and the
-// instruction count does not fall).  Marsaglia & Tsang's
-// ziggurat with 1024 layers and 52-bit candidates (tools/gen/zig_tables.py: tables, numpy model, tail checks): 64 random
-// bits give (layer: 10 bits, sign, j: 52 bits), x = j * w_layer, accepted at once when j < k_layer -- 99.6 % of the
-// candidates, about a dozen instructions of which two are FP64, against ~35 FP64 instructions per element for the
-// Box-Muller pair (log, 1/sqrt, sine and cosine polynomials).  One Philox block still serves two elements; the rest
-// (wedge test with exp, the tail beyond R by Marsaglia's exponential rejection, restart on rejection) runs in a
-// non-inlined slow path on blocks of a derived key, so a draw stays a pure function of (seed, sweep, chain, site,
-// element) whatever the tiling or sharding.
-__device__ __forceinline__ bool zig_fast(unsigned int lo, unsigned int hi, double& z) {
-  const ulonglong2 raw = __ldg(reinterpret_cast<const ulonglong2*>(omc_zig_kw) + (lo & (OMC_ZIG_LAYERS - 1)));   // one 16-byte gather
-  struct { unsigned long long k; double w; } t = {raw.x, __longlong_as_double((long long)raw.y)};
-  const unsigned int jhi = hi >> 12, jlo = (hi << 20) | (lo >> 12);          // j = bits 12..63
-  const double dj = __hiloint2double((int)(0x43300000u | jhi), (int)jlo) - 4503599627370496.0;   // exact: no int -> fp convert
-  const double x = dj * t.w;
-  z = __hiloint2double(__double2hiint(x) ^ (int)((lo << 21) & 0x80000000u), __double2loint(x));   // sign = bit 10
-  return (((unsigned long long)jhi << 32) | jlo) < t.k;
-}
-__device__ __noinline__ double zig_slow(unsigned long long sw, uint2 key, unsigned int gchain, unsigned int site,
-                                        unsigned long long elem) {
-  const uint4 ctr = normal_counter(sw, gchain, site, elem >> 1);
-  uint4 b = philox4x32_10(ctr, key);
-  unsigned int lo = (elem & 1ull) ? b.z : b.x, hi = (elem & 1ull) ? b.w : b.y;
-  unsigned int attempt = 0;
-  while (true) {
-    double z;
-    if (zig_fast(lo, hi, z)) return z;
-    const int i = (int)(lo & (OMC_ZIG_LAYERS - 1));
-    const bool neg = (lo >> 10) & 1u;
-    ++attempt;
-    b = philox4x32_10(ctr, make_uint2(key.x ^ 0x5A1C0DE5u, key.y + 2u * attempt + (unsigned int)(elem & 1ull)));
-    if (i == 0) {                       // the tail beyond R: x = R + E1 / R accepted when 2 E2 > (E1 / R)^2
-      while (true) {
-        const double xx = -log(omc_u01(b.x, b.y)) * OMC_ZIG_INV_R, yy = -log(omc_u01(b.z, b.w));
-        if (yy + yy > xx * xx) return neg ? -(OMC_ZIG_R + xx) : OMC_ZIG_R + xx;
-        ++attempt;
-        b = philox4x32_10(ctr, make_uint2(key.x ^ 0x5A1C0DE5u, key.y + 2u * attempt + (unsigned int)(elem & 1ull)));
-      }
-    }
-    const double f1 = __ldg(omc_zig_f + i), f0 = __ldg(omc_zig_f + i - 1);   // wedge: density at a uniform height of the layer
-    if (fma(f0 - f1, omc_u01(b.x, b.y), f1) < exp(-0.5 * z * z)) return z;
-    lo = b.z;                           // rejected: a fresh candidate
-    hi = b.w;
-  }
 }
 
 // ---------------------------------------------------------------------------------------------- tile scan
@@ -594,8 +447,9 @@ __global__ void __launch_bounds__(TS_NT) tg_tilescan_kernel(Workspace* ws, Layou
   tilescan_chain<TS_NT>(ws, L, C, (int)blockIdx.x, (int)threadIdx.x, s_tot);
 }
 
-// ---------------------------------------------------------------------------------------------- aggregate kernels
-// The compute part shared by the two aggregate kernels: thread aggregate over 18 staged elements, CTA scan, stores.
+// ---------------------------------------------------------------------------------------------- aggregate kernel
+// The compute part of the aggregate kernel: thread aggregate over 18 staged elements, CTA scan, stores.  (A separate
+// function: written inline in the kernel, the same code allocates registers differently.)
 template <bool GENERAL, int G>
 __device__ __forceinline__ void aggregate_compute(const omc_tridiag_nn_t& a, char* wsb, const Layout& L,
                                                   double (&s_tot)[G][TG_NW][7], const double* spe, const double* spd,
@@ -632,17 +486,17 @@ __device__ __forceinline__ void aggregate_compute(const omc_tridiag_nn_t& a, cha
         tm_step(t, dd, eprev * eprev, bb, eprev);
         eprev = lam * pe2.y;
       }
-      if (c == TG_AGG_NORM_A || c == TG_AGG_NORM_B) tm_normalize(t);
+      if (c == TG_AGG_NORM) tm_normalize(t);
     }
     tm_normalize(t);
   }
-  // ---- CTA scan of the transfer matrices (thread order): inclusive within the warp, then across the 4 warps
+  // ---- CTA scan of the transfer matrices (thread order): inclusive within the warp, then across the 4 warps.
+  //      Normalised inputs grow by < 2^63 over the five levels of the warp scan, so it renormalises only at the end.
   TM inc = t;
 #pragma unroll
   for (int d = 1; d < 32; d <<= 1) {
     const TM o = tm_shfl_up(inc, d);
     if (lane >= d) inc = tm_mul(inc, o);
-    if (TG_AGG_NORM_SCAN && d == 4) tm_normalize(inc);
   }
   tm_normalize(inc);
   if (lane == 31) {
@@ -728,115 +582,30 @@ __global__ void __launch_bounds__(TG_NT* G) tg_aggregate_kernel(omc_tridiag_nn_t
   aggregate_compute<GENERAL, G>(a, wsb, L, s_tot, spe, spd, sy, sw, sh, lam, tau, sub, tid, live, chain, tile);
 }
 
-// Persistent, double-buffered form of the lean aggregate kernel (no weights / prior mean): two CTAs per SM, each
-// walking a contiguous run of (tile, chain group) items in tile-major order.  The y tiles of item k+1 stream into the
-// other stage while item k is computed, and the shared P tile is re-staged only when the run crosses into the next
-// tile -- the one-shot kernel above is load -> compute -> store per CTA with nothing in flight during the compute
-// phase (ncu: a third of its stall samples sat on the tile's mbarrier, profiles/r02_ncu_tridiag_f32.txt).
-template <int G>
-__global__ void __launch_bounds__(TG_NT* G, 2)
-tg_aggregate_pipe_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L, int n_groups, long long n_items) {
-  extern __shared__ __align__(128) double sm[];
-  __shared__ double s_tot[G][TG_NW][7];
-  unsigned long long* bars = reinterpret_cast<unsigned long long*>(sm);   // [0] P tile, [1], [2] the two y stages
-  double* spe = sm + 4;                                                    // (sm[3] is pe[-1])
-  double* spd = spe + TG_TILE;
-  double* sy0 = spd + TG_TILE;                                             // [2 stages][G chains][TG_TILE]
-  const int sub = threadIdx.x / TG_NT;
-  const int tid = threadIdx.x % TG_NT;
-  if (threadIdx.x == 0) {
-    mbar_init(bars, 1);
-    mbar_init(bars + 1, 1);
-    mbar_init(bars + 2, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-  }
-  __syncthreads();
-  const int C = a.n_chains;
-  const long long n = a.n;
-  char* wsb = reinterpret_cast<char*>(ws);
-  const long long it0 = (long long)blockIdx.x * n_items / gridDim.x, it1 = (long long)(blockIdx.x + 1) * n_items / gridDim.x;
-  if (it0 >= it1) return;
-
-  auto issue_p = [&](long long tile) -> bool {
-    const long long i_t = tile * TG_TILE;
-    if (threadIdx.x == 0) spe[-1] = (a.pe && i_t > 0 && i_t - 1 < n - 1) ? __ldg(a.pe + i_t - 1) : 0.0;
-    const Stage st[2] = {{a.pe, n - 1, 0.0, spe}, {a.pd, n, 1.0, spd}};
-    return stage_issue<2>(st, i_t, n, bars, threadIdx.x, TG_NT * G);
-  };
-  auto issue_y = [&](long long item, int stage) -> bool {
-    const long long i_t = (item / n_groups) * TG_TILE;
-    const int chain0 = (int)(item % n_groups) * G;
-    Stage st[G];
-#pragma unroll
-    for (int g = 0; g < G; ++g)
-      st[g] = Stage{a.y.ptr + (long long)min(chain0 + g, C - 1) * a.y.chain_stride, n, 0.0, sy0 + (stage * G + g) * TG_TILE};
-    return stage_issue<G>(st, i_t, n, bars + 1 + stage, threadIdx.x, TG_NT * G);
-  };
-
-  long long cur_tile = it0 / n_groups;
-  unsigned ph_p = 0, ph_y0 = 0, ph_y1 = 0;      // parities of the three barriers
-  bool p_bulk = issue_p(cur_tile), p_pending = true;
-  bool y_bulk[2];
-  y_bulk[0] = issue_y(it0, 0);
-  y_bulk[1] = false;
-  int stage = 0;
-  for (long long item = it0; item < it1; ++item, stage ^= 1) {
-    if (item + 1 < it1) y_bulk[stage ^ 1] = issue_y(item + 1, stage ^ 1);   // that stage was released by the barrier below
-    if (p_pending) {
-      if (p_bulk) { mbar_wait(bars, ph_p); ph_p ^= 1u; }
-      p_pending = false;
-    }
-    if (y_bulk[stage]) {
-      if (stage == 0) { mbar_wait(bars + 1, ph_y0); ph_y0 ^= 1u; }
-      else { mbar_wait(bars + 2, ph_y1); ph_y1 ^= 1u; }
-    }
-    __syncthreads();                            // plain-load fills (ragged last tile, odd alignments) visible
-    const long long tile = item / n_groups;
-    const int chain = (int)(item % n_groups) * G + sub;
-    const bool live = chain < C;
-    const int cc = live ? chain : C - 1;
-    const double lam = a.lambda.ptr ? a.lambda.ptr[(long long)cc * a.lambda.chain_stride] : 1.0;
-    const double tau = a.tau.ptr ? a.tau.ptr[(long long)cc * a.tau.chain_stride] : 1.0;
-    const double* sy = sy0 + (stage * G + sub) * TG_TILE;
-    aggregate_compute<false, G>(a, wsb, L, s_tot, spe, spd, sy, nullptr, nullptr, lam, tau, sub, tid, live, chain, tile);
-    __syncthreads();                            // everybody is done with this stage, the P tile and s_tot
-    if (item + 1 < it1 && (item + 1) / n_groups != cur_tile) {
-      cur_tile = (item + 1) / n_groups;
-      p_bulk = issue_p(cur_tile);
-      p_pending = true;
-    }
-  }
-}
-
 // ---------------------------------------------------------------------------------------------- solve kernel
 // GENERAL: diagonal weights w, prior-mean terms h = P mu0 and mu0 are staged too (absent ones are filled with 1 / 0).
 // DEBUG  : injected normals (debug_z), log-det / factor probes, and the factorisation-only mode (x == NULL).
 // Tiles are taken in blockIdx order, top tile first: the reverse look-back of a tile waits only on tiles with a LOWER
 // block index, which the hardware dispatches earlier (the usual assumption of single-pass scans).
 template <bool GENERAL, bool DEBUG>
-__global__ void __launch_bounds__(TG_SNT, DEBUG ? 1 : (GENERAL ? 2 * TG_SUB : TG_SOLVE_MINB))
+__global__ void __launch_bounds__(TG_NT, DEBUG ? 1 : (GENERAL ? 2 : TG_SOLVE_MINB))
 tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
   extern __shared__ __align__(128) double sm[];
-  __shared__ double s_red[2 * TG_SNW];
-  __shared__ double s_part[3 * TG_SNW];
-#ifndef TG_BOX_MULLER
-  constexpr int ZIG_SLOTS = 64;
-  __shared__ unsigned short s_zig_item[TG_SNW][ZIG_SLOTS];
-  __shared__ double s_zig_val[TG_SNW][ZIG_SLOTS];
-#endif
+  __shared__ double s_red[2 * TG_NW];
+  __shared__ double s_part[3 * TG_NW];
   __shared__ int s_bad;
   unsigned long long* bar = reinterpret_cast<unsigned long long*>(sm);
   double* spe = sm + 4;
-  double* spd = spe + TG_STILE;
-  double* sy = spd + TG_STILE;
-  double* sz = sy + TG_STILE;                          // DEBUG: the injected debug_z tile
-  double* sw = DEBUG ? sz + TG_STILE : sz;             // GENERAL
-  double* sh = sw + TG_STILE;                          // GENERAL
-  double* smu = sh + TG_STILE;                         // GENERAL (TG_STILE + 2: mu0 of the next tile's first element)
+  double* spd = spe + TG_TILE;
+  double* sy = spd + TG_TILE;
+  double* sz = sy + TG_TILE;                          // DEBUG: the injected debug_z tile
+  double* sw = DEBUG ? sz + TG_TILE : sz;             // GENERAL
+  double* sh = sw + TG_TILE;                          // GENERAL
+  double* smu = sh + TG_TILE;                         // GENERAL (TG_TILE + 2: mu0 of the next tile's first element)
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const unsigned long long epoch = *reinterpret_cast<volatile unsigned long long*>(&ws->epoch);
   const int C = a.n_chains;
-  const long long T = L.n_stiles;            // solve tiles per chain
+  const long long T = L.n_tiles;             // tiles per chain
   const long long work = blockIdx.x;
   const long long tile = T - 1 - work / C;   // top tiles first; tile-major over the chains
   const int chain = (int)(work % C);
@@ -846,26 +615,13 @@ tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
   RecB* rec = recs + tile * C + chain;
   double* parts = reinterpret_cast<double*>(wsb + L.off_parts) + (tile * C + chain) * 4;
   const unsigned long long FLAG_A = epoch * 4 + 1, FLAG_P = epoch * 4 + 2;
-  const long long i_t = tile * TG_STILE;
+  const long long i_t = tile * TG_TILE;
   const bool solve = !DEBUG || a.x != nullptr;
   const bool inject = DEBUG && a.debug_z != nullptr;
   const int j0 = tid * TG_K;
   const long long i0 = i_t + j0;
   const int nvalid = (int)max(0ll, min((long long)TG_K, n - i0));   // this thread's elements inside the chain
 
-#ifdef TG_LOGTAB_SMEM
-  __shared__ double2 s_logtab[128];   // the -ln U table next to the SM (the lookups were L1 round trips)
-  for (int j = tid; j < 128; j += TG_SNT) s_logtab[j] = __ldg(reinterpret_cast<const double2*>(omc_logtab) + j);
-  if (TG_SNT > 32) __syncthreads(); else __syncwarp();
-#endif
-  TG_TRACE(0);
-#ifdef TG_EXP_TRACE
-  if (tid == 0 && blockIdx.x < 32768) {
-    unsigned int smid;
-    asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-    g_trace[blockIdx.x * 16 + 7] = smid;
-  }
-#endif
   // ---- stage the tile (thread 0 issues the bulk copies; nobody waits yet)
   bool bulk;
   {
@@ -883,7 +639,7 @@ tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
       mbar_init(bar, 1);
       asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
       spe[-1] = (a.pe && i_t > 0 && i_t - 1 < n - 1) ? __ldg(a.pe + i_t - 1) : 0.0;
-      if (GENERAL) smu[TG_STILE] = (mp && i_t + TG_STILE < n) ? __ldg(mp + i_t + TG_STILE) : 0.0;
+      if (GENERAL) smu[TG_TILE] = (mp && i_t + TG_TILE < n) ? __ldg(mp + i_t + TG_TILE) : 0.0;
     }
     const Stage st[7] = {{a.pe, n - 1, 0.0, spe},
                          {a.pd, n, 1.0, spd},
@@ -892,21 +648,11 @@ tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
                          {hp, n, 0.0, GENERAL ? sh : nullptr},
                          {mp, n, 0.0, GENERAL ? smu : nullptr},
                          {zp, n, 0.0, inject ? sz : nullptr}};
-    bulk = stage_issue<7, TG_STILE>(st, i_t, n, bar, tid, TG_SNT);
-  }
-  if (TG_PREFETCH_AHEAD > 0 && tid == 32 % TG_SNT) {   // pull the y tile of a CTA that starts later into L2
-    const long long w2 = work + TG_PREFETCH_AHEAD;
-    if (w2 < (long long)gridDim.x) {
-      const long long i2 = (T - 1 - w2 / C) * TG_STILE;
-      const double* p2 = a.y.ptr + (w2 % C) * a.y.chain_stride + i2;
-      if (i2 + TG_STILE < n && al16(p2)) bulk_prefetch_l2(p2, TG_STILE * 8);
-    }
+    bulk = stage_issue<7>(st, i_t, n, bar, tid, TG_NT);
   }
   // ---- loads of the thread prefix / tile input / scalars go out now; their latency hides under the normals
-  const long long atile = tile / TG_SUB;     // the aggregate tile this solve tile is a slice of
-  const double* exg = reinterpret_cast<const double*>(wsb + L.off_ex) + ((long long)chain * L.n_tiles + atile) * 7 * TG_NT +
-                      (int)(tile % TG_SUB) * TG_SNT + tid;
-  const double* sin_p = reinterpret_cast<const double*>(wsb + L.off_sin) + (atile * C + chain) * 2;
+  const double* exg = reinterpret_cast<const double*>(wsb + L.off_ex) + ((long long)chain * L.n_tiles + tile) * 7 * TG_NT + tid;
+  const double* sin_p = reinterpret_cast<const double*>(wsb + L.off_sin) + (tile * C + chain) * 2;
   const double ea = ld_nc_now(exg), eb = ld_nc_now(exg + TG_NT), ec = ld_nc_now(exg + 2 * TG_NT),
                ed = ld_nc_now(exg + 3 * TG_NT), ee = ld_nc_now(exg + 4 * TG_NT), ef = ld_nc_now(exg + 5 * TG_NT),
                eg = ld_nc_now(exg + 6 * TG_NT);
@@ -915,25 +661,12 @@ tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
   const double tau = a.tau.ptr ? ld_nc_now(a.tau.ptr + (long long)chain * a.tau.chain_stride) : 1.0;
   // ---- this thread's 18 normals, drawn into registers while the tile loads are in flight
   double g[TG_K], m[TG_K];
-#ifdef TG_EXP_NORNG
-  if (false) {
-#else
-#ifdef TG_BOX_MULLER
   if (!inject && solve && nvalid > 0) {
-#else
-  if (!inject && solve) {          // block-uniform: the rejected candidates are resolved by warp-collective code
-#endif
-#endif
     const unsigned long long sweep = a.rng.sweep ? *a.rng.sweep : 0ull;
     const uint2 key = make_uint2((unsigned int)a.rng.seed, (unsigned int)(a.rng.seed >> 32));
     const unsigned int gchain = a.rng.chain_offset + (unsigned int)chain;
-    const unsigned long long pair0 = (unsigned long long)(i0 >> 1);
     unsigned int redo = 0;
-#ifdef TG_NORMALS_F32
     const unsigned long long block0 = (unsigned long long)(i0 / TG_K) * TG_F32_BLOCKS;
-#ifndef TG_F32_GROUP
-#define TG_F32_GROUP 3
-#endif
 #pragma unroll
     for (int k0 = 0; k0 < TG_F32_BLOCKS; k0 += TG_F32_GROUP) {
       uint4 b[TG_F32_GROUP];
@@ -955,85 +688,6 @@ tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
       for (int cc = 0; cc < TG_PAIRS; ++cc)
         if (cc == c) { g[2 * cc] = z.x; g[2 * cc + 1] = z.y; }
     }
-#else
-#pragma unroll
-    for (int c0 = 0; c0 < TG_PAIRS; c0 += TG_RNG_GROUP) {
-      uint4 b[TG_RNG_GROUP];
-#pragma unroll
-      for (int i = 0; i < TG_RNG_GROUP; ++i) b[i] = normal_counter(sweep, gchain, a.rng.site, pair0 + c0 + i);
-      philox_group<TG_RNG_GROUP>(b, key);
-#pragma unroll
-      for (int i = 0; i < TG_RNG_GROUP; ++i) {
-        const int c = c0 + i;
-#ifdef TG_BOX_MULLER
-#ifdef TG_LOGTAB_SMEM
-        if (c < TG_PAIRS && !normal_pair_fast<true>(b[i], g[2 * c], g[2 * c + 1], s_logtab)) redo |= 1u << c;
-#else
-        if (c < TG_PAIRS && !normal_pair_fast(b[i], g[2 * c], g[2 * c + 1])) redo |= 1u << c;
-#endif
-#else
-        if (c < TG_PAIRS) {
-          if (!zig_fast(b[i].x, b[i].y, g[2 * c])) redo |= 1u << (2 * c);
-          if (!zig_fast(b[i].z, b[i].w, g[2 * c + 1])) redo |= 1u << (2 * c + 1);
-        }
-#endif
-      }
-    }
-#ifdef TG_BOX_MULLER
-    while (redo) {   // probability 2^-12 per pair
-      const int c = __ffs(redo) - 1;
-      redo &= redo - 1;
-      const double2 z = normal_pair_slow(sweep, key, gchain, a.rng.site, pair0 + c);
-#pragma unroll
-      for (int cc = 0; cc < TG_PAIRS; ++cc)
-        if (cc == c) { g[2 * cc] = z.x; g[2 * cc + 1] = z.y; }
-    }
-#else
-    // Rejected candidates (0.4 % of the elements: ~2 per warp and tile) are redone by the WARP together: the lanes
-    // list their rejected elements in shared memory and every item gets a lane of its own for the slow path (wedge /
-    // tail / restart), instead of the whole warp walking the slow path once per item of its unluckiest lane.
-    {
-      redo &= (1u << nvalid) - 1u;                                 // elements beyond the end of the chain need no draw
-      const int cnt = __popc(redo);
-      int pre = cnt;
-#pragma unroll
-      for (int d = 1; d < 32; d <<= 1) {
-        const int o = __shfl_up_sync(FULL, pre, d);
-        if (lane >= d) pre += o;
-      }
-      const int total = __shfl_sync(FULL, pre, 31);
-      pre -= cnt;                                                  // exclusive prefix
-      if (total > 0) {                                             // warp-uniform
-        unsigned short* list = s_zig_item[warp];
-        double* res = s_zig_val[warp];
-        {
-          unsigned int m = redo;
-          for (int k = pre; m; ++k) {
-            const int e = __ffs(m) - 1;
-            m &= m - 1;
-            if (k < ZIG_SLOTS) list[k] = (unsigned short)(lane * 32 + e);
-          }
-        }
-        __syncwarp();
-        for (int it = lane; it < min(total, ZIG_SLOTS); it += 32) {
-          const int item = list[it];
-          const long long elem = i_t + (long long)(warp * 32 + (item >> 5)) * TG_K + (item & 31);
-          res[it] = zig_slow(sweep, key, gchain, a.rng.site, (unsigned long long)elem);
-        }
-        __syncwarp();
-        unsigned int m = redo;
-        for (int k = pre; m; ++k) {
-          const int e = __ffs(m) - 1;
-          m &= m - 1;
-          const double z = (k < ZIG_SLOTS) ? res[k] : zig_slow(sweep, key, gchain, a.rng.site, (unsigned long long)i0 + e);
-#pragma unroll
-          for (int ee = 0; ee < TG_K; ++ee)
-            if (ee == e) g[ee] = z;
-        }
-      }
-    }
-#endif
-#endif   // TG_NORMALS_F32
   } else {
 #pragma unroll
     for (int k = 0; k < TG_K; ++k) g[k] = 0.0;
@@ -1045,10 +699,8 @@ tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
     iu_prev = q / p;
     f_prev = h / q;
   }
-  TG_TRACE(1);                   // thread 0: normals drawn
   __syncthreads();               // mbarrier initialised, plain-load fills visible
   if (bulk) mbar_wait(bar, 0);
-  TG_TRACE(2);                   // tile in shared memory
   if (inject) {
 #pragma unroll
     for (int c = 0; c < TG_PAIRS; ++c) {
@@ -1126,7 +778,6 @@ tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
     }
   }
   if (bad) s_bad = 1;
-  TG_TRACE(3);                   // ascending pass done (thread 0)
 
   double ssp = 0.0, ssp2 = 0.0, ssl = 0.0;
   bool bulk_out = false;
@@ -1143,7 +794,7 @@ tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
     Aff wex{1.0, 0.0};    // composition of the warps above this one
     Aff tot{1.0, 0.0};    // the whole tile
 #pragma unroll
-    for (int w = TG_SNW - 1; w >= 0; --w) {
+    for (int w = TG_NW - 1; w >= 0; --w) {
       if (w == warp) wex = tot;
       tot = aff_mul(Aff{s_red[2 * w], s_red[2 * w + 1]}, tot);
     }
@@ -1154,17 +805,11 @@ tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
     //      (no CTA barrier, nobody idles); warp 0 publishes the tile's records.
     double xfar = 0.0;     // x beyond the last element is 0 (and its multiplier m_{n-1} is 0)
     Aff R{1.0, 0.0};
-    TG_TRACE(4);                 // CTA scan done, about to publish / poll
-#ifdef TG_EXP_NOLOOKBACK
-    if (false) {
-#else
     if (tile < T - 1) {
-#endif
       if (tid == 0) {
         st_word(&rec->a, tot.a, FLAG_A);
         st_word(&rec->b, tot.b, FLAG_A);
       }
-      TG_TRACE(8);               // aggregate published
       // The first round polls only the TG_LB_WIN nearest successors: the resolving record is almost always among them,
       // and records written long ago may have left L2 (a full-width first round paid a DRAM round trip for them).
       long long base = tile + 1;
@@ -1199,7 +844,6 @@ tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
         win = 32;
       }
     }
-    TG_TRACE(5);                 // look-back resolved (warp 0)
     const double x_in = fma(R.a, xfar, R.b);
     if (tid == 0) st_word(&rec->x, fma(tot.a, x_in, tot.b), FLAG_P);
     // ---- descending pass: x and both quadratic forms; x overwrites y in shared memory
@@ -1235,10 +879,8 @@ tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
       }
       *reinterpret_cast<double2*>(sy + j0 + 2 * c) = x2;
     }
-    bulk_out = (i_t + TG_STILE <= n) && al16(a.x + (long long)chain * n + i_t);
-#ifndef TG_GENERIC_STORE
+    bulk_out = (i_t + TG_TILE <= n) && al16(a.x + (long long)chain * n + i_t);
     if (bulk_out) asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");
-#endif
   }
   // ---- per-tile partial sums (fixed order: shuffle tree, then the 4 warps in order)
   ssp = omc_warp_sum(fma(2.0, ssp2, ssp));
@@ -1246,36 +888,27 @@ tg_solve_kernel(omc_tridiag_nn_t a, Workspace* ws, Layout L) {
   if (DEBUG) logdet = omc_warp_sum(logdet);
   if (lane == 0) {
     s_part[warp] = ssp;
-    s_part[TG_SNW + warp] = ssl;
-    s_part[2 * TG_SNW + warp] = logdet;
+    s_part[TG_NW + warp] = ssl;
+    s_part[2 * TG_NW + warp] = logdet;
   }
   __syncthreads();
   if (solve) {   // x tile: shared -> global (one bulk store for full aligned tiles)
     double* xg = a.x + (long long)chain * n + i_t;
     if (bulk_out) {
-#ifdef TG_GENERIC_STORE
-#pragma unroll 3
-      for (int j = 2 * tid; j < TG_STILE; j += 2 * TG_SNT)    // coalesced 16-byte stores: no proxy fence, no bulk wait
-        *reinterpret_cast<double2*>(xg + j) = *reinterpret_cast<const double2*>(sy + j);
-#else
-      if (tid == 0) bulk_s2g(xg, sy, TG_STILE * 8);
-#endif
+      if (tid == 0) bulk_s2g(xg, sy, TG_TILE * 8);
     } else {
-      for (int j = tid; j < TG_STILE; j += TG_SNT)
+      for (int j = tid; j < TG_TILE; j += TG_NT)
         if (i_t + j < n) xg[j] = sy[j];
     }
   }
   if (tid == 0) {   // per-tile partials; tg_partials_kernel reduces them per chain in a fixed order
     double sp = 0.0, sl = 0.0, ld = 0.0;
-    for (int w = 0; w < TG_SNW; ++w) { sp += s_part[w]; sl += s_part[TG_SNW + w]; ld += s_part[2 * TG_SNW + w]; }
+    for (int w = 0; w < TG_NW; ++w) { sp += s_part[w]; sl += s_part[TG_NW + w]; ld += s_part[2 * TG_NW + w]; }
     *reinterpret_cast<double2*>(parts) = make_double2(sp, sl);
     parts[2] = ld;
     if (s_bad && a.status) atomicOr(&a.status[chain], OMC_STATUS_NOT_PD);
-#ifndef TG_GENERIC_STORE
     if (solve && bulk_out) bulk_store_wait();   // shared memory must stay alive until the bulk store has read it
-#endif
   }
-  TG_TRACE(6);
 }
 
 // Per-chain sums of the per-tile partials, fixed order (deterministic): one warp per chain.
@@ -1382,13 +1015,13 @@ __global__ void tridiag_matvec_kernel(const double* pd, const double* pe, omc_ve
 int check_args(const omc_tridiag_nn_t* a, const char* who) {
   OMC_REQUIRE(a && a->pd && a->workspace, "%s: null argument", who);
   OMC_REQUIRE(a->n_chains >= 1 && a->n >= 1, "%s: n_chains=%d n=%lld", who, a->n_chains, a->n);
-  OMC_REQUIRE((long long)a->n_chains * ((a->n + TG_STILE - 1) / TG_STILE) < 0x7fffffffll, "%s: too many tiles", who);
+  OMC_REQUIRE((long long)a->n_chains * ((a->n + TG_TILE - 1) / TG_TILE) < 0x7fffffffll, "%s: too many tiles", who);
   return 0;
 }
 
 constexpr int aggregate_smem_doubles(bool general, int g) { return 4 + (general ? 5 : 2 + g) * TG_TILE + 4; }
 constexpr int solve_smem_doubles(bool general, bool debug) {
-  return 4 + (3 + (debug ? 1 : 0) + (general ? 3 : 0)) * TG_STILE + 4;
+  return 4 + (3 + (debug ? 1 : 0) + (general ? 3 : 0)) * TG_TILE + 4;
 }
 
 template <bool GENERAL, int G>
@@ -1400,31 +1033,11 @@ int launch_aggregate(const omc_tridiag_nn_t& a, Workspace* ws, const Layout& L, 
   OMC_LAUNCH_CHECK();
   return 0;
 }
-#ifndef TG_AGG_PIPE
-#define TG_AGG_PIPE 0                     // lean aggregate pass: persistent double-buffered kernel (0: one CTA per item)
-#endif
-template <int G>
-int launch_aggregate_pipe(const omc_tridiag_nn_t& a, Workspace* ws, const Layout& L, cudaStream_t st) {
-  static int n_sm = 0;
-  if (!n_sm) {
-    int dev = 0;
-    OMC_CHECK_CUDA(cudaGetDevice(&dev));
-    OMC_CHECK_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
-  }
-  const int smem = (4 + (2 + 2 * G) * TG_TILE) * 8;
-  const int n_groups = (a.n_chains + G - 1) / G;
-  const long long n_items = L.n_tiles * n_groups;
-  const unsigned int grid = (unsigned int)std::min<long long>(n_items, 2ll * n_sm);
-  OMC_CHECK_CUDA(cudaFuncSetAttribute(tg_aggregate_pipe_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  tg_aggregate_pipe_kernel<G><<<grid, TG_NT * G, smem, st>>>(a, ws, L, n_groups, n_items);
-  OMC_LAUNCH_CHECK();
-  return 0;
-}
 template <bool GENERAL, bool DEBUG>
 int launch_solve(const omc_tridiag_nn_t& a, Workspace* ws, const Layout& L, unsigned grid, cudaStream_t st) {
   const int smem = solve_smem_doubles(GENERAL, DEBUG) * 8;
   OMC_CHECK_CUDA(cudaFuncSetAttribute(tg_solve_kernel<GENERAL, DEBUG>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  tg_solve_kernel<GENERAL, DEBUG><<<grid, TG_SNT, smem, st>>>(a, ws, L);
+  tg_solve_kernel<GENERAL, DEBUG><<<grid, TG_NT, smem, st>>>(a, ws, L);
   OMC_LAUNCH_CHECK();
   return 0;
 }
@@ -1432,12 +1045,6 @@ int launch_solve(const omc_tridiag_nn_t& a, Workspace* ws, const Layout& L, unsi
 }  // namespace
 
 extern "C" {
-
-#ifdef TG_EXP_TRACE
-int omc_debug_trace_read(void* dst, long long bytes) {
-  return (int)cudaMemcpyFromSymbol(dst, g_trace, (size_t)bytes);
-}
-#endif
 
 int omc_tridiag_workspace(int n_chains, long long n, long long* bytes) {
   OMC_REQUIRE(n_chains >= 1 && n >= 1 && bytes, "omc_tridiag_workspace: bad argument");
@@ -1458,33 +1065,24 @@ int omc_tridiag_nn_draw(const omc_tridiag_nn_t* a, void* stream) {
   if (int rc = check_args(a, "omc_tridiag_nn_draw")) return rc;
   OMC_REQUIRE(a->y.ptr, "omc_tridiag_nn_draw: y missing");
   const Layout L = make_layout(a->n_chains, a->n);
-  const unsigned int grid = (unsigned int)(L.n_stiles * a->n_chains);
+  const unsigned int grid = (unsigned int)(L.n_tiles * a->n_chains);
   Workspace* ws = reinterpret_cast<Workspace*>(a->workspace);
   cudaStream_t st = (cudaStream_t)stream;
   const bool general = a->w.ptr || a->h.ptr || a->mu0.ptr;
   const bool debug = a->debug_z || a->logdet || a->probe_l || a->probe_c || !a->x;
-#ifndef TG_EXP_SKIP_AGG
-  {
-    int rc;
-    if (general) rc = launch_aggregate<true, 1>(*a, ws, L, st);
-    else if (TG_AGG_PIPE && a->n_chains >= TG_AGG_G) rc = launch_aggregate_pipe<TG_AGG_G>(*a, ws, L, st);
-    else if (a->n_chains >= TG_AGG_G) rc = launch_aggregate<false, TG_AGG_G>(*a, ws, L, st);
-    else rc = launch_aggregate<false, 1>(*a, ws, L, st);
-    if (rc) return rc;
-  }
-#endif
+  int rc;
+  if (general) rc = launch_aggregate<true, 1>(*a, ws, L, st);
+  else if (a->n_chains >= TG_AGG_G) rc = launch_aggregate<false, TG_AGG_G>(*a, ws, L, st);
+  else rc = launch_aggregate<false, 1>(*a, ws, L, st);
+  if (rc) return rc;
   tg_tilescan_kernel<<<a->n_chains, TS_NT, 0, st>>>(ws, L, a->n_chains);
   OMC_LAUNCH_CHECK();
-  int rc;
-#ifdef TG_EXP_SKIP_SOLVE
-  return 0;
-#endif
   if (general) rc = debug ? launch_solve<true, true>(*a, ws, L, grid, st) : launch_solve<true, false>(*a, ws, L, grid, st);
   else rc = debug ? launch_solve<false, true>(*a, ws, L, grid, st) : launch_solve<false, false>(*a, ws, L, grid, st);
   if (rc) return rc;
   const bool solve = a->x != nullptr;
   if ((solve && (a->ss_prior || a->ss_lik)) || a->logdet) {
-    tg_partials_kernel<<<a->n_chains, 32, 0, st>>>(ws, L, L.n_stiles, a->n_chains, solve ? a->ss_prior : nullptr,
+    tg_partials_kernel<<<a->n_chains, 32, 0, st>>>(ws, L, L.n_tiles, a->n_chains, solve ? a->ss_prior : nullptr,
                                                    solve ? a->ss_lik : nullptr, a->logdet);
     OMC_LAUNCH_CHECK();
   }

@@ -5,7 +5,7 @@
 # PARENT_LIB: libomc.so of the parent commit, built into an untracked directory of the tree
 # (e.g. git worktree add /tmp/parent HEAD~1 && make -C /tmp/parent/openmcmc_b200/csrc && cp /tmp/parent/openmcmc_b200/libomc.so ab_parent/).
 # Runs: the card's name / power limit / max SM clock; tests/test_gpu_dense_warp.py; the draw alone at p = 48, 56, 63, 64
-# (4096 chains; parent, default selection, register kernel forced); the C2 headline (bench.py --no-cpu --no-e2e
+# (4096 chains; parent and new); the C2 headline (bench.py --no-cpu --no-e2e
 # --no-extras) alternating parent / new 3 times each; --dump-outputs of both and their largest relative difference;
 # one parent / new pair of every workload in WORKLOADS (default: c1 c3 c4a c4b c5).
 set -u
@@ -24,7 +24,6 @@ echo "test_gpu_dense_warp rc=$?"; tail -3 "$OUT/pytest_dense_warp.log"
 for p in 48 56 63 64; do
   OMC_LIB=$PARENT timeout 300 python tools/perf_dense_draw.py 4096 $p | sed 's/^/parent /'
   OMC_LIB=$NEW timeout 300 python tools/perf_dense_draw.py 4096 $p | sed 's/^/new    /'
-  OMC_LIB=$NEW OMC_DENSE_DRAW_IMPL=w timeout 300 python tools/perf_dense_draw.py 4096 $p | sed 's/^/new    /'
 done | tee "$OUT/draw_only.txt"
 
 for r in 1 2 3; do

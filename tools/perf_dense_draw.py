@@ -47,6 +47,5 @@ for _ in range(reps):
     call()
 e1.record()
 torch.cuda.synchronize()
-import os
-print(json.dumps({"impl": os.environ.get("OMC_DENSE_DRAW_IMPL", "default"), "C": C, "p": p, "ms": e0.elapsed_time(e1) / reps, "mean_rel_err_vs_torch": err,
+print(json.dumps({"C": C, "p": p, "ms": e0.elapsed_time(e1) / reps, "mean_rel_err_vs_torch": err,
                   "status_bad": int((status != 0).sum())}))
