@@ -113,7 +113,10 @@ typedef struct {
   int* status;          /* optional [n_chains], OR-ed with OMC_STATUS_*                      */
   /* Truncated prior (domain_response_lower / upper on the Normal prior): the draw becomes ONE coordinate-wise Gibbs
    * scan from the current beta,  beta_i ~ N(v_i (b_i - Q_i. beta + Q_ii beta_i), v_i = 1/Q_ii) truncated to
-   * [lo_i, hi_i], one truncnorm.rvs uniform per coordinate; p == 1 draws from N(b/Q, 1/Q) truncated.
+   * [lo_i, hi_i], one truncnorm.rvs uniform per coordinate (Philox block i of the chain, or debug_u); p == 1 draws
+   * from N(b/Q, 1/Q) truncated.  p <= 64: Q in shared memory, one CTA per chain; 64 < p <= 512: one warp per chain
+   * streaming the rows of G (and of a dense P0) through shared memory; p > 512 is refused.  probe_Q / probe_b are
+   * written; center, rss_out, mode and workspace are ignored.
    *   ref: sampler.py:196-205, gmrf.py:201-266 (gibbs_canonical_truncated_normal), gmrf.py:269-292 */
   int truncated;        /* 0: plain draw above (trunc_* ignored)                             */
   omc_vec_t trunc_lo, trunc_hi; /* bounds, trunc_lo_len / trunc_hi_len in {1, p} values (NULL => -inf / +inf) */

@@ -359,7 +359,9 @@ extern "C" int omc_nn_dense_draw(const omc_nn_dense_t* args, void* stream) {
   OMC_REQUIRE(args->prior_kind == OMC_MAT_EYE || args->prior_P.ptr, "omc_nn_dense_draw: prior_P missing");
   const int p = args->p;
   if (args->truncated) {
-    OMC_REQUIRE(p <= 128, "omc_nn_dense_draw: the truncated-prior scan holds Q in shared memory (p=%d > 128)", p);
+    // p <= 64: Q in shared memory, the scan in one warp of a CTA per chain; above: one warp per chain streaming the rows
+    // of G (and P0) through shared memory (trunc_scan.cu)
+    if (p > 64) return omc_launch_trunc_stream(*args, (cudaStream_t)stream);
     const size_t smem = (size_t)(p * (p + 1) + 4 * p) * sizeof(double);
     OMC_CHECK_CUDA(cudaFuncSetAttribute(nn_truncated_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     nn_truncated_scan_kernel<<<args->n_chains, DD_THREADS, smem, (cudaStream_t)stream>>>(*args);

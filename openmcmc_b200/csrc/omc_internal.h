@@ -17,3 +17,5 @@ long long omc_blocked_workspace_doubles(int p);
 // (32 < p <= 64)
 int omc_launch_warp_draw(const omc_nn_dense_t& a, cudaStream_t st);
 int omc_launch_left_draw(const omc_nn_dense_t& a, cudaStream_t st);
+// trunc_scan.cu: truncated-prior Gibbs scan for 64 < p <= 512, one warp per chain, rows of G / P0 streamed
+int omc_launch_trunc_stream(const omc_nn_dense_t& a, cudaStream_t st);

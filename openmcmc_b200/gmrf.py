@@ -313,7 +313,8 @@ def gibbs_canonical_truncated_normal(b, Q, x, lower=-np.inf, upper=np.inf, u=Non
     """One coordinate-wise Gibbs scan of N_c(Q^-1 b, Q^-1) truncated to [lower, upper] from the current `x`
     (Rue & Held 2005, Lemma 2.1): x_i ~ N(v_i (b_i - Q_i. x + Q_ii x_i), v_i = 1 / Q_ii) truncated, one truncnorm
     inverse-CDF draw per coordinate (`u`: the uniforms behind them).  Unbounded: a plain canonical draw.  The scan is
-    the truncated-prior mode of omc_nn_dense_draw (p <= 64).  ref: gmrf.py:201-266"""
+    the truncated-prior mode of omc_nn_dense_draw: Q in shared memory up to p = 64, the rows of Q streamed through
+    shared memory by one warp above that, up to p = 512.  ref: gmrf.py:201-266"""
     def unbounded(v, inf):
         return v is None or (np.ndim(v) == 0 and v == inf)
 
@@ -323,8 +324,8 @@ def gibbs_canonical_truncated_normal(b, Q, x, lower=-np.inf, upper=np.inf, u=Non
     dev = _dev()
     Qd = Q.toarray() if sparse.issparse(Q) else np.asarray(Q, dtype=np.float64)
     p = Qd.shape[0]
-    if p > 64:
-        raise NotImplementedError("gibbs_canonical_truncated_normal on the device holds Q in shared memory (p <= 64)")
+    if p > 512:
+        raise NotImplementedError(f"gibbs_canonical_truncated_normal on the device supports p <= 512 (p = {p})")
     rec = torch.zeros(1, p * p + p + 2, dtype=torch.float64, device=dev)
     rec[0, : p * p] = _t(Qd.reshape(-1), dev)
     rec[0, p * p: p * p + p] = _t(np.asarray(b, dtype=np.float64).reshape(-1), dev)

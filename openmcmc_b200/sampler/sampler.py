@@ -81,13 +81,13 @@ class NormalNormal(MCMCSampler):
 
     Device paths (chosen from the model structure at compile time):
       * dense   : one Normal likelihood with mean X @ param (LinearCombination), diagonal/identity response precision,
-                  any small (p <= 64) prior precision          -> omc_reg_pass + omc_nn_dense_draw
+                  any prior precision up to p = 512            -> omc_reg_pass + omc_nn_dense_draw
       * banded  : one Normal likelihood with mean = param (Identity), diagonal/identity response precision, tridiagonal
                   prior precision (temporal GMRF)              -> omc_tridiag_nn_draw
     Truncated priors (domain_response_lower / upper on the Normal prior; sampler.py:196-205 ->
-    gmrf.gibbs_canonical_truncated_normal, SURVEY §8 f3) are supported on the dense path: the draw becomes one
-    coordinate-wise truncated-normal Gibbs scan from the current value.  `debug_draws={"u": ...}` injects the uniforms
-    behind the reference's truncnorm.rvs calls.
+    gmrf.gibbs_canonical_truncated_normal, SURVEY §8 f3) are supported on the dense path up to p = 512: the draw
+    becomes one coordinate-wise truncated-normal Gibbs scan from the current value.  `debug_draws={"u": ...}` injects
+    the uniforms behind the reference's truncnorm.rvs calls.
     """
 
     def __post_init__(self):
@@ -210,6 +210,8 @@ class NormalNormal(MCMCSampler):
             ctx["trunc"] = None
             lo, hi = prior.domain_response_lower, prior.domain_response_upper
             if lo is not None or hi is not None:
+                if p > 512:
+                    raise engine.PlanError(f"NormalNormal with a truncated prior supports p <= 512 coefficients (p = {p})")
                 # ref gmrf.py:236-243: missing bounds are -inf / +inf, scalars broadcast over the p coordinates
                 def bound(v):
                     if v is None:
