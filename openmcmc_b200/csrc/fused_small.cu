@@ -35,7 +35,8 @@ __device__ __forceinline__ void op_gamma(const omc_logp_gamma_t& a, int c, int l
     const double scale = 1.0 / rt;
     const double y = x / scale;
     double lp = omc_xlogy(sh - 1.0, y) - y - lgamma(sh) - log(scale);
-    if (!(y >= 0.0)) lp = isnan(y) ? y : -INFINITY;
+    if (!(sh > 0.0) || rt < 0.0) lp = nan("");               // scipy: invalid shape / rate -> nan
+    else if (!(y >= 0.0)) lp = isnan(y) ? y : -INFINITY;
     acc += lp;
   }
   acc = lanes_sum<LPC>(acc);
@@ -48,7 +49,8 @@ __device__ __forceinline__ void op_poisson(const omc_logp_poisson_t& a, int c, i
     const double k = fvat(a.k, c, i, 0.0);
     const double mu = fvat(a.rate, c, a.rate_len > 1 ? i : 0, 1.0);
     double lp = omc_xlogy(k, mu) - lgamma(k + 1.0) - mu;
-    if (!(k >= 0.0) || floor(k) != k) lp = isnan(k) ? k : -INFINITY;
+    if (!(mu >= 0.0)) lp = nan("");                           // scipy: invalid rate -> nan
+    else if (!(k >= 0.0) || floor(k) != k) lp = isnan(k) ? k : -INFINITY;   // off the support
     acc += lp;
   }
   acc = lanes_sum<LPC>(acc);

@@ -31,7 +31,8 @@ __global__ void __launch_bounds__(LP_THREADS) logp_gamma_kernel(omc_logp_gamma_t
     const double scale = 1.0 / rt;
     const double y = x / scale;
     double lp = omc_xlogy(sh - 1.0, y) - y - lgamma(sh) - log(scale);
-    if (!(y >= 0.0)) lp = isnan(y) ? y : -INFINITY;
+    if (!(sh > 0.0) || rt < 0.0) lp = nan("");               // scipy: invalid shape / rate -> nan
+    else if (!(y >= 0.0)) lp = isnan(y) ? y : -INFINITY;
     acc += lp;
   }
   acc = omc_block_sum(acc, scratch);
@@ -46,7 +47,8 @@ __global__ void __launch_bounds__(LP_THREADS) logp_poisson_kernel(omc_logp_poiss
     const double k = vat(a.k, c, i, 0.0);
     const double mu = vat(a.rate, c, a.rate_len > 1 ? i : 0, 1.0);
     double lp = omc_xlogy(k, mu) - lgamma(k + 1.0) - mu;
-    if (!(k >= 0.0) || floor(k) != k) lp = isnan(k) ? k : -INFINITY;
+    if (!(mu >= 0.0)) lp = nan("");                           // scipy: invalid rate -> nan
+    else if (!(k >= 0.0) || floor(k) != k) lp = isnan(k) ? k : -INFINITY;   // off the support
     acc += lp;
   }
   acc = omc_block_sum(acc, scratch);
@@ -222,14 +224,15 @@ int omc_logp_normal_ss(const omc_logp_normal_ss_t* a, void* stream) {
   return 0;
 }
 int omc_logp_gamma(const omc_logp_gamma_t* a, void* stream) {
-  OMC_REQUIRE(a && a->out && a->x.ptr, "omc_logp_gamma: null argument");
+  OMC_REQUIRE(a && a->out && (a->x.ptr || a->n_elem == 0), "omc_logp_gamma: null argument");
   OMC_REQUIRE(a->n_chains >= 1 && a->n_elem >= 0, "omc_logp_gamma: bad shape");
   logp_gamma_kernel<<<a->n_chains, LP_THREADS, 0, (cudaStream_t)stream>>>(*a);
   OMC_LAUNCH_CHECK();
   return 0;
 }
 int omc_logp_poisson(const omc_logp_poisson_t* a, void* stream) {
-  OMC_REQUIRE(a && a->out && a->k.ptr, "omc_logp_poisson: null argument");
+  OMC_REQUIRE(a && a->out && (a->k.ptr || a->n_elem == 0), "omc_logp_poisson: null argument");
+  OMC_REQUIRE(a->n_chains >= 1 && a->n_elem >= 0, "omc_logp_poisson: bad shape");
   logp_poisson_kernel<<<a->n_chains, LP_THREADS, 0, (cudaStream_t)stream>>>(*a);
   OMC_LAUNCH_CHECK();
   return 0;
