@@ -15,19 +15,24 @@
 // * Left-looking kernel (nn_left_draw_kernel, larger p; dense_draw.cu selects): only block column k in registers
 //   (<= 16 doubles per lane, read from the record at the top of step k), the finished factor in the warp's slice of
 //   shared memory.  Step k: C(i, k) = Q(i, k) - sum_{j<k} L(i, j) L(k, j)', i >= k, on the tensor pipe with both operand
-//   fragments (element [g][4s + kq] of a tile) read straight from shared memory; the pivot stages of column k; L(:, k)
-//   back to shared memory.  Every tile sees the same DMMAs with the same operands in the same order as in the
-//   right-looking form.  At p = 64: 128 registers and 16,352 bytes of shared memory per warp, 14 chains per SM,
+//   fragments (element [g][4s + kq] of a tile) read straight from shared memory; the pivot stages of the diagonal tile
+//   alone, an identity tile riding along and coming out as L_kk^-T; the panel L(i, k) = C(i, k) L_kk^-T as two DMMAs
+//   per tile and w[i] -= L(i, k) w[k] as a mat-vec; L(:, k), with L_kk^-1 in place of L_kk, back to shared memory.  The
+//   backward solve is then one 8 x 8 mat-vec per block instead of 8 dependent substitution steps.  The pivot stages
+//   no longer touch the off-diagonal tiles (224 of the 288 tile updates at p = 64, shuffle + 3 FMAs + select each).
+//   At p = 64: 128 registers and 16,352 bytes of shared memory per warp, 14 chains per SM,
 //   persistent warps, the next chain's record prefetched into L2 while the current one runs.  (A register copy of
 //   block column k + 1 loaded one step ahead does not fit in the 128 registers: 4 of the 14 warps share one quarter
 //   of the register file.)
 //
-// Pivot stages of block column k (both forms): pivot from the diagonal tile by shuffle, 1/sqrt by MUFU.RSQ64H + two
+// Pivot stages of block column k (register kernel): pivot from the diagonal tile by shuffle, 1/sqrt by MUFU.RSQ64H + two
 // Newton steps, scale column, rank-1 update of the remaining columns of EVERY tile of the block column (independent work
 // across the tiles hides the pivot chain); the right-hand side b (row layout, element 8i + g) rides along, so
-// w = L^-1 b is there when the factorisation ends; 1/L_cc replaces L_cc on the diagonal.
+// w = L^-1 b is there when the factorisation ends; 1/L_cc replaces L_cc on the diagonal.  The left-looking kernel runs
+// the same stages on the diagonal tile only (factor_diag: L_kk and w[k] come out bit for bit the same).
 // Backward solve L' x = w + z block by block from the bottom: partial sums of the off-diagonal products stay private
-// per lane and are reduced over g (3 xor-shuffles) once per block; the 8 x 8 diagonal solves are quad-local.
+// per lane and are reduced over g (3 xor-shuffles) once per block; the 8 x 8 diagonal solves are quad-local
+// substitutions (register kernel) or mat-vecs with L_jj^-1 (left-looking kernel).
 // Epilogue: rss(beta) = rss0 - 2 d'c0 + d'G d from the centre record (omc.h), G read a second time (L2).
 #include "../../include/omc.h"
 #include "omc_common.cuh"
@@ -205,13 +210,42 @@ __device__ __forceinline__ void factor_panel(Tile tile, double (&w)[PB], int k, 
   }
 }
 
-// Backward solve L' x = w + z, x -> beta.  ldiag(j, c, l0, l1): L_jj[c][2kq], L_jj[c][2kq+1] (1 / L_cc on the
-// diagonal; only the lower triangle is used); loff(j, tc, r): L(j, tc)[g][2kq + r], tc < j.
-template <int PB, class Diag, class Off>
-__device__ __forceinline__ void back_solve(double* beta, int p, const double (&w)[PB], double z0, double z1, int g, int kq,
-                                           Diag ldiag, Off loff) {
-  // r = w + z in column layout; racc = per-lane partial sums (the g == 0 lanes start from r)
-  double racc[PB][2];
+// The pivot stages of the diagonal tile D = C(k, k) alone, with w[k] riding along: D and w[k] come out exactly as from
+// factor_panel.  E enters as the identity and sees the same column operations, so it leaves as L_kk^-T (upper
+// triangular, exact zeros below the diagonal) in accumulator layout.  D's diagonal keeps L_cc: nothing reads D again.
+__device__ __forceinline__ void factor_diag(double (&D)[2], double (&E)[2], double& wk, int g, int kq, bool& bad) {
+#pragma unroll 1
+  for (int jq = 0; jq < 4; ++jq) {
+    const bool own = kq == jq;
+#pragma unroll
+    for (int reg = 0; reg < 2; ++reg) {
+      const int jj = 2 * jq + reg;
+      const double piv = shf(D[reg], 4 * jj + jq);
+      if (!(piv > 0.0)) bad = true;
+      const double rd = wrsqrt(piv);
+      D[reg] = own ? D[reg] * rd : D[reg];
+      E[reg] = own ? E[reg] * rd : E[reg];
+      const double wc = shf(wk, 4 * jj) * rd;
+      if (g == jj) wk = wc;
+      double lc0 = shf(D[reg], 8 * kq + jq);        // L[2kq][jj]
+      double lc1 = shf(D[reg], 8 * kq + 4 + jq);    // L[2kq+1][jj]
+      if (!(2 * kq > jj)) lc0 = 0.0;
+      if (!(2 * kq + 1 > jj)) lc1 = 0.0;
+      const double lg = shf(D[reg], 4 * g + jq);    // L[g][jj]
+      const double le = shf(E[reg], 4 * g + jq);    // E[g][jj]
+      D[0] = fma(-lg, lc0, D[0]);
+      D[1] = fma(-lg, lc1, D[1]);
+      if (g > jj) wk = fma(-lg, wc, wk);
+      E[0] = fma(-le, lc0, E[0]);
+      E[1] = fma(-le, lc1, E[1]);
+    }
+  }
+}
+
+// r = w + z in column layout; racc = per-lane partial sums of the backward solve (the g == 0 lanes start from r)
+template <int PB>
+__device__ __forceinline__ void solve_rhs(double (&racc)[PB][2], const double (&w)[PB], double z0, double z1, int g,
+                                          int kq) {
 #pragma unroll
   for (int tc = 0; tc < PB; ++tc)
 #pragma unroll
@@ -220,6 +254,15 @@ __device__ __forceinline__ void back_solve(double* beta, int p, const double (&w
       const double zcol = shf(r ? z1 : z0, 4 * tc + kq);
       racc[tc][r] = (g == 0) ? wcol + zcol : 0.0;
     }
+}
+
+// Backward solve L' x = w + z, x -> beta.  ldiag(j, c, l0, l1): L_jj[c][2kq], L_jj[c][2kq+1] (1 / L_cc on the
+// diagonal; only the lower triangle is used); loff(j, tc, r): L(j, tc)[g][2kq + r], tc < j.
+template <int PB, class Diag, class Off>
+__device__ __forceinline__ void back_solve(double* beta, int p, const double (&w)[PB], double z0, double z1, int g, int kq,
+                                           Diag ldiag, Off loff) {
+  double racc[PB][2];
+  solve_rhs<PB>(racc, w, z0, z1, g, kq);
 #pragma unroll
   for (int j = PB - 1; j >= 0; --j) {
     double v0 = racc[j][0], v1 = racc[j][1];
@@ -253,6 +296,34 @@ __device__ __forceinline__ void back_solve(double* beta, int p, const double (&w
         racc[tc][0] = fma(-loff(j, tc, 0), xg, racc[tc][0]);
         racc[tc][1] = fma(-loff(j, tc, 1), xg, racc[tc][1]);
       }
+    }
+  }
+}
+
+// Backward solve L' x = w + z with the inverted diagonal blocks, x -> beta: x_j = L_jj^-T v_j is one 8 x 8 mat-vec
+// (lane-local) and a quad reduction, which leaves x_j in row layout (x[8j + g]), the form the off-diagonal updates
+// take.  linv(j, l0, l1): L_jj^-1[2kq][g], L_jj^-1[2kq+1][g] (0 above the diagonal); loff as in back_solve.
+template <int PB, class Inv, class Off>
+__device__ __forceinline__ void back_solve_inv(double* beta, int p, const double (&w)[PB], double z0, double z1, int g,
+                                               int kq, Inv linv, Off loff) {
+  double racc[PB][2];
+  solve_rhs<PB>(racc, w, z0, z1, g, kq);
+#pragma unroll
+  for (int j = PB - 1; j >= 0; --j) {
+    double v0 = racc[j][0], v1 = racc[j][1];
+    v0 += shx(v0, 4); v1 += shx(v1, 4);
+    v0 += shx(v0, 8); v1 += shx(v1, 8);
+    v0 += shx(v0, 16); v1 += shx(v1, 16);
+    double l0, l1;
+    linv(j, l0, l1);
+    double xg = fma(l0, v0, l1 * v1);
+    xg += shx(xg, 1);
+    xg += shx(xg, 2);                                           // x[8j + g], the same bits in all four lanes
+    if (kq == 0 && 8 * j + g < p) beta[8 * j + g] = xg;
+#pragma unroll
+    for (int tc = 0; tc < j; ++tc) {
+      racc[tc][0] = fma(-loff(j, tc, 0), xg, racc[tc][0]);
+      racc[tc][1] = fma(-loff(j, tc, 1), xg, racc[tc][1]);
     }
   }
 }
@@ -381,8 +452,8 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, ctas_per_sm<PB>()) nn_warp
 
 // ---------------------------------------------------------------------------------------------------------------------
 // Left-looking kernel.  Shared-memory slice of one warp: the PB(PB-1)/2 off-diagonal tiles of L full, then the PB-1
-// first diagonal tiles as packed lower triangles (36 doubles, element [r][c] at r(r+1)/2 + c, 1 / L_cc on the
-// diagonal); the last diagonal tile stays in registers.
+// first diagonal blocks' INVERSES L_kk^-1 as packed lower triangles (36 doubles, element [r][c] at r(r+1)/2 + c; the
+// backward solve is their only reader); the last one stays in registers, as L_77^-T in accumulator layout.
 template <int PB>
 struct LeftSmem {
   static constexpr int DIAG_OFF = 64 * (PB * (PB - 1) / 2);
@@ -422,6 +493,7 @@ __device__ __forceinline__ void left_chain(const omc_nn_dense_t& a, int chain, i
   }
 
   double C[PB][2];   // block column k: C[i] = tile (i, k), i >= k
+  double E[2];       // L_kk^-T of the current step (of the last one, for the backward solve)
   double w[PB];
   rhs_rows<PB>(a, ci, p, chain, g, w);
   __syncwarp();      // the previous chain's reads of the slice are done
@@ -447,16 +519,41 @@ __device__ __forceinline__ void left_chain(const omc_nn_dense_t& a, int chain, i
         wdmma(C[i][0], C[i][1], -ai.y, bk.y);
       }
     }
-    factor_panel<PB>([&](int i) -> double* { return C[i]; }, w, k, g, kq, bad);
+    E[0] = g == 2 * kq ? 1.0 : 0.0;
+    E[1] = g == 2 * kq + 1 ? 1.0 : 0.0;
+    factor_diag(C[k], E, w[k], g, kq, bad);
     if (k + 1 < PB) {
+      // B fragments of E = L_kk^-T: step s needs E[4s + kq][g], held by lane (4s + kq, g >> 1), register g & 1
+      double bf[2];
+#pragma unroll
+      for (int s = 0; s < 2; ++s) {
+        const int src = 4 * (4 * s + kq) + (g >> 1);
+        const double e0 = shf(E[0], src), e1 = shf(E[1], src);
+        bf[s] = (g & 1) ? e1 : e0;
+      }
+      const double wk0 = shf(w[k], 8 * kq), wk1 = shf(w[k], 8 * kq + 4);   // w[k] at 2kq, 2kq + 1
 #pragma unroll
       for (int i = k + 1; i < PB; ++i) {
-        sm[S::off(i, k) + lpos(g, 2 * kq)] = C[i][0];
-        sm[S::off(i, k) + lpos(g, 2 * kq + 1)] = C[i][1];
+        // L(i, k) = C(i, k) L_kk^-T: A = element [g][4s + kq] of C(i, k) (quad-local re-layout)
+        double l0 = 0.0, l1 = 0.0;
+#pragma unroll
+        for (int s = 0; s < 2; ++s) {
+          const int src = 4 * g + 2 * s + (kq >> 1);
+          const double v0 = shf(C[i][0], src), v1 = shf(C[i][1], src);
+          wdmma(l0, l1, (kq & 1) ? v1 : v0, bf[s]);
+        }
+        sm[S::off(i, k) + lpos(g, 2 * kq)] = l0;
+        sm[S::off(i, k) + lpos(g, 2 * kq + 1)] = l1;
+        // w[i] -= L(i, k) w[k]
+        double t = fma(l0, wk0, l1 * wk1);
+        t += shx(t, 1);
+        t += shx(t, 2);
+        w[i] -= t;
       }
-      double* dt = sm + S::DIAG_OFF + 36 * k + g * (g + 1) / 2;
-      if (2 * kq <= g) dt[2 * kq] = C[k][0];
-      if (2 * kq + 1 <= g) dt[2 * kq + 1] = C[k][1];
+      // L_kk^-1 as a packed lower triangle: element [r][c] = E[c][r], r = 2kq + e, c = g
+      double* dt = sm + S::DIAG_OFF + 36 * k + g;
+      if (2 * kq >= g) dt[kq * (2 * kq + 1)] = E[0];
+      if (2 * kq + 1 >= g) dt[(2 * kq + 1) * (kq + 1)] = E[1];
       __syncwarp();
     }
   });
@@ -464,16 +561,16 @@ __device__ __forceinline__ void left_chain(const omc_nn_dense_t& a, int chain, i
   if (bad) return not_pd(a, chain, beta, lane);
   double z0, z1;
   draw_z<PB>(a, p, chain, g, kq, z0, z1);
-  back_solve<PB>(
+  back_solve_inv<PB>(
       beta, p, w, z0, z1, g, kq,
-      [&](int j, int c, double& l0, double& l1) {
-        if (j == PB - 1) {
-          l0 = shf(C[PB - 1][0], 4 * c + kq);
-          l1 = shf(C[PB - 1][1], 4 * c + kq);
-        } else {                                      // above the diagonal (unused): another element of the tile
-          const double* dt = sm + S::DIAG_OFF + 36 * j + c * (c + 1) / 2 + 2 * kq;
-          l0 = dt[0];
-          l1 = dt[1];
+      [&](int j, double& l0, double& l1) {
+        if (j == PB - 1) {                            // E of the last step is L_77^-T: E[g][2kq + e] = L_77^-1[2kq + e][g]
+          l0 = E[0];
+          l1 = E[1];
+        } else {
+          const double* dt = sm + S::DIAG_OFF + 36 * j + g;
+          l0 = 2 * kq >= g ? dt[kq * (2 * kq + 1)] : 0.0;
+          l1 = 2 * kq + 1 >= g ? dt[(2 * kq + 1) * (kq + 1)] : 0.0;
         }
       },
       [&](int j, int tc, int r) { return sm[S::off(j, tc) + lpos(g, 2 * kq + r)]; });
