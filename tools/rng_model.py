@@ -1,17 +1,18 @@
 #!/usr/bin/env python
-"""numpy model of the device normal generator of tridiag.cu / omc_common.cuh (omc_normal_pair_fast): checks the
-log / sincos approximations against libm and the output distribution against N(0,1)."""
+"""numpy model of `normal_from` in tridiag.cu: the fp64 Box-Muller pair built from the omc_logtab.cuh table, a
+degree-7 log series, Taylor sin / cos and the swap and sign bits.  The solve kernel's fp32-assisted generator uses it
+only to redo the pairs whose radius word is below 2^12 (oracle/tridiag_stream.py restates the whole stream on top of
+it).  Run as a script, it checks the log / sincos approximations against libm and the output distribution against
+N(0,1)."""
 import math
-import sys
-
-import numpy as np
-from scipy import stats
-
-sys.path.insert(0, ".")
+import os
 import re
 
+import numpy as np
+
+_LOGTAB = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "openmcmc_b200", "csrc", "omc_logtab.cuh")
 tab = []
-for line in open("openmcmc_b200/csrc/omc_logtab.cuh"):
+for line in open(_LOGTAB):
     m = re.findall(r"0x[0-9a-f.]+p[-+]?\d+", line)
     if len(m) == 2:
         tab.append((float.fromhex(m[0]), float.fromhex(m[1])))
@@ -42,8 +43,10 @@ def clz64(r):
 
 
 def normal_pair(r, a, fast=True):
-    """r = (y << 32) | x, a = (w << 32) | z of the Philox block.  fast=True models normal_pair_fast (valid when y has
-    fewer than 12 leading zeros; the device redoes the other pairs with the slow path), fast=False normal_pair_slow."""
+    """normal_from on the 64-bit radius word r and angle word a = (w << 32) | z.  fast=False is normal_from as
+    normal_pair_f32_slow calls it: r = (w1 << 32) | the second block's word, every bit of r below its leading one
+    feeds the mantissa.  fast=True is the earlier all-fp64 pair generator, which took the 52 low bits of r as the
+    mantissa unless its high word had 12 or more leading zeros; no kernel runs it now."""
     j = clz64(r)
     sh = np.where(j >= 63, np.uint64(0), r << np.minimum(j + 1, 63).astype(np.uint64))
     mb = sh >> np.uint64(12)
@@ -73,6 +76,8 @@ def normal_pair(r, a, fast=True):
 
 
 if __name__ == "__main__":
+    from scipy import stats
+
     rng = np.random.default_rng(1)
     N = 4_000_000
     r = rng.integers(0, 2 ** 64, size=N, dtype=np.uint64)
