@@ -451,9 +451,16 @@ typedef struct {
 } omc_random_walk_t;
 int omc_random_walk(const omc_random_walk_t* args, void* stream);
 
-/* ManifoldMALA: proposal N(theta + 1/2 s^2 H^-1 g, s^2 H^-1) forward and reverse, dense H (n_elem <= 64).
- * ref: metropolis_hastings.py:292-373.  A non-PD Hessian or a NaN (proposal outside the support) REJECTS the move and
- * sets the chain's status bits; the reference raises instead (SURVEY F6). */
+/* ManifoldMALA: proposal N(theta + 1/2 s^2 H^-1 g, s^2 H^-1) forward and reverse.  ref: metropolis_hastings.py:292-373.
+ * Ranges:
+ *   - n_elem <= 64: any model, analytic (method 0) or the reference's finite-difference (method 1) derivatives;
+ *   - 64 < n_elem <= 4096, analytic derivatives of a model whose terms are all sums over elements (Poisson rate, Gamma /
+ *     Uniform response, Normal response with an identity or diagonal precision): diagonal Hessian, O(n) per chain;
+ *   - 64 < n_elem <= 512, any other model (dense Hessian, blocked Cholesky); method 1 only when every term is Normal,
+ *     LogNormal or Normal-linear (whose finite differences the reference replaces by analytic derivatives).
+ *   Anything else returns non-zero.  workspace: see the field.
+ * A non-PD Hessian or a NaN (proposal outside the support) REJECTS the move and sets the chain's status bits; the
+ * reference raises instead (SURVEY F6). */
 typedef struct {
   omc_mh_model_t model;
   double* theta;             /* [n_chains][n_elem] in/out                                               */
@@ -469,6 +476,8 @@ typedef struct {
   double* probe_L;           /* optional [n_chains][n_elem^2] forward proposal Cholesky factor          */
   double* probe_prop;        /* optional [n_chains][n_elem]   proposed point                            */
   double* probe_scalars;     /* optional [n_chains][6]: logp_cur, logp_prop, logq_fwd, logq_rev, log_accept, accepted */
+  double* workspace;         /* dense Hessian above the shared-memory limit (n_elem > 136): omc_nn_dense_workspace(
+                                n_chains, n_elem) doubles; ignored otherwise                            */
 } omc_mmala_t;
 int omc_mmala(const omc_mmala_t* args, void* stream);
 

@@ -187,7 +187,7 @@ class MMalaArgs(C.Structure):
                 ("debug_z", C.c_void_p), ("debug_u", C.c_void_p), ("debug_sweep_stride_z", C.c_longlong),
                 ("debug_sweep_stride_u", C.c_longlong), ("counters", C.c_void_p), ("status", C.c_void_p),
                 ("probe_mu", C.c_void_p), ("probe_L", C.c_void_p), ("probe_prop", C.c_void_p),
-                ("probe_scalars", C.c_void_p)]
+                ("probe_scalars", C.c_void_p), ("workspace", C.c_void_p)]
 
 
 class TridiagNN(C.Structure):

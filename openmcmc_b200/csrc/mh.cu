@@ -2,7 +2,8 @@
 // RandomWalk / RandomWalkLoop (Gaussian and truncated-Gaussian proposals) and ManifoldMALA, batched over chains.
 //
 // Mapping: one WARP per chain for log_p / gradients / random-walk steps (lanes stride over the n_elem parameters, warp
-// shuffles reduce the sums); one CTA per chain for ManifoldMALA (dense Hessian + Cholesky in shared memory).  Chain
+// shuffles reduce the sums); a warp or a CTA per chain for ManifoldMALA (dense Hessian + Cholesky in shared memory to 64
+// parameters, the blocked Cholesky of omc_blocked.cuh to 512, a CTA over the elements of an element-wise model).  Chain
 // state stays in HBM between sweeps; within a kernel it lives in shared memory.  These kernels are latency / FP64-ALU
 // bound (lgamma, log, erfc): bytes per chain-iteration are ~1 KB (DESIGN.md).
 #include "../../include/omc.h"
@@ -12,6 +13,8 @@
 #include "omc_special.cuh"
 
 namespace {
+
+#include "omc_blocked.cuh"
 
 constexpr double LOG_2PI = 1.8378770664093454835606594728112;
 constexpr int MH_WARPS = 4;  // warps (= chains) per CTA in the warp-per-chain kernels
@@ -893,6 +896,451 @@ __global__ void __launch_bounds__(MD_WARPS * 32) mmala_diag_kernel(omc_mmala_t a
   }
 }
 
+// ---- ManifoldMALA above 64 parameters, dense Hessian (64 < n_elem <= 512): one CTA of MB_THREADS per chain on the
+// blocked Cholesky of omc_blocked.cuh.  The augmented matrix [H / step^2 ; g'] lives in shared memory while
+// omc_blocked_workspace_doubles(n) is zero (n <= 136) and in a per-chain global workspace (L2-resident) above, exactly as
+// for the dense conjugate draw.  g rides along as the extra row, so L^-1 g is done when the factorisation ends; one
+// backward solve with the two right-hand sides [L^-1 g, z] gives mu = th + 1/2 (L L')^-1 g and prop = mu + L^-T z.
+// Derivatives are always analytic here: omc_mmala admits method = 1 above 64 only for models whose terms the reference
+// differentiates analytically anyway (model_grad_hess_warp).
+constexpr int MB_THREADS = 256;
+
+// log p of one term at th (n doubles, shared memory) by every thread of the CTA: the expressions of term_logp_warp, with
+// the per-column operand (residual, log-residual or f(theta)) formed once in `col` (n doubles of shared scratch) instead
+// of inside the row loop, and the matrix read by columns (r'P r = r'P'r) so that consecutive threads read consecutive
+// addresses.  Result valid in every thread.
+__device__ double term_logp_block(const omc_term_t& t, int n, int chain, const double* th, double* col, double* red) {
+  const int tid = threadIdx.x, nt = blockDim.x;
+  double acc = 0.0;
+  switch (t.kind) {
+    case OMC_TERM_POISSON_RATE:
+      for (int i = tid; i < n; i += nt) {
+        const double k = vat(t.data, chain, i, 0.0), mu = th[i];
+        double lp = omc_xlogy(k, mu) - lgamma(k + 1.0) - mu;
+        if (!(mu >= 0.0)) lp = nan("");
+        else if (!(k >= 0.0) || floor(k) != k) lp = -INFINITY;
+        acc += lp;
+      }
+      break;
+    case OMC_TERM_GAMMA_RESPONSE:
+      for (int i = tid; i < n; i += nt) {
+        const double x = th[i];
+        const double sh = vat(t.p1, chain, t.p1_len > 1 ? i : 0, 1.0), rt = vat(t.p2, chain, t.p2_len > 1 ? i : 0, 1.0);
+        const double scale = 1.0 / rt, y = x / scale;
+        double lp = omc_xlogy(sh - 1.0, y) - y - lgamma(sh) - log(scale);
+        if (!(y >= 0.0)) lp = isnan(y) ? y : -INFINITY;
+        acc += lp;
+      }
+      break;
+    case OMC_TERM_UNIFORM_RESPONSE:
+      for (int i = tid; i < n; i += nt)
+        acc -= log(vat(t.p2, chain, t.p2_len > 1 ? i : 0, 1.0) - vat(t.p1, chain, t.p1_len > 1 ? i : 0, 0.0));
+      break;
+    case OMC_TERM_NORMAL_RESPONSE:
+    case OMC_TERM_LOGNORMAL_RESPONSE: {
+      const bool logn = t.kind == OMC_TERM_LOGNORMAL_RESPONSE, dense = t.mat_kind == OMC_MAT_DENSE;
+      const double s = vat(t.scalar, chain, 0, 1.0);
+      const double* P = dense ? t.P.ptr + (long long)chain * t.P.chain_stride : nullptr;
+      if (dense) {
+        for (int j = tid; j < n; j += nt)
+          col[j] = (logn ? log(th[j]) : th[j]) - vat(t.p1, chain, t.p1_len > 1 ? j : 0, 0.0);
+        __syncthreads();
+      }
+      bool outside = false;
+      double sumlog = 0.0;
+      for (int i = tid; i < n; i += nt) {
+        const double li = logn ? log(th[i]) : th[i];
+        const double ri = li - vat(t.p1, chain, t.p1_len > 1 ? i : 0, 0.0);
+        if (!logn && (th[i] < t.dom_lo || th[i] > t.dom_hi)) outside = true;
+        double q;
+        if (dense) {
+          q = 0.0;
+          for (int j = 0; j < n; ++j) q += P[(long long)j * n + i] * col[j];
+        } else {
+          q = mat_at(t.mat_kind, t.P, chain, n, i, i) * ri;
+        }
+        acc += ri * q;
+        sumlog += li;
+      }
+      acc = omc_block_sum(acc, red);
+      if (logn) {
+        sumlog = omc_block_sum(sumlog, red);
+        return 0.5 * (n * log(s) + vat(t.logdet, chain, 0, 0.0) - n * LOG_2PI - s * acc) - sumlog;
+      }
+      if (__syncthreads_or(outside)) return -INFINITY;
+      return 0.5 * (n * log(s) + vat(t.logdet, chain, 0, 0.0) - n * LOG_2PI - s * acc);
+    }
+    case OMC_TERM_NORMAL_LINEAR: {
+      const double s = vat(t.scalar, chain, 0, 1.0);
+      const double* rec = t.stats.ptr + (long long)chain * t.stats.chain_stride;
+      const double* G = rec;
+      const double* gv = rec + n * n;
+      for (int k = tid; k < n; k += nt) col[k] = t.transform_exp ? exp(th[k]) : th[k];
+      __syncthreads();
+      for (int j = tid; j < n; j += nt) {
+        double gf = 0.0;
+        for (int k = 0; k < n; ++k) gf = fma(G[(long long)k * n + j], col[k], gf);
+        acc = fma(col[j], gf - 2.0 * gv[j], acc);
+      }
+      const double S = rec[(long long)n * n + n] + omc_block_sum(acc, red);
+      return 0.5 * (t.n_data * log(s) + vat(t.logdet, chain, 0, 0.0) - t.n_data * LOG_2PI - s * S);
+    }
+    default:
+      break;
+  }
+  return omc_block_sum(acc, red);
+}
+
+__device__ double model_logp_block(const omc_mh_model_t& m, int chain, const double* th, double* col, double* red) {
+  double s = 0.0;
+  for (int k = 0; k < m.n_terms; ++k) s += term_logp_block(m.terms[k], m.n_elem, chain, th, col, red);
+  return s;
+}
+
+// [H / step^2 ; g'] at th into W (zeroed first, so the padding the trailing update reads is zero), then the blocked
+// factorisation: on true the lower triangle of W.A holds L and row n holds L^-1 g.  False (uniformly) on a NaN / inf in H
+// or g or a non-positive pivot -- what mmala_params reports.  ref: metropolis_hastings.py:325-348
+__device__ bool mmala_params_blocked(const omc_mmala_t& a, int chain, const double* th, const Workspace& W, int* s_bad) {
+  const int n = a.model.n_elem, tid = threadIdx.x, LD = W.LD;
+  for (long long e = tid; e < (long long)W.rows_pad * LD; e += MB_THREADS) W.A[e] = 0.0;
+  for (int e = tid; e < W.rows_pad * PLD; e += MB_THREADS) W.Pn[e] = 0.0;
+  if (tid == 0) *s_bad = 0;
+  __syncthreads();
+  double* g = W.A + (long long)n * LD;
+  for (int k = 0; k < a.model.n_terms; ++k)   // thread tid owns rows tid, tid + MB_THREADS, ... in every term
+    term_grad_hess_analytic(a.model.terms[k], n, chain, th, g, W.A, LD, tid, MB_THREADS);
+  const double inv_s2 = 1.0 / (a.step * a.step);
+  bool bad = false;
+  for (int r = tid; r < n; r += MB_THREADS) {
+    double* row = W.A + (long long)r * LD;
+    for (int c = 0; c < n; ++c) {
+      const double v = row[c] * inv_s2;     // precision_cr = hessian_cr / step**2
+      row[c] = v;
+      if (isnan(v) || isinf(v)) bad = true;
+    }
+    if (isnan(g[r]) || isinf(g[r])) bad = true;
+  }
+  if (__syncthreads_or(bad)) return false;
+  return blocked_cholesky<MB_THREADS>(W, n, 1, s_bad);
+}
+
+// log N(x | mu, (L L')^-1) up to the constant the reference drops: sum log diag L - 1/2 |L'(x - mu)|^2, L in W.A and
+// r = x - mu in shared memory; thread i forms (L'r)_i = sum_{j >= i} L_ji r_j (consecutive threads, consecutive
+// addresses).  ref: metropolis_hastings.py:350-373
+__device__ double mmala_log_density_blocked(const Workspace& W, int n, const double* r, double* red) {
+  double ld = 0.0, ww = 0.0;
+  for (int i = threadIdx.x; i < n; i += MB_THREADS) {
+    double w = 0.0;
+    for (int j = i; j < n; ++j) w = fma(W.A[(long long)j * W.LD + i], r[j], w);
+    ww = fma(w, w, ww);
+    ld += log(W.A[(long long)i * W.LD + i]);
+  }
+  ld = omc_block_sum(ld, red);
+  ww = omc_block_sum(ww, red);
+  return ld - 0.5 * ww;
+}
+
+template <bool GLOBAL_A>
+__global__ void __launch_bounds__(MB_THREADS) mmala_blocked_kernel(omc_mmala_t a) {
+  extern __shared__ __align__(16) double sm[];
+  __shared__ int s_bad;
+  __shared__ double red[32];
+  const int n = a.model.n_elem, chain = blockIdx.x, tid = threadIdx.x;
+  const int pp = (n + 15) & ~15;
+  double* rest;
+  const Workspace W = carve(sm, GLOBAL_A ? a.workspace + (long long)chain * (((n + 1 + 7) & ~7) * (long long)(pp + 4)) : nullptr, n, 1,
+                            &rest);
+  double* cur = rest;          // pp
+  double* prop = cur + pp;     // pp
+  double* mu = prop + pp;      // pp: forward, then reverse proposal mean
+  double* X = mu + pp;         // 2 x pp: L^-1 g -> (L L')^-1 g | z -> L^-T z
+  double* col = X + 2 * pp;    // pp: residuals of the log-densities
+  const int LD = W.LD;
+  double* gth = a.theta + (long long)chain * n;
+  for (int i = tid; i < n; i += MB_THREADS) cur[i] = gth[i];
+  __syncthreads();
+  const long long sw = a.rng.sweep ? (long long)(*a.rng.sweep) : 0ll;
+  const OmcRng rng = to_rng(a.rng);
+  int status = 0;
+  double lpc = 0.0, lpp = 0.0, lq = 0.0, lqr = 0.0;
+  bool ok = mmala_params_blocked(a, chain, cur, W, &s_bad);
+  if (!ok) status |= OMC_STATUS_NOT_PD;
+  if (ok) {
+    // z (pair t holds elements 2t, 2t + 1), then mu = th + 1/2 L^-T (L^-1 g) and prop = mu + L^-T z
+    if (a.debug_z) {
+      const double* dz = a.debug_z + sw * a.debug_sweep_stride_z + (long long)chain * n;
+      for (int i = tid; i < n; i += MB_THREADS) X[pp + i] = dz[i];
+    } else {
+      for (int t = tid; 2 * t < n; t += MB_THREADS) {
+        double z0, z1;
+        omc_normal2(rng, chain, t, z0, z1);
+        X[pp + 2 * t] = z0;
+        if (2 * t + 1 < n) X[pp + 2 * t + 1] = z1;
+      }
+    }
+    for (int i = tid; i < n; i += MB_THREADS) X[i] = W.A[(long long)n * LD + i];
+    __syncthreads();
+    blocked_backsolve<MB_THREADS>(W, n, X, pp, 2);
+    for (int i = tid; i < n; i += MB_THREADS) {
+      mu[i] = cur[i] + 0.5 * X[i];
+      prop[i] = X[pp + i] + mu[i];
+      col[i] = prop[i] - mu[i];
+    }
+    __syncthreads();
+    lq = mmala_log_density_blocked(W, n, col, red);
+    if (a.probe_mu) for (int i = tid; i < n; i += MB_THREADS) a.probe_mu[(long long)chain * n + i] = mu[i];
+    if (a.probe_prop) for (int i = tid; i < n; i += MB_THREADS) a.probe_prop[(long long)chain * n + i] = prop[i];
+    if (a.probe_L)
+      for (int r = 0; r < n; ++r)
+        for (int c = tid; c < n; c += MB_THREADS)
+          a.probe_L[(long long)chain * n * n + (long long)r * n + c] = (c <= r) ? W.A[(long long)r * LD + c] : 0.0;
+    lpc = model_logp_block(a.model, chain, cur, col, red);
+    lpp = model_logp_block(a.model, chain, prop, col, red);
+    __syncthreads();
+    // reverse proposal parameters at the proposed point
+    const bool ok2 = mmala_params_blocked(a, chain, prop, W, &s_bad);
+    if (!ok2) { status |= OMC_STATUS_OUT_OF_SUPPORT; ok = false; }   // invalid PROPOSAL: reject, chain stays healthy
+    else {
+      for (int i = tid; i < n; i += MB_THREADS) X[i] = W.A[(long long)n * LD + i];
+      __syncthreads();
+      blocked_backsolve<MB_THREADS>(W, n, X, pp, 1);
+      for (int i = tid; i < n; i += MB_THREADS) col[i] = cur[i] - (prop[i] + 0.5 * X[i]);
+      __syncthreads();
+      lqr = mmala_log_density_blocked(W, n, col, red);
+    }
+  }
+  bool accept = false;
+  double log_accept = nan("");
+  if (ok) {
+    double u;
+    if (a.debug_u) u = a.debug_u[sw * a.debug_sweep_stride_u + chain];
+    else {
+      uint4 b = omc_rng_block(rng, chain, 0xFFFFu);
+      u = omc_u01(b.x, b.y);
+    }
+    log_accept = lpp + lqr - (lpc + lq);
+    accept = log(u) < log_accept;
+    if (isnan(log_accept)) status |= isnan(lpc) ? OMC_STATUS_NAN : OMC_STATUS_OUT_OF_SUPPORT;
+  }
+  if (accept)
+    for (int i = tid; i < n; i += MB_THREADS) gth[i] = prop[i];
+  if (tid == 0) {
+    if (a.counters) {
+      a.counters[2 * (long long)chain] += accept ? 1 : 0;
+      a.counters[2 * (long long)chain + 1] += 1;
+    }
+    if (a.status && status) atomicOr(&a.status[chain], status);
+    if (a.probe_scalars) {
+      double* ps = a.probe_scalars + (long long)chain * 6;
+      ps[0] = lpc; ps[1] = lpp; ps[2] = lq; ps[3] = lqr; ps[4] = log_accept; ps[5] = accept ? 1.0 : 0.0;
+    }
+  }
+}
+
+size_t mmala_blocked_smem(int n, bool global_A) {
+  const int pp = (n + 15) & ~15, LD = pp + 4, rows_pad = (n + 1 + 7) & ~7;
+  size_t d = (size_t)rows_pad * PLD + NB * SDLD + 3 + pp /*sinv*/ + 6 * (size_t)pp;
+  if (!global_A) d += (size_t)rows_pad * LD;
+  return d * sizeof(double);
+}
+
+// ---- ManifoldMALA above 64 elements on a model whose terms are all sums over elements (64 < n_elem <= MDW_MAX): the
+// step of mmala_diag_kernel with one CTA per chain.  Thread tid owns the element pairs t = tid + k * MDW_THREADS
+// (elements 2t, 2t + 1), so each pair's normals come from one Philox block, as in every other ManifoldMALA kernel.  The
+// proposal of its (at most 2 * MDW_PAIRS) elements stays in registers until the accept decision; state, L and mu are
+// per-element temporaries.  Nothing passes through shared memory except the one block reduction of the per-chain sums
+// and flags, and the proposal is written only where accepted.
+// Cap: 2 * MDW_PAIRS * MDW_THREADS = 4096 elements, 16 per thread, keeps the proposal array register-resident at 256
+// threads next to the per-element temporaries.  The normal pairs use Philox blocks 0 .. n/2 - 1, which must stay below block 0xFFFF (the accept
+// uniform's), so a cap above 131070 elements would need a different block layout, not just more pairs per thread.
+constexpr int MDW_THREADS = 256;
+constexpr int MDW_PAIRS = 8;
+constexpr int MDW_MAX = 2 * MDW_PAIRS * MDW_THREADS;
+constexpr int MDW_NSUM = 8;
+
+// element e's share of log p at x, summed over the terms: the per-element expressions of term_logp_warp; a Normal term
+// contributes -1/2 s r q here and its constant 1/2 (n log s + logdet - n log 2 pi) once per chain (elem_logp_const)
+__device__ __forceinline__ double elem_logp(const omc_mh_model_t& m, int n, int chain, int e, double x) {
+  double lp = 0.0;
+  for (int k = 0; k < m.n_terms; ++k) {
+    const omc_term_t& t = m.terms[k];
+    switch (t.kind) {
+      case OMC_TERM_POISSON_RATE: {
+        const double kk = vat(t.data, chain, e, 0.0);
+        double l = omc_xlogy(kk, x) - lgamma(kk + 1.0) - x;
+        if (!(x >= 0.0)) l = nan("");
+        else if (!(kk >= 0.0) || floor(kk) != kk) l = -INFINITY;
+        lp += l;
+        break;
+      }
+      case OMC_TERM_GAMMA_RESPONSE: {
+        const double sh = vat(t.p1, chain, t.p1_len > 1 ? e : 0, 1.0), rt = vat(t.p2, chain, t.p2_len > 1 ? e : 0, 1.0);
+        const double scale = 1.0 / rt, y = x / scale;
+        double l = omc_xlogy(sh - 1.0, y) - y - lgamma(sh) - log(scale);
+        if (!(y >= 0.0)) l = isnan(y) ? y : -INFINITY;
+        lp += l;
+        break;
+      }
+      case OMC_TERM_NORMAL_RESPONSE: {
+        if (x < t.dom_lo || x > t.dom_hi) { lp += -INFINITY; break; }
+        const double ri = x - vat(t.p1, chain, t.p1_len > 1 ? e : 0, 0.0);
+        const double q = mat_at(t.mat_kind, t.P, chain, n, e, e) * ri;
+        lp += -0.5 * vat(t.scalar, chain, 0, 1.0) * (ri * q);
+        break;
+      }
+      case OMC_TERM_UNIFORM_RESPONSE:
+        lp -= log(vat(t.p2, chain, t.p2_len > 1 ? e : 0, 1.0) - vat(t.p1, chain, t.p1_len > 1 ? e : 0, 0.0));
+        break;
+      default:
+        break;
+    }
+  }
+  return lp;
+}
+__device__ double elem_logp_const(const omc_mh_model_t& m, int n, int chain) {
+  double c = 0.0;
+  for (int k = 0; k < m.n_terms; ++k) {
+    const omc_term_t& t = m.terms[k];
+    if (t.kind == OMC_TERM_NORMAL_RESPONSE)
+      c += 0.5 * (n * log(vat(t.scalar, chain, 0, 1.0)) + vat(t.logdet, chain, 0, 0.0) - n * LOG_2PI);
+  }
+  return c;
+}
+
+// element e's proposal parameters at x (mmala_params_diag without the warp vote): false when NaN / inf or not positive
+__device__ __forceinline__ bool elem_params(const omc_mmala_t& a, int n, int chain, int e, double x, double& L,
+                                            double& mu) {
+  double g, h;
+  elem_grad_hess(a.model, n, chain, e, x, g, h);
+  const double v = h * (1.0 / (a.step * a.step));
+  const bool bad = isnan(v) || isinf(v) || isnan(g) || isinf(g) || !(v > 0.0);
+  L = sqrt(v);
+  double x0 = g / L;
+  x0 = x0 / L;
+  mu = x + 0.5 * x0;
+  return !bad;
+}
+
+__global__ void __launch_bounds__(MDW_THREADS) mmala_diag_wide_kernel(omc_mmala_t a) {
+  __shared__ double red[MDW_THREADS / 32][MDW_NSUM];
+  const int n = a.model.n_elem, chain = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  double* gth = a.theta + (long long)chain * n;
+  const long long sw = a.rng.sweep ? (long long)(*a.rng.sweep) : 0ll;
+  const OmcRng rng = to_rng(a.rng);
+  const double* dz = a.debug_z ? a.debug_z + sw * a.debug_sweep_stride_z + (long long)chain * n : nullptr;
+  double xp[2 * MDW_PAIRS];    // the proposal; the probes recompute L and mu from the (unchanged) state
+  // s: logp_cur, logp_prop, sum log L, |L'(prop - mu)|^2, reverse sum log L, |L2'(cur - mu2)|^2, bad fwd, bad rev
+  double s[MDW_NSUM] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+#pragma unroll
+  for (int k = 0; k < MDW_PAIRS; ++k) {
+    const int t = tid + k * MDW_THREADS;
+    double z[2] = {0.0, 0.0};
+    if (2 * t < n) {
+      if (dz) {
+        z[0] = dz[2 * t];
+        if (2 * t + 1 < n) z[1] = dz[2 * t + 1];
+      } else {
+        omc_normal2(rng, chain, t, z[0], z[1]);
+      }
+    }
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int q = 2 * k + h, e = 2 * t + h;
+      xp[q] = 0.0;
+      if (e < n) {
+        const double xc = gth[e];
+        double L, mu;
+        if (!elem_params(a, n, chain, e, xc, L, mu)) s[6] = 1.0;
+        xp[q] = z[h] / L + mu;
+        const double w = L * (xp[q] - mu);
+        s[2] += log(L);
+        s[3] += w * w;
+        double L2, mu2;
+        if (!elem_params(a, n, chain, e, xp[q], L2, mu2)) s[7] = 1.0;
+        const double w2 = L2 * (xc - mu2);
+        s[4] += log(L2);
+        s[5] += w2 * w2;
+        s[0] += elem_logp(a.model, n, chain, e, xc);
+        s[1] += elem_logp(a.model, n, chain, e, xp[q]);
+      }
+    }
+  }
+#pragma unroll
+  for (int v = 0; v < MDW_NSUM; ++v) s[v] = omc_warp_sum(s[v]);
+  if (lane == 0)
+#pragma unroll
+    for (int v = 0; v < MDW_NSUM; ++v) red[warp][v] = s[v];
+  __syncthreads();
+#pragma unroll
+  for (int v = 0; v < MDW_NSUM; ++v) {
+    s[v] = 0.0;
+    for (int w = 0; w < MDW_THREADS / 32; ++w) s[v] += red[w][v];
+  }
+  int status = 0;
+  bool ok = s[6] == 0.0;
+  if (!ok) status |= OMC_STATUS_NOT_PD;
+  const double lc = ok ? elem_logp_const(a.model, n, chain) : 0.0;
+  const double lpc = ok ? s[0] + lc : 0.0, lpp = ok ? s[1] + lc : 0.0, lq = ok ? s[2] - 0.5 * s[3] : 0.0;
+  double lqr = 0.0;
+  if (ok) {
+    if (s[7] != 0.0) { status |= OMC_STATUS_OUT_OF_SUPPORT; ok = false; }
+    else lqr = s[4] - 0.5 * s[5];
+  }
+  bool accept = false;
+  double log_accept = nan("");
+  if (ok) {
+    double u;
+    if (a.debug_u) u = a.debug_u[sw * a.debug_sweep_stride_u + chain];
+    else {
+      uint4 b = omc_rng_block(rng, chain, 0xFFFFu);
+      u = omc_u01(b.x, b.y);
+    }
+    log_accept = lpp + lqr - (lpc + lq);
+    accept = log(u) < log_accept;
+    if (isnan(log_accept)) status |= isnan(lpc) ? OMC_STATUS_NAN : OMC_STATUS_OUT_OF_SUPPORT;
+  }
+  // probes of a valid forward proposal (the L probe is the dense n x n factor: zeros, then the diagonal)
+  if (s[6] == 0.0) {
+    if (a.probe_L) {
+      double* pl = a.probe_L + (long long)chain * n * n;
+      for (long long e = tid; e < (long long)n * n; e += MDW_THREADS) pl[e] = 0.0;
+      __syncthreads();
+    }
+#pragma unroll
+    for (int k = 0; k < MDW_PAIRS; ++k)
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int q = 2 * k + h, e = 2 * (tid + k * MDW_THREADS) + h;
+        if (e < n) {
+          double L, mu;
+          elem_params(a, n, chain, e, gth[e], L, mu);
+          if (a.probe_mu) a.probe_mu[(long long)chain * n + e] = mu;
+          if (a.probe_prop) a.probe_prop[(long long)chain * n + e] = xp[q];
+          if (a.probe_L) a.probe_L[(long long)chain * n * n + (long long)e * n + e] = L;
+        }
+      }
+  }
+  if (accept)
+#pragma unroll
+    for (int k = 0; k < MDW_PAIRS; ++k)
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int q = 2 * k + h, e = 2 * (tid + k * MDW_THREADS) + h;
+        if (e < n) gth[e] = xp[q];
+      }
+  if (tid == 0) {
+    if (a.counters) {
+      a.counters[2 * (long long)chain] += accept ? 1 : 0;
+      a.counters[2 * (long long)chain + 1] += 1;
+    }
+    if (a.status && status) atomicOr(&a.status[chain], status);
+    if (a.probe_scalars) {
+      double* ps = a.probe_scalars + (long long)chain * 6;
+      ps[0] = lpc; ps[1] = lpp; ps[2] = lq; ps[3] = lqr; ps[4] = log_accept; ps[5] = accept ? 1.0 : 0.0;
+    }
+  }
+}
+
 __global__ void truncnorm_rv_kernel(const double* mean, const double* scale, const double* lower, const double* upper,
                                     const double* u, long long n, double* out) {
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -913,8 +1361,48 @@ int check_model(const omc_mh_model_t* m, const char* who) {
     if (t.kind == OMC_TERM_NORMAL_RESPONSE || t.kind == OMC_TERM_LOGNORMAL_RESPONSE)
       OMC_REQUIRE(t.mat_kind == OMC_MAT_EYE || t.P.ptr, "%s: Normal term without precision", who);
     if (t.kind == OMC_TERM_NORMAL_LINEAR)
-      OMC_REQUIRE(t.stats.ptr && t.n_data >= 1 && m->n_elem <= 64, "%s: Normal-linear term needs a regression record", who);
+      OMC_REQUIRE(t.stats.ptr && t.n_data >= 1 && m->n_elem <= 512,
+                  "%s: Normal-linear term needs a regression record (n_elem <= 512)", who);
   }
+  return 0;
+}
+
+// n_elem > 64: the element-wise kernel for analytic derivatives of a model whose terms are all sums over elements (up
+// to MDW_MAX), the blocked dense kernel otherwise (up to 512).  Finite differences are admitted only where they equal
+// the analytic derivatives (every term Normal, LogNormal or Normal-linear): the in-kernel FD Hessian costs 4 n^2
+// log-density evaluations.
+int launch_mmala_wide(const omc_mmala_t& a, cudaStream_t st) {
+  const int n = a.model.n_elem;
+  bool separable = (a.method == 0), fd_exact = true;
+  for (int k = 0; k < a.model.n_terms; ++k) {
+    const omc_term_t& t = a.model.terms[k];
+    separable = separable && (t.kind == OMC_TERM_POISSON_RATE || t.kind == OMC_TERM_GAMMA_RESPONSE ||
+                              t.kind == OMC_TERM_UNIFORM_RESPONSE ||
+                              (t.kind == OMC_TERM_NORMAL_RESPONSE && t.mat_kind != OMC_MAT_DENSE));
+    fd_exact = fd_exact && (t.kind == OMC_TERM_NORMAL_RESPONSE || t.kind == OMC_TERM_LOGNORMAL_RESPONSE ||
+                            t.kind == OMC_TERM_NORMAL_LINEAR);
+  }
+  if (separable) {
+    OMC_REQUIRE(n <= MDW_MAX, "omc_mmala: element-wise model with n_elem=%d > %d is not supported", n, MDW_MAX);
+    mmala_diag_wide_kernel<<<a.model.n_chains, MDW_THREADS, 0, st>>>(a);
+    OMC_LAUNCH_CHECK();
+    return 0;
+  }
+  OMC_REQUIRE(n <= 512, "omc_mmala: dense-Hessian model with n_elem=%d > 512 is not supported", n);
+  OMC_REQUIRE(a.method == 0 || fd_exact,
+              "omc_mmala: finite-difference derivatives above 64 parameters need every term Normal, LogNormal or "
+              "Normal-linear (n_elem=%d)", n);
+  const bool global_A = omc_blocked_workspace_doubles(n) > 0;
+  OMC_REQUIRE(!global_A || a.workspace, "omc_mmala: n_elem=%d needs a workspace of omc_nn_dense_workspace() doubles", n);
+  const size_t smem = mmala_blocked_smem(n, global_A);
+  if (global_A) {
+    OMC_CHECK_CUDA(cudaFuncSetAttribute(mmala_blocked_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    mmala_blocked_kernel<true><<<a.model.n_chains, MB_THREADS, smem, st>>>(a);
+  } else {
+    OMC_CHECK_CUDA(cudaFuncSetAttribute(mmala_blocked_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    mmala_blocked_kernel<false><<<a.model.n_chains, MB_THREADS, smem, st>>>(a);
+  }
+  OMC_LAUNCH_CHECK();
   return 0;
 }
 
@@ -971,8 +1459,8 @@ int omc_mmala(const omc_mmala_t* a, void* stream) {
   OMC_REQUIRE(a && a->theta, "omc_mmala: null argument");
   if (int rc = check_model(&a->model, "omc_mmala")) return rc;
   const int n = a->model.n_elem;
-  OMC_REQUIRE(n <= 64, "omc_mmala: n_elem=%d > 64 is not supported", n);
   OMC_REQUIRE(a->step > 0.0, "omc_mmala: step=%g", a->step);
+  if (n > 64) return launch_mmala_wide(*a, (cudaStream_t)stream);
   const size_t smem = (size_t)(n * (n + 1) + 8 * n) * sizeof(double);
   bool separable = (a->method == 0);   // analytic derivatives of a model whose terms are sums over elements
   for (int k = 0; k < a->model.n_terms; ++k) {

@@ -515,7 +515,8 @@ def random_walk(model, theta, p_dim, n_rep, loop, step, step_rows, step_cols, li
 
 
 def mmala(model, theta, step, method, rng_, debug_z=None, debug_u=None, stride_z=0, stride_u=0, counters=None,
-          status=None, probe_mu=None, probe_L=None, probe_prop=None, probe_scalars=None):
+          status=None, probe_mu=None, probe_L=None, probe_prop=None, probe_scalars=None, workspace=None):
+    """workspace: nn_dense_workspace(n_chains, n_elem) doubles when that is > 0 (dense Hessian above n_elem = 136)."""
     a = _cabi.MMalaArgs()
     a.model = model
     a.theta = theta.data_ptr()
@@ -525,7 +526,7 @@ def mmala(model, theta, step, method, rng_, debug_z=None, debug_u=None, stride_z
     a.debug_u = debug_u.data_ptr() if debug_u is not None else None
     a.debug_sweep_stride_z, a.debug_sweep_stride_u = int(stride_z), int(stride_u)
     for name, t in (("counters", counters), ("status", status), ("probe_mu", probe_mu), ("probe_L", probe_L),
-                    ("probe_prop", probe_prop), ("probe_scalars", probe_scalars)):
+                    ("probe_prop", probe_prop), ("probe_scalars", probe_scalars), ("workspace", workspace)):
         setattr(a, name, t.data_ptr() if t is not None else None)
     check(lib().omc_mmala(C.byref(a), stream_ptr()), "omc_mmala")
 

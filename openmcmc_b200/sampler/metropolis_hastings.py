@@ -252,6 +252,34 @@ class ManifoldMALA(MetropolisHastings):
         plan.emit(launch, f"rj_coef_mmala[{self.param}]")
         plan.wrote(self.param)
 
+    @staticmethod
+    def _wide_workspace(plan, model, n, method):
+        """Above 64 parameters (omc.h, omc_mmala): an element-wise model (every term a sum over elements, analytic
+        derivatives) runs up to 4096 elements; any other model runs its dense Hessian through the blocked Cholesky up to
+        p = 512, with finite differences only where the reference itself is analytic (Normal, LogNormal, Normal-linear
+        terms).  Returns the per-plan factor workspace the dense path needs above p = 136, or None."""
+        from openmcmc_b200 import engine
+        from openmcmc_b200 import kernels as K
+
+        terms = [model.terms[i] for i in range(model.n_terms)]
+        separable = method == 0 and all(
+            t.kind in (K.TERM_POISSON_RATE, K.TERM_GAMMA_RESPONSE, K.TERM_UNIFORM_RESPONSE)
+            or (t.kind == K.TERM_NORMAL_RESPONSE and t.mat_kind != K.MAT_DENSE) for t in terms)
+        if separable:
+            if n > 4096:
+                raise engine.PlanError(f"ManifoldMALA on an element-wise model with n={n} > 4096 elements is not "
+                                       "supported by the device path")
+            return None
+        if n > 512:
+            raise engine.PlanError(f"ManifoldMALA with a dense Hessian and p={n} > 512 parameters is not supported by "
+                                   "the device path")
+        if method == 1 and any(t.kind not in (K.TERM_NORMAL_RESPONSE, K.TERM_LOGNORMAL_RESPONSE, K.TERM_NORMAL_LINEAR)
+                               for t in terms):
+            raise engine.PlanError(f"ManifoldMALA with derivatives='fd' and p={n} > 64 parameters needs every term "
+                                   "Normal, LogNormal or Normal-linear; use derivatives='analytic'")
+        ws = K.nn_dense_workspace(plan.state.n_chains, n)
+        return plan.new(ws) if ws > 0 else None
+
     def compile(self, plan, host_state, debug_draws=None):
         from openmcmc_b200 import devdist, engine
         from openmcmc_b200 import kernels as K
@@ -267,12 +295,12 @@ class ManifoldMALA(MetropolisHastings):
         if theta.cols != 1:
             raise engine.PlanError("ManifoldMALA on the device needs a (p, 1) parameter")
         n = theta.rows
-        if n > 64:
-            raise engine.PlanError(f"ManifoldMALA with p={n} > 64 parameters is not supported by the device path")
         step = np.asarray(self.step, dtype=np.float64)
         if step.size != 1:
             raise engine.PlanError("ManifoldMALA on the device needs a scalar step")
+        method = 1 if self.derivatives == "fd" else 0
         model, _ = devdist.build_terms(plan, host_state, self.model, self.param)
+        workspace = self._wide_workspace(plan, model, n, method) if n > 64 else None
         ctx = self._mh_context(plan, 1, n, debug_draws)
         if "probes" not in ctx:
             ctx["probes"] = None
@@ -281,13 +309,12 @@ class ManifoldMALA(MetropolisHastings):
                                  "scalars": plan.new(C, 6)}
                 plan.probes[self.param] = ctx["probes"]
         pr = ctx["probes"] or {}
-        method = 1 if self.derivatives == "fd" else 0
 
         def launch():
             K.mmala(model, theta.data, float(step.item()), method, ctx["rng"], debug_z=ctx["dz"], debug_u=ctx["du"],
                     stride_z=ctx["dz_stride"], stride_u=ctx["du_stride"], counters=ctx["counters"], status=plan.status,
                     probe_mu=pr.get("mu"), probe_L=pr.get("L"), probe_prop=pr.get("prop"),
-                    probe_scalars=pr.get("scalars"))
+                    probe_scalars=pr.get("scalars"), workspace=workspace)
 
         plan.emit(launch, f"mmala[{self.param}]")
         plan.wrote(self.param)
