@@ -14,11 +14,13 @@
 //   tile).  At p = 64 it needs 254 registers per thread: 8 chains per SM.
 // * Left-looking kernel (nn_left_draw_kernel, larger p; dense_draw.cu selects): only block column k in registers
 //   (<= 16 doubles per lane, read from the record at the top of step k), the finished factor in the warp's slice of
-//   shared memory.  Step k: C(i, k) = Q(i, k) - sum_{j<k} L(i, j) L(k, j)', i >= k, on the tensor pipe with both operand
-//   fragments (element [g][4s + kq] of a tile) read straight from shared memory; the pivot stages of the diagonal tile
-//   alone, an identity tile riding along and coming out as L_kk^-T; the panel L(i, k) = C(i, k) L_kk^-T as two DMMAs
-//   per tile and w[i] -= L(i, k) w[k] as a mat-vec; L(:, k), with L_kk^-1 in place of L_kk, back to shared memory.  The
-//   backward solve is then one 8 x 8 mat-vec per block instead of 8 dependent substitution steps.  The pivot stages
+//   shared memory.  Step k: C(i, k) = Q(i, k) - sum_{j<k} L(i, j) L(k, j)', i >= k, on the tensor pipe, summed from
+//   zero with Q's tile added last (the record's latency hides behind the products); the products take a tile's k
+//   index as 2kq + s in m8n8k4 step s, so both operand fragments are a lane's own accumulator element [g][2kq + s],
+//   read as one 16-byte load per lane; the pivot stages of the diagonal tile alone, an identity tile riding along and
+//   coming out as L_kk^-T; the panel L(i, k) = C(i, k) L_kk^-T as two DMMAs per tile straight from C's registers and
+//   w[i] -= L(i, k) w[k] as a mat-vec; L(:, k), with L_kk^-1 in place of L_kk, back to shared memory; the rss epilogue
+//   takes d from the backward solve's registers.  The backward solve is then one 8 x 8 mat-vec per block instead of 8 dependent substitution steps.  The pivot stages
 //   no longer touch the off-diagonal tiles (224 of the 288 tile updates at p = 64, shuffle + 3 FMAs + select each).
 //   At p = 64: 128 registers and 16,352 bytes of shared memory per warp, 14 chains per SM,
 //   persistent warps, the next chain's record prefetched into L2 while the current one runs.  (A register copy of
@@ -302,10 +304,11 @@ __device__ __forceinline__ void back_solve(double* beta, int p, const double (&w
 
 // Backward solve L' x = w + z with the inverted diagonal blocks, x -> beta: x_j = L_jj^-T v_j is one 8 x 8 mat-vec
 // (lane-local) and a quad reduction, which leaves x_j in row layout (x[8j + g]), the form the off-diagonal updates
-// take.  linv(j, l0, l1): L_jj^-1[2kq][g], L_jj^-1[2kq+1][g] (0 above the diagonal); loff as in back_solve.
+// take.  linv(j, l0, l1): L_jj^-1[2kq][g], L_jj^-1[2kq+1][g] (0 above the diagonal); loff(j, tc): L(j, tc)[g][2kq],
+// L(j, tc)[g][2kq + 1] as one double2, tc < j.  xr[j] = x[8j + g] stays behind for the rss epilogue.
 template <int PB, class Inv, class Off>
 __device__ __forceinline__ void back_solve_inv(double* beta, int p, const double (&w)[PB], double z0, double z1, int g,
-                                               int kq, Inv linv, Off loff) {
+                                               int kq, Inv linv, Off loff, double (&xr)[PB]) {
   double racc[PB][2];
   solve_rhs<PB>(racc, w, z0, z1, g, kq);
 #pragma unroll
@@ -320,10 +323,12 @@ __device__ __forceinline__ void back_solve_inv(double* beta, int p, const double
     xg += shx(xg, 1);
     xg += shx(xg, 2);                                           // x[8j + g], the same bits in all four lanes
     if (kq == 0 && 8 * j + g < p) beta[8 * j + g] = xg;
+    xr[j] = xg;
 #pragma unroll
     for (int tc = 0; tc < j; ++tc) {
-      racc[tc][0] = fma(-loff(j, tc, 0), xg, racc[tc][0]);
-      racc[tc][1] = fma(-loff(j, tc, 1), xg, racc[tc][1]);
+      const double2 l = loff(j, tc);
+      racc[tc][0] = fma(-l.x, xg, racc[tc][0]);
+      racc[tc][1] = fma(-l.y, xg, racc[tc][1]);
     }
   }
 }
@@ -339,22 +344,18 @@ __device__ __forceinline__ void not_pd(const omc_nn_dense_t& a, int chain, doubl
   for (int c = lane; c < a.p; c += 32) beta[c] = nan("");
 }
 
-// rss(beta) = rss0 - 2 d'c0 + d'G d  (omc.h), d = beta - beta_hat; beta is read back through L2, G from the record
-// again (not as |L'd|^2 - lam d'P0 d, which would carry the factorisation's backward error, ~cond(Q))
+// rss(beta) = rss0 - 2 d'c0 + d'G d  (omc.h), d = beta - beta_hat from the centre record cen, G from the record again
+// (not as |L'd|^2 - lam d'P0 d, which would carry the factorisation's backward error, ~cond(Q)).  dcol[j][r] =
+// d[8j + 2kq + r], drow[j] = d[8j + g], 0 past p.
 template <int PB, bool VEC>
-__device__ __forceinline__ void rss_epilogue(const omc_nn_dense_t& a, int p, int chain, const double* __restrict__ rec,
-                                             const double* beta, int lane) {
+__device__ __forceinline__ void rss_sum(const omc_nn_dense_t& a, int p, int chain, const double* __restrict__ rec,
+                                        const double* cen, const double (&dcol)[PB][2], const double (&drow)[PB],
+                                        int lane) {
   const int g = lane >> 2, kq = lane & 3;
-  __syncwarp();
-  const double* cen = a.center.ptr + (long long)chain * a.center.chain_stride;
   double acc = 0.0;
-  double dcol[PB][2], drow[PB];
 #pragma unroll
   for (int j = 0; j < PB; ++j) {
-    const int e0 = 8 * j + 2 * kq, er = 8 * j + g;
-    dcol[j][0] = e0 < p ? __ldcg(beta + e0) - cen[e0] : 0.0;
-    dcol[j][1] = e0 + 1 < p ? __ldcg(beta + e0 + 1) - cen[e0 + 1] : 0.0;
-    drow[j] = er < p ? __ldcg(beta + er) - cen[er] : 0.0;
+    const int e0 = 8 * j + 2 * kq;
     if (g == 0) {
       if (e0 < p) acc = fma(-2.0 * cen[p + e0], dcol[j][0], acc);
       if (e0 + 1 < p) acc = fma(-2.0 * cen[p + e0 + 1], dcol[j][1], acc);
@@ -383,6 +384,24 @@ __device__ __forceinline__ void rss_epilogue(const omc_nn_dense_t& a, int p, int
     }
   acc = omc_warp_sum(acc);
   if (lane == 0) a.rss_out[(long long)chain * a.stats.chain_stride] = cen[2 * p] + acc;
+}
+
+// rss epilogue of the register kernel: beta is read back through L2
+template <int PB, bool VEC>
+__device__ __forceinline__ void rss_epilogue(const omc_nn_dense_t& a, int p, int chain, const double* __restrict__ rec,
+                                             const double* beta, int lane) {
+  const int g = lane >> 2, kq = lane & 3;
+  __syncwarp();
+  const double* cen = a.center.ptr + (long long)chain * a.center.chain_stride;
+  double dcol[PB][2], drow[PB];
+#pragma unroll
+  for (int j = 0; j < PB; ++j) {
+    const int e0 = 8 * j + 2 * kq, er = 8 * j + g;
+    dcol[j][0] = e0 < p ? __ldcg(beta + e0) - cen[e0] : 0.0;
+    dcol[j][1] = e0 + 1 < p ? __ldcg(beta + e0 + 1) - cen[e0 + 1] : 0.0;
+    drow[j] = er < p ? __ldcg(beta + er) - cen[er] : 0.0;
+  }
+  rss_sum<PB, VEC>(a, p, chain, rec, cen, dcol, drow, lane);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -454,16 +473,15 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, ctas_per_sm<PB>()) nn_warp
 // Left-looking kernel.  Shared-memory slice of one warp: the PB(PB-1)/2 off-diagonal tiles of L full, then the PB-1
 // first diagonal blocks' INVERSES L_kk^-1 as packed lower triangles (36 doubles, element [r][c] at r(r+1)/2 + c; the
 // backward solve is their only reader); the last one stays in registers, as L_77^-T in accumulator layout.
+// An off-diagonal tile is stored in accumulator layout, lane l's two elements ([g][2kq], [g][2kq + 1]) at 2l, 2l + 1:
+// one 16-byte store or load per lane, 512 contiguous bytes per warp.  The products take the tile's k index in the
+// order k = 2kq + s in m8n8k4 step s, so that a lane's operand fragment of step s is its own element [g][2kq + s].
 template <int PB>
 struct LeftSmem {
   static constexpr int DIAG_OFF = 64 * (PB * (PB - 1) / 2);
   static constexpr int DOUBLES = DIAG_OFF + 36 * (PB - 1);                // 2044 at PB = 8
   __host__ __device__ static constexpr int off(int i, int j) { return 64 * (i * (i - 1) / 2 + j); }   // tile (i, j), i > j
 };
-// Position of element [r][c] inside an off-diagonal tile: pair 2f + s of fragment lane f = 4r + (c & 3), s = c >> 2,
-// so that a lane reads both of its operand fragments ([g][kq], [g][4 + kq]) as one 16-byte load.  XOR 2 on rows
-// r & 2: the 8-byte stores of one accumulator register by a half-warp (rows 4h .. 4h+3) then hit 16 distinct banks.
-__device__ __forceinline__ int lpos(int r, int c) { return (8 * r + 2 * (c & 3) + (c >> 2)) ^ (r & 2); }
 
 // FULL: p = 8 PB and a 16-byte aligned record (16-byte loads, every bound known at compile time); else any p of the
 // block count, element by element
@@ -496,54 +514,60 @@ __device__ __forceinline__ void left_chain(const omc_nn_dense_t& a, int chain, i
   double E[2];       // L_kk^-T of the current step (of the last one, for the backward solve)
   double w[PB];
   rhs_rows<PB>(a, ci, p, chain, g, w);
+  double z0, z1;     // drawn in the last step, in the issue gaps of its pivot stages (earlier they would spill)
   __syncwarp();      // the previous chain's reads of the slice are done
 
   bool bad = false;
   // the steps are unrolled by hand: every register array must be indexed by constants
   static_for(std::make_integer_sequence<int, PB>{}, [&](auto kc) {
     constexpr int k = decltype(kc)::value;
-    // block column k from the record (in L2 by now): its latency overlaps the fragment reads and DMMAs below
+    // block column k of Q from the record (in L2 by now), added once the products are summed: its latency overlaps
+    // the whole j loop instead of holding up the first DMMA
+    double q[PB][2];
 #pragma unroll
-    for (int i = k; i < PB; ++i) q_pair<VEC>(a, ci, p, i, k, g, kq, C[i][0], C[i][1]);
-    // C(i, k) -= L(i, j) L(k, j)', j < k: A = element [g][4s + kq] of L(i, j), B the same element of L(k, j)
+    for (int i = k; i < PB; ++i) q_pair<VEC>(a, ci, p, i, k, g, kq, q[i][0], q[i][1]);
+    // C(i, k) = Q(i, k) - sum_j L(i, j) L(k, j)', j < k: in step s, A = element [g][2kq + s] of L(i, j), B the same
+    // element of L(k, j)
+#pragma unroll
+    for (int i = k; i < PB; ++i) C[i][0] = C[i][1] = 0.0;
 #pragma unroll
     for (int j = 0; j < k; ++j) {
-      const int fr = (2 * lane) ^ (g & 2);
-      const double2 bk = *reinterpret_cast<const double2*>(sm + S::off(k, j) + fr);
+      const double2 bk = *reinterpret_cast<const double2*>(sm + S::off(k, j) + 2 * lane);
       wdmma(C[k][0], C[k][1], -bk.x, bk.x);
       wdmma(C[k][0], C[k][1], -bk.y, bk.y);
 #pragma unroll
       for (int i = k + 1; i < PB; ++i) {
-        const double2 ai = *reinterpret_cast<const double2*>(sm + S::off(i, j) + fr);
+        const double2 ai = *reinterpret_cast<const double2*>(sm + S::off(i, j) + 2 * lane);
         wdmma(C[i][0], C[i][1], -ai.x, bk.x);
         wdmma(C[i][0], C[i][1], -ai.y, bk.y);
       }
     }
+#pragma unroll
+    for (int i = k; i < PB; ++i) {
+      C[i][0] += q[i][0];
+      C[i][1] += q[i][1];
+    }
+    if (k == PB - 1) draw_z<PB>(a, p, chain, g, kq, z0, z1);
     E[0] = g == 2 * kq ? 1.0 : 0.0;
     E[1] = g == 2 * kq + 1 ? 1.0 : 0.0;
     factor_diag(C[k], E, w[k], g, kq, bad);
     if (k + 1 < PB) {
-      // B fragments of E = L_kk^-T: step s needs E[4s + kq][g], held by lane (4s + kq, g >> 1), register g & 1
+      // B fragments of E = L_kk^-T: step s needs E[2kq + s][g], held by lane (2kq + s, g >> 1), register g & 1
       double bf[2];
 #pragma unroll
       for (int s = 0; s < 2; ++s) {
-        const int src = 4 * (4 * s + kq) + (g >> 1);
+        const int src = 4 * (2 * kq + s) + (g >> 1);
         const double e0 = shf(E[0], src), e1 = shf(E[1], src);
         bf[s] = (g & 1) ? e1 : e0;
       }
       const double wk0 = shf(w[k], 8 * kq), wk1 = shf(w[k], 8 * kq + 4);   // w[k] at 2kq, 2kq + 1
 #pragma unroll
       for (int i = k + 1; i < PB; ++i) {
-        // L(i, k) = C(i, k) L_kk^-T: A = element [g][4s + kq] of C(i, k) (quad-local re-layout)
+        // L(i, k) = C(i, k) L_kk^-T: A of step s = the lane's own element [g][2kq + s] of C(i, k)
         double l0 = 0.0, l1 = 0.0;
-#pragma unroll
-        for (int s = 0; s < 2; ++s) {
-          const int src = 4 * g + 2 * s + (kq >> 1);
-          const double v0 = shf(C[i][0], src), v1 = shf(C[i][1], src);
-          wdmma(l0, l1, (kq & 1) ? v1 : v0, bf[s]);
-        }
-        sm[S::off(i, k) + lpos(g, 2 * kq)] = l0;
-        sm[S::off(i, k) + lpos(g, 2 * kq + 1)] = l1;
+        wdmma(l0, l1, C[i][0], bf[0]);
+        wdmma(l0, l1, C[i][1], bf[1]);
+        *reinterpret_cast<double2*>(sm + S::off(i, k) + 2 * lane) = make_double2(l0, l1);
         // w[i] -= L(i, k) w[k]
         double t = fma(l0, wk0, l1 * wk1);
         t += shx(t, 1);
@@ -559,8 +583,13 @@ __device__ __forceinline__ void left_chain(const omc_nn_dense_t& a, int chain, i
   });
   double* beta = a.beta + (long long)chain * p;
   if (bad) return not_pd(a, chain, beta, lane);
-  double z0, z1;
-  draw_z<PB>(a, p, chain, g, kq, z0, z1);
+  // the centre record's beta_hat in row layout, on its way while the backward solve runs
+  const bool rss = a.center.ptr && a.rss_out;
+  const double* cen = a.center.ptr + (long long)chain * a.center.chain_stride;
+  double crow[PB];
+#pragma unroll
+  for (int j = 0; j < PB; ++j) crow[j] = rss && 8 * j + g < p ? cen[8 * j + g] : 0.0;
+  double xr[PB];
   back_solve_inv<PB>(
       beta, p, w, z0, z1, g, kq,
       [&](int j, double& l0, double& l1) {
@@ -573,8 +602,20 @@ __device__ __forceinline__ void left_chain(const omc_nn_dense_t& a, int chain, i
           l1 = 2 * kq + 1 >= g ? dt[(2 * kq + 1) * (kq + 1)] : 0.0;
         }
       },
-      [&](int j, int tc, int r) { return sm[S::off(j, tc) + lpos(g, 2 * kq + r)]; });
-  if (a.center.ptr && a.rss_out) rss_epilogue<PB, VEC>(a, p, chain, ci.rec, beta, lane);
+      [&](int j, int tc) { return *reinterpret_cast<const double2*>(sm + S::off(j, tc) + 2 * lane); }, xr);
+  if (rss) {
+    // d from the solve's own registers: drow[j] = x[8j + g] - beta_hat[8j + g], the column layout by shuffle (the
+    // same doubles, with no store -> load round trip through L2)
+    double dcol[PB][2], drow[PB];
+#pragma unroll
+    for (int j = 0; j < PB; ++j) drow[j] = 8 * j + g < p ? xr[j] - crow[j] : 0.0;
+#pragma unroll
+    for (int j = 0; j < PB; ++j) {
+      dcol[j][0] = shf(drow[j], 8 * kq);
+      dcol[j][1] = shf(drow[j], 8 * kq + 4);
+    }
+    rss_sum<PB, VEC>(a, p, chain, ci.rec, cen, dcol, drow, lane);
+  }
 }
 
 template <int PB, bool FULL>

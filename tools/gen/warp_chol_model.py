@@ -147,59 +147,71 @@ def tile_matrix(T, PB):
     return M
 
 
+def factor_diag(D, E, wk):
+    """The 8 pivot stages of a diagonal tile D (accumulator layout) with E (identity on entry -> L_kk^-T) and the
+    right-hand side block wk riding along, as csrc/dense_warp.cu's factor_diag.  Returns (Lk, E, wk), Lk the factor
+    L_kk (lower triangle)."""
+    D, E, wk = D.copy(), E.copy(), wk.copy()
+    Lk = np.zeros((8, 8))
+    for jj in range(8):
+        reg, jq = jj & 1, jj >> 1
+        own = KQ == jq
+        piv = shfl(D[:, reg], 4 * jj + jq)
+        assert np.all(piv > 0)
+        rd = 1.0 / np.sqrt(piv)
+        D[:, reg] = np.where(own, D[:, reg] * rd, D[:, reg])
+        E[:, reg] = np.where(own, E[:, reg] * rd, E[:, reg])
+        wc = shfl(wk, 4 * jj) * rd
+        wk = np.where(G == jj, wc, wk)
+        lc0 = np.where(2 * KQ > jj, shfl(D[:, reg], 8 * KQ + jq), 0.0)
+        lc1 = np.where(2 * KQ + 1 > jj, shfl(D[:, reg], 8 * KQ + 4 + jq), 0.0)
+        lg, le = shfl(D[:, reg], 4 * G + jq), shfl(E[:, reg], 4 * G + jq)
+        Lk[G[KQ == 0], jj] = lg[KQ == 0]
+        D[:, 0] -= lg * lc0
+        D[:, 1] -= lg * lc1
+        wk = np.where(G > jj, wk - lg * wc, wk)
+        E[:, 0] -= le * lc0
+        E[:, 1] -= le * lc1
+    return np.tril(Lk), E, wk
+
+
 def run_left(Q, b, z, PB):
     """The left-looking kernel (nn_left_draw_kernel): block column k accumulated from the finished columns on the
     tensor pipe, the pivot stages on the diagonal tile only with an identity tile E riding along (E -> L_kk^-T), the
     panel L(i,k) = C(i,k) E by two m8n8k4 steps, w[i] -= L(i,k) w[k] as a lane-local mat-vec and a quad reduction,
-    L_kk^-1 kept in place of L_kk, and the backward solve x_j = L_jj^-T v_j as a mat-vec per block.
+    L_kk^-1 kept in place of L_kk, and the backward solve x_j = L_jj^-T v_j as a mat-vec per block.  The products
+    take a tile's k index as k = 2kq + s in step s, so every operand fragment is a lane's own accumulator element
+    [g][2kq + s] (no re-layout), except E's, which is E[2kq + s][g] by shuffle.
     Returns (x, L, Linv): L the factor (lower block triangle, diagonal blocks included), Linv its diagonal blocks'
     inverses as a block-diagonal matrix."""
     p = Q.shape[0]
     n = 8 * PB
     Qp, bp, zp = np.eye(n), np.zeros(n), np.zeros(n)
     Qp[:p, :p], bp[:p], zp[:p] = Q, b, z
-    L, Dk, Inv = {}, {}, {}
+    L, Lkk, Inv = {}, {}, {}
     w = [bp[8 * i + G].copy() for i in range(PB)]
     for k in range(PB):
-        C = {i: np.stack([Qp[8 * i + G, 8 * k + 2 * KQ], Qp[8 * i + G, 8 * k + 2 * KQ + 1]], axis=1) for i in range(k, PB)}
+        # the products from zero, block column k of Q added once at the end
+        C = {i: np.zeros((32, 2)) for i in range(k, PB)}
         for j in range(k):
-            Bk = rowfrag(L[k, j])
             for i in range(k, PB):
-                A = rowfrag(L[i, j])
                 for s in range(2):
-                    C[i] = dmma(C[i], -A[s], Bk[s])
-        D = C[k]
+                    C[i] = dmma(C[i], -L[i, j][:, s], L[k, j][:, s])
+        for i in range(k, PB):
+            C[i] = C[i] + np.stack([Qp[8 * i + G, 8 * k + 2 * KQ], Qp[8 * i + G, 8 * k + 2 * KQ + 1]], axis=1)
         E = np.stack([(G == 2 * KQ).astype(float), (G == 2 * KQ + 1).astype(float)], axis=1)
-        for jj in range(8):
-            reg, jq = jj & 1, jj >> 1
-            own = KQ == jq
-            piv = shfl(D[:, reg], 4 * jj + jq)
-            assert np.all(piv > 0)
-            rd = 1.0 / np.sqrt(piv)
-            D[:, reg] = np.where(own, D[:, reg] * rd, D[:, reg])
-            E[:, reg] = np.where(own, E[:, reg] * rd, E[:, reg])
-            wc = shfl(w[k], 4 * jj) * rd
-            w[k] = np.where(G == jj, wc, w[k])
-            lc0 = np.where(2 * KQ > jj, shfl(D[:, reg], 8 * KQ + jq), 0.0)
-            lc1 = np.where(2 * KQ + 1 > jj, shfl(D[:, reg], 8 * KQ + 4 + jq), 0.0)
-            lg, le = shfl(D[:, reg], 4 * G + jq), shfl(E[:, reg], 4 * G + jq)
-            D[:, 0] -= lg * lc0
-            D[:, 1] -= lg * lc1
-            w[k] = np.where(G > jj, w[k] - lg * wc, w[k])
-            E[:, 0] -= le * lc0
-            E[:, 1] -= le * lc1
-        Dk[k], Inv[k] = D, E
-        # B fragments of E: lane (g, kq), step s needs E[4s + kq][g], held by lane (4s + kq, g >> 1), register g & 1
+        Lkk[k], E, w[k] = factor_diag(C[k], E, w[k])
+        Inv[k] = E
+        # B fragments of E: lane (g, kq), step s needs E[2kq + s][g], held by lane (2kq + s, g >> 1), register g & 1
         Bf = []
         for s in range(2):
-            src = 4 * (4 * s + KQ) + (G >> 1)
+            src = 4 * (2 * KQ + s) + (G >> 1)
             Bf.append(np.where(G & 1, shfl(E[:, 1], src), shfl(E[:, 0], src)))
         wk0, wk1 = shfl(w[k], 8 * KQ), shfl(w[k], 8 * KQ + 4)
         for i in range(k + 1, PB):
-            A = rowfrag(C[i])
             c = np.zeros((32, 2))
             for s in range(2):
-                c = dmma(c, A[s], Bf[s])
+                c = dmma(c, C[i][:, s], Bf[s])
             L[i, k] = c
             t = c[:, 0] * wk0 + c[:, 1] * wk1
             t = t + shfl(t, LANES ^ 1)
@@ -227,7 +239,9 @@ def run_left(Q, b, z, PB):
         for tc in range(j):
             for r in range(2):
                 racc[tc, r] = racc[tc, r] - L[j, tc][:, r] * xg
-    Lfull = tile_matrix({**L, **{(k, k): Dk[k] for k in range(PB)}}, PB)
+    Lfull = tile_matrix(L, PB)
+    for k in range(PB):
+        Lfull[8 * k:8 * k + 8, 8 * k:8 * k + 8] = Lkk[k]
     Linv = tile_matrix({(k, k): Inv[k] for k in range(PB)}, PB).T
     return x[:p], np.tril(Lfull)[:p, :p], Linv[:p, :p]
 

@@ -2,6 +2,8 @@
 """SASS opcode summary of libomc.so, one block per cubin / kernel family: what the judge would otherwise have to dump.
 
     python tools/sass_summary.py > profiles/r02_sass_summary.txt
+    python tools/sass_summary.py --lib OTHER/libomc.so --match nn_left_draw     (every counted mnemonic of the kernels
+                                                                                 whose name contains the string)
 
 Counts the mnemonics that prove which hardware paths the kernels use: DMMA (FP64 tensor pipe; tcgen05 has no f64 kind),
 UBLKCP (1-D bulk copies through the TMA engine), SYNCS (mbarrier), LDGSTS, MUFU.RSQ64H, MEMBAR, local-memory traffic
@@ -17,14 +19,16 @@ import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "openmcmc_b200", "libomc.so")
-KEYS = ["DMMA", "DFMA", "DMUL", "DADD", "MUFU.RSQ64H", "MUFU.RCP64H", "UBLKCP", "SYNCS", "LDGSTS", "MEMBAR", "SHFL", "BAR.SYNC",
+KEYS = ["DMMA", "FSEL", "DFMA", "DMUL", "DADD", "MUFU.RSQ64H", "MUFU.RCP64H", "UBLKCP", "SYNCS", "LDGSTS", "MEMBAR", "SHFL", "BAR.SYNC",
         "ATOM", "RED", "LDS", "STS", "LDG", "STG", "LDL", "STL", "UTMALDG", "UTCHMMA", "UTCQMMA", "LDTM", "HMMA", "IMMA"]
 
 
 def main():
+    lib = sys.argv[sys.argv.index("--lib") + 1] if "--lib" in sys.argv else LIB
+    match = sys.argv[sys.argv.index("--match") + 1] if "--match" in sys.argv else None
     tmp = tempfile.mkdtemp()
-    subprocess.run(["cuobjdump", "-xelf", "all", LIB], cwd=tmp, check=True, capture_output=True)
-    print(f"# SASS summary of {os.path.relpath(LIB, ROOT)} (cuobjdump -xelf all; nvdisasm -c), mnemonic counts per kernel")
+    subprocess.run(["cuobjdump", "-xelf", "all", lib], cwd=tmp, check=True, capture_output=True)
+    print(f"# SASS summary of {os.path.relpath(lib, ROOT)} (cuobjdump -xelf all; nvdisasm -c), mnemonic counts per kernel")
     for cub in sorted(os.listdir(tmp)):
         if not cub.endswith(".cubin"):
             continue
@@ -50,11 +54,13 @@ def main():
         print("   totals: " + ", ".join(f"{k} {tot[k]}" for k in KEYS if tot[k]))
         print("   absent: " + ", ".join(k for k in ("UTMALDG", "UTCHMMA", "UTCQMMA", "LDTM", "HMMA", "IMMA") if not tot[k]))
         for kn, c in per.items():
+            if match and match not in kn:
+                continue
             short = subprocess.run(["c++filt", kn], capture_output=True, text=True).stdout.strip()
             short = re.sub(r"\(anonymous namespace\)::", "", short)
             short = re.sub(r"\(.*", "", short)[-90:]
-            print(f"   {c['_n']:6d}  {short:90s} " + " ".join(f"{k}={c[k]}" for k in KEYS if c[k] and k in
-                                                                  ("DMMA", "UBLKCP", "SYNCS", "LDGSTS", "MUFU.RSQ64H", "MEMBAR", "BAR.SYNC", "LDL", "STL")))
+            shown = KEYS if match else ("DMMA", "UBLKCP", "SYNCS", "LDGSTS", "MUFU.RSQ64H", "MEMBAR", "BAR.SYNC", "LDL", "STL")
+            print(f"   {c['_n']:6d}  {short:90s} " + " ".join(f"{k}={c[k]}" for k in KEYS if c[k] and k in shown))
 
 
 if __name__ == "__main__":
