@@ -141,6 +141,45 @@ int omc_nn_dense_draw(const omc_nn_dense_t* args, void* stream);
  * matrix fits in shared memory, p <= 136) */
 int omc_nn_dense_workspace(int n_chains, int p, long long* doubles);
 
+/* The same draw in a fixed eigenbasis, p <= 64, when G | g, the prior precision P0 (scaled identity or positive
+ * diagonal), mu0 and the centre record depend on data alone.  omc_nn_eigen_prep (once per run) factors
+ *   M'P0M = I, M'GM = D  (two-sided cyclic Jacobi on R^-1 G R^-1, R = diag(sqrt(P0)), M = R^-1 W)
+ * into the per-chain eigen record  M [p*p, column-major] | D [p] | h = M'g [p] | m = M'P0 mu0 [p] |
+ * u_hat = M'P0 beta_hat [p] | k = M'c0 [p]  (p*p + 5p doubles per chain; center NULL => u_hat = k = 0).  A chain whose
+ * Jacobi does not converge or whose record is not finite gets D[0] = NaN.
+ * omc_nn_eigen_draw (every sweep) then draws, with S = lambda I + tau D,
+ *   beta = M u,  u = S^-1 (tau h + lambda m) + S^-1/2 z,
+ * the same distribution as omc_nn_dense_draw (M S^-1/2 is a square root of Q^-1) from the same normals z (Philox block
+ * l of the chain for elements 2l, 2l+1), and, with center and rss_out, rss(beta) = rss0 - 2 e'k + e'D e, e = u - u_hat,
+ * to rss_out[chain * rss_stride].  Some S_i <= 0 or not finite: beta = NaN and OMC_STATUS_NOT_PD.
+ *   ref: sampler.py:154-207 (NormalNormal.sample), gmrf.py:167-198 */
+typedef struct {
+  int n_chains, p;
+  omc_vec_t stats;      /* records from omc_reg_pass (chain_stride = p*p+p+2): G | g                */
+  int prior_kind;       /* 0 scaled identity, 1 diagonal                                            */
+  omc_vec_t prior_P;    /* un-scaled prior precision (kind 0: 1 value or NULL => 1)                 */
+  omc_vec_t mu0;        /* prior mean [p]; NULL => 0                                                */
+  omc_vec_t center;     /* centre record beta_hat | c0 | rss0 (omc_nn_dense_t.center); NULL => 0    */
+  double* eig;          /* out [n_chains][p*p + 5p]                                                 */
+} omc_nn_eigen_prep_t;
+int omc_nn_eigen_prep(const omc_nn_eigen_prep_t* args, void* stream);
+
+typedef struct {
+  int n_chains, p;
+  const double* eig;    /* records from omc_nn_eigen_prep                                           */
+  omc_vec_t tau;        /* NULL => 1                                                                */
+  omc_vec_t lambda;     /* NULL => 1                                                                */
+  double* beta;         /* out [n_chains][p]                                                        */
+  omc_rng_t rng;
+  const double* debug_z; /* injected standard normals [n_chains][p]; NULL => Philox                */
+  long long debug_sweep_stride;
+  int* status;          /* optional [n_chains], OR-ed with OMC_STATUS_NOT_PD                        */
+  omc_vec_t center;     /* rss0 at element 2p of the centre record; NULL => rss not written         */
+  double* rss_out;
+  long long rss_stride; /* doubles between consecutive chains' rss_out                              */
+} omc_nn_eigen_draw_t;
+int omc_nn_eigen_draw(const omc_nn_eigen_draw_t* args, void* stream);
+
 /* omc_dense_factor: stand-alone dense SPD factorisation and solves, one CTA per matrix (n <= 512), the blocked Cholesky
  * with the DMMA trailing update that omc_nn_dense_draw runs:
  *   L = chol(Q)                              ref: gmrf.py:465-486 (cholesky), 489-520 (sparse_cholesky, dense branch)

@@ -67,6 +67,21 @@ class NNDense(C.Structure):
     ]
 
 
+class NNEigenPrep(C.Structure):
+    """omc_nn_eigen_prep_t"""
+
+    _fields_ = [("n_chains", C.c_int), ("p", C.c_int), ("stats", Vec), ("prior_kind", C.c_int), ("prior_P", Vec),
+                ("mu0", Vec), ("center", Vec), ("eig", C.c_void_p)]
+
+
+class NNEigenDraw(C.Structure):
+    """omc_nn_eigen_draw_t"""
+
+    _fields_ = [("n_chains", C.c_int), ("p", C.c_int), ("eig", C.c_void_p), ("tau", Vec), ("lam", Vec),
+                ("beta", C.c_void_p), ("rng", Rng), ("debug_z", C.c_void_p), ("debug_sweep_stride", C.c_longlong),
+                ("status", C.c_void_p), ("center", Vec), ("rss_out", C.c_void_p), ("rss_stride", C.c_longlong)]
+
+
 class DenseFactor(C.Structure):
     """omc_dense_factor_t"""
 
@@ -231,7 +246,8 @@ class FusedSmall(C.Structure):
 
 
 EXTRA_STRUCTS = {"omc_tridiag_nn_t": TridiagNN, "omc_dense_factor_t": DenseFactor, "omc_fop_t": FOp,
-                 "omc_fused_small_t": FusedSmall}
+                 "omc_fused_small_t": FusedSmall, "omc_nn_eigen_prep_t": NNEigenPrep,
+                 "omc_nn_eigen_draw_t": NNEigenDraw}
 
 # name -> (restype, argtypes); every symbol include/omc.h declares must be listed here (tests check both ways)
 PROTOTYPES = {
@@ -262,6 +278,8 @@ PROTOTYPES = {
     ),
     "omc_nn_dense_draw": (C.c_int, [C.POINTER(NNDense), C.c_void_p]),
     "omc_nn_dense_workspace": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_longlong)]),
+    "omc_nn_eigen_prep": (C.c_int, [C.POINTER(NNEigenPrep), C.c_void_p]),
+    "omc_nn_eigen_draw": (C.c_int, [C.POINTER(NNEigenDraw), C.c_void_p]),
     "omc_dense_factor": (C.c_int, [C.POINTER(DenseFactor), C.c_void_p]),
     "omc_quadform": (C.c_int, [C.POINTER(Quadform), C.c_void_p]),
     "omc_fused_small": (C.c_int, [C.POINTER(FusedSmall), C.c_void_p]),

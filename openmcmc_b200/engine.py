@@ -508,6 +508,8 @@ class RegressionLikelihood:
             self.center = plan.new(C, 2 * self.p + 2, fill=0.0)     # beta_hat | c0 | rss0 | cnt
             self.q_center = f"center[{dist.response}]"
             plan.add_quantity(Quantity(self.q_center, deps_data, self._emit_center))
+        self.deps_data = deps_data
+        self.eig = None
 
     def _emit_center(self):
         """Prologue only: centre beta_hat = (G with a 1e-12 relative diagonal jitter)^-1 g, then ONE explicit-residual
@@ -533,6 +535,27 @@ class RegressionLikelihood:
             self.center[:, p:].copy_(scratch[:, p * p:])
 
         plan.emit(launch, "reg_center")
+
+    def eigen_record(self, P0, mu0, prior_names):
+        """The eigen record M | D | h | m | u_hat | k of the element-wise dense draw (omc.h: omc_nn_eigen_prep), for the
+        prior precision P0 (eye or diagonal DevArray) and mean mu0 named in prior_names.  Data only, like the centre it
+        reads: computed in the prologue.  Returns (record [C, p*p + 5p], quantity name)."""
+        if self.eig is None:
+            self.eig = self.plan.new(self.plan.state.n_chains, K.eigen_record_len(self.p), fill=0.0)
+            self.q_eig = f"eigen[{self.dist.response}]"
+            self.plan.add_quantity(Quantity(self.q_eig, self.deps_data | frozenset(prior_names),
+                                            lambda: self._emit_eigen(P0, mu0)))
+        return self.eig, self.q_eig
+
+    def _emit_eigen(self, P0, mu0):
+        plan = self.plan
+        plan.require(self.q_center)
+        C, p = plan.state.n_chains, self.p
+
+        def launch():
+            K.nn_eigen_prep(C, p, self.stats, _mat_kind(P0), P0.vec(), mu0.vec(), self.center, self.eig)
+
+        plan.emit(launch, "nn_eigen_prep")
 
     def rss_ptr(self):
         return self.stats.data_ptr() + 8 * (self.p * self.p + self.p)

@@ -215,6 +215,45 @@ def nn_dense_draw(n_chains, p, stats, tau, prior_kind, prior_P, lam, mu0, beta, 
     check(lib().omc_nn_dense_draw(C.byref(a), stream_ptr()), "omc_nn_dense_draw")
 
 
+EIGEN_MAX_P = 64
+
+
+def eigen_record_len(p) -> int:
+    """Doubles per chain of the eigen record M | D | h | m | u_hat | k (omc_nn_eigen_prep)."""
+    return p * p + 5 * p
+
+
+def nn_eigen_prep(n_chains, p, stats, prior_kind, prior_P, mu0, center, eig):
+    """omc_nn_eigen_prep: per-chain eigenbasis M'P0M = I, M'GM = D of the records' G (P0 eye or diagonal) and the
+    vectors the draw needs, into eig [C, p*p + 5p]; center [C, 2p+1] (beta_hat | c0 | rss0) or None."""
+    a = _cabi.NNEigenPrep()
+    a.n_chains, a.p = int(n_chains), int(p)
+    a.stats = Vec(stats.data_ptr(), p * p + p + 2)
+    a.prior_kind, a.prior_P, a.mu0 = int(prior_kind), prior_P, mu0
+    a.center = Vec(center.data_ptr(), center.shape[1]) if center is not None else Vec(None, 0)
+    a.eig = eig.data_ptr()
+    check(lib().omc_nn_eigen_prep(C.byref(a), stream_ptr()), "omc_nn_eigen_prep")
+
+
+def nn_eigen_draw(n_chains, p, eig, tau, lam, beta, rng_, status=None, debug_z=None, debug_sweep_stride=0, center=None,
+                  rss_out=None, rss_stride=0):
+    """omc_nn_eigen_draw: beta = M u from the eigen record; with center and rss_out (a pointer, rss_stride doubles
+    between chains) also rss(beta)."""
+    a = _cabi.NNEigenDraw()
+    a.n_chains, a.p = int(n_chains), int(p)
+    a.eig = eig.data_ptr()
+    a.tau, a.lam = tau, lam
+    a.beta = beta.data_ptr()
+    a.rng = rng_
+    a.debug_z = debug_z.data_ptr() if debug_z is not None else None
+    a.debug_sweep_stride = int(debug_sweep_stride)
+    a.status = status.data_ptr() if status is not None else None
+    if center is not None:
+        a.center = Vec(center.data_ptr(), center.shape[1])
+        a.rss_out, a.rss_stride = rss_out, int(rss_stride)
+    check(lib().omc_nn_eigen_draw(C.byref(a), stream_ptr()), "omc_nn_eigen_draw")
+
+
 def dense_factor(Q, n, b=None, z=None, L=None, logdet=None, mean=None, x=None, status=None, factored=False,
                  backward_only=False, workspace=None, n_mats=None):
     """omc_dense_factor: blocked Cholesky / solves of n_mats dense SPD matrices [n_mats, n, n] (omc.h)."""

@@ -170,6 +170,7 @@ class NormalNormal(MCMCSampler):
         p = source["p"]
         tau = source["tau"]
         requires = list(source["require"]) if isinstance(source["require"], (list, tuple)) else [source["require"]]
+        eigen_prior = False
         if isinstance(prior.mean, MixtureParameterVector) and isinstance(prior.precision, MixtureParameterMatrix):
             mix = engine.get_mixture(plan, host_state, prior)
             requires.append(mix.qname)
@@ -195,6 +196,9 @@ class NormalNormal(MCMCSampler):
                 P0 = st.arrays[dname]
             lam = st[lam_name] if lam_name else None
             mu0_vec, P0_kind, P0_vec = mu0.vec, engine._mat_kind(P0), P0.vec
+            # the eigenbasis of (G, P0) is data when P0 and mu0 are (and a positive diagonal P0 has one)
+            eigen_prior = (P0.kind == "eye" or (P0.kind == "diag" and P0.npos == p)) and not (
+                {pm_name, prior.mean.form} & set(st.per_chain_names))
         beta = st[self.param]
         ctx = plan.ctx(self)
         if "rng" not in ctx:
@@ -231,6 +235,12 @@ class NormalNormal(MCMCSampler):
         centred = rl is not None and rl.center is not None and trunc is None
         if centred:
             requires.append(rl.q_center)
+        # G, g, P0, mu0 and the centre all data, nothing injected or probed: the draw runs in the fixed eigenbasis of
+        # (G, P0) (omc_nn_eigen_draw), a mat-vec per chain instead of a Cholesky of Q
+        eigen = centred and eigen_prior and p <= K.EIGEN_MAX_P and dz is None and probes is None
+        if eigen:
+            eig, q_eig = rl.eigen_record(P0, mu0, (pm_name, prior.mean.form))
+            requires.append(q_eig)
         for q in requires:
             plan.require(q)
         stats = source["stats"]
@@ -244,6 +254,10 @@ class NormalNormal(MCMCSampler):
         if source.get("pre"):
             plan.emit(*source["pre"])
 
+        def launch_eigen():
+            K.nn_eigen_draw(C, p, eig, tau.vec() if tau else K.vec(None), lam.vec() if lam else K.vec(None), beta.data,
+                            rng, status=plan.status, center=center, rss_out=rss_out, rss_stride=rl.rec)
+
         def launch():
             K.nn_dense_draw(
                 C, p, stats, tau.vec() if tau else K.vec(None), P0_kind, P0_vec(),
@@ -253,7 +267,7 @@ class NormalNormal(MCMCSampler):
                 debug_sweep_stride=dz_stride, trunc=trunc, debug_u=dz if trunc else None, center=center,
                 rss_out=rss_out, workspace=workspace)
 
-        plan.emit(launch, f"nn_dense_draw[{self.param}]")
+        plan.emit(launch_eigen if eigen else launch, f"nn_dense_draw[{self.param}]")
         plan.wrote(self.param)
         if centred:
             plan.valid[rl.q_rss] = True
